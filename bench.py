@@ -23,6 +23,11 @@ Headline line (one JSON object on stdout, rank 0):
                compute_reward() - each beside the C port and the NumPy port of the same call
   cpu_baseline the C oracle port on all host cores over a bounded sample of the same workload
   headline     both halves of BASELINE.json's metric once more, last on the line
+
+--dump-outputs DIR writes, after the timed steps, what the last timed IK step and the last timed reward step of rank 0
+computed, as DIR/<name>.npy (float32 / float64, about 40 MB): the IKResult fields of a fixed, seeded sample of 2^19
+queries, the rewards of a sample of 2^19 rows, and the indices of both samples.  The inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -38,6 +43,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: leave no __pycache__ behind in it
 
 import numpy as np  # noqa: E402
 
@@ -48,6 +54,7 @@ LOG2_N_IK = 24
 LOG2_N_REWARD = 24
 REWARD_KEYS = ("achieved_goal", "desired_goal", "ee_pos", "ee_quat", "fingers_width", "task_index")
 NEUTRAL = np.array([0.00, 0.41, 0.00, -1.85, 0.00, 2.26, 0.79])
+DUMP_SAMPLE = 1 << 19  # rows per --dump-outputs sample: 64 B per IK query + 12 B per reward row, 38 MiB in all
 
 
 def host_cores() -> int:
@@ -389,6 +396,36 @@ def cuda_time_steps(fn, steps, torch, presync=True):
     return total, [e0.elapsed_time(e1) for e0, e1 in evs]
 
 
+def dump_rows(n: int, seed: int) -> np.ndarray:
+    """Ascending row indices of the --dump-outputs sample: all n rows, or a fixed seeded DUMP_SAMPLE of them."""
+    if n <= DUMP_SAMPLE:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, DUMP_SAMPLE, replace=False))
+
+
+def write_dump(out_dir: str, ik_rows, q8, aux4, rw_rows, reward) -> None:
+    """The sampled outputs of the last timed steps as out_dir/<name>.npy: what ik_solve's BatchIKResult and reward()
+    return for those rows, flags and iteration counts as float32, indices as float64."""
+    from mujoco_panda_pnp_b200 import engine
+
+    q, pos_error, final_pos, word = engine.unpack_ik(q8, aux4)
+    arrays = {
+        "ik_query_index": ik_rows.astype(np.float64),
+        "ik_q": q,
+        "ik_final_pos": final_pos,
+        "ik_pos_error": pos_error,
+        "ik_iterations": (word & 0xFFFFFF).astype(np.float32),
+        "ik_converged": ((word & (1 << 24)) != 0).astype(np.float32),
+        "ik_success": ((word & (2 << 24)) != 0).astype(np.float32),
+        "reward_row_index": rw_rows.astype(np.float64),
+        "reward": reward,
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+    print(f"[bench] wrote {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 2**20:.1f} MiB) to {out_dir}")
+
+
 def run_ours(args) -> int:
     import torch
 
@@ -474,6 +511,11 @@ def run_ours(args) -> int:
     torch.cuda.synchronize()
     ik_total = ev0.elapsed_time(ev1)
     launches_ik = lib.pnp_launch_count() - launches0
+    dump = args.dump_outputs and rank == 0
+    if dump:  # the output set the last timed step wrote, before the launches below reuse it
+        ik_rows = dump_rows(n_ik, seed=0)
+        last = ik_outs[(ik_step_no[0] - 1) & 1]
+        ik_dump = {k: last[k].index_select(0, torch.from_numpy(ik_rows).to(dev)).cpu().numpy() for k in ("q8", "aux4")}
     D.barrier()
     ik_ms_total = D.reduce_max(ik_total, dev)
     ik_kernel_ms = ik_total / K
@@ -494,6 +536,9 @@ def run_ours(args) -> int:
     torch.cuda.synchronize()
     D.barrier()
     rw_total, t_rw = cuda_time_steps(rw_step, K, torch)
+    if dump:
+        rw_rows = dump_rows(n_rw, seed=1)
+        rw_dump = rw_out.index_select(0, torch.from_numpy(rw_rows).to(dev)).cpu().numpy()
     D.barrier()
     rw_ms_total = D.reduce_max(rw_total, dev)
     rw_kernel_ms = sum(t_rw) / K
@@ -504,14 +549,13 @@ def run_ours(args) -> int:
     h_targets = targets.cpu().pin_memory()
     h_neutral = NEUTRAL.astype(np.float32)
     h_out = dict(q8=torch.empty((n_ik, 8)).pin_memory().numpy(), aux4=torch.empty((n_ik, 4)).pin_memory().numpy())
-    Ke = max(3, min(K, 10))
     for _ in range(2):
         engine.ik_solve_host(h_targets, h_neutral, params, out=h_out)
     D.barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     conv_e2e = 0
-    for _ in range(Ke):
+    for _ in range(K):
         r = engine.ik_solve_host(h_targets, h_neutral, params, out=h_out)  # blocks until outputs are on the host
         conv_e2e += int(r["counters"][1])
     ik_e2e_s = D.reduce_max(time.perf_counter() - t0, dev)
@@ -526,7 +570,7 @@ def run_ours(args) -> int:
     D.barrier()
     t0 = time.perf_counter()
     conv_c = 0
-    for _ in range(Ke):
+    for _ in range(K):
         r = engine.ik_solve_host(h_targets, h_neutral, params, out=h_out, compact=True)
         conv_c += int(r["counters"][1])
     ik_e2e_c_s = D.reduce_max(time.perf_counter() - t0, dev)
@@ -550,9 +594,9 @@ def run_ours(args) -> int:
     raw_copies()
     D.barrier()
     t0 = time.perf_counter()
-    for _ in range(Ke):
+    for _ in range(K):
         raw_copies()
-    link_s = D.reduce_max(time.perf_counter() - t0, dev) / Ke
+    link_s = D.reduce_max(time.perf_counter() - t0, dev) / K
     link = {"h2d_plus_d2h_gbs_all_ranks": (n_ik * 60.0) * world / link_s / 1e9,
             "d2h_gbs_all_ranks": (n_ik * 48.0) * world / link_s / 1e9,
             "ceiling_solves_per_s": float(c[1]) / float(c[0]) * n_ik * world / link_s,
@@ -566,10 +610,10 @@ def run_ours(args) -> int:
         engine.reward_host(*h_rows, rw_params, want_success=False, out=h_rw)
     D.barrier()
     t0 = time.perf_counter()
-    for _ in range(Ke):
+    for _ in range(K):
         engine.reward_host(*h_rows, rw_params, want_success=False, out=h_rw)
     rw_e2e_s = D.reduce_max(time.perf_counter() - t0, dev)
-    rw_e2e = n_rw * world * Ke / rw_e2e_s
+    rw_e2e = n_rw * world * K / rw_e2e_s
 
     # ---------------- side configs (rank 0 only, short) ---------------------------------
     side = {}
@@ -771,9 +815,9 @@ def run_ours(args) -> int:
                     "note": "host-resident rows are PCIe bound (64 B/row over a ~57 GB/s link): about the speed of the CPU "
                             "port; the GPU reward pays when the rows are already resident (value, her_relabel)"}
         e2e = {"value": ik_e2e, "unit": "solves/s", "h2d_bytes_per_step": ik_h2d, "d2h_bytes_per_step": ik_d2h,
-               "steps": Ke, "api": "pnp_ik_solve_packed_host_f32 (pinned host buffers, 3-stream chunk pipeline)", "link": link}
+               "steps": K, "api": "pnp_ik_solve_packed_host_f32 (pinned host buffers, 3-stream chunk pipeline)", "link": link}
         e2e_compact = {"value": ik_e2e_c, "unit": "solves/s", "h2d_bytes_per_step": ik_h2d, "d2h_bytes_per_step": n_ik * 32 + 32,
-                       "steps": Ke, "api": "pnp_ik_solve_compact_host_f32 (q, iterations, converged, success; no final_pos / pos_error)"}
+                       "steps": K, "api": "pnp_ik_solve_compact_host_f32 (q, iterations, converged, success; no final_pos / pos_error)"}
         line = {
             "metric": "panda_ik_converged_solves_per_s", "value": ik_value, "unit": "solves/s", "n_gpus": world,
             "steps": K, "warmup": W, "ms_per_step": ik_ms_total / K, "higher_is_better": True, "scaling": "weak",
@@ -806,6 +850,8 @@ def run_ours(args) -> int:
                                for k, v in latency.items()},
             },
         }
+        if dump:
+            write_dump(args.dump_outputs, ik_rows, ik_dump["q8"], ik_dump["aux4"], rw_rows, rw_dump)
         emit(line)
     if world > 1:
         import torch.distributed as dist
@@ -840,7 +886,13 @@ def main() -> int:
     ap.add_argument("--log2-n-ik", type=int, default=LOG2_N_IK)
     ap.add_argument("--log2-n-reward", type=int, default=LOG2_N_REWARD)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's outputs to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 ASSET = os.path.join(ROOT, "mujoco_panda_pnp_b200", "assets", "panda_shelf_kinematic.xml")
-REFERENCE_XML = "/root/reference/panda_mujoco_gym/assets/shelf_pnp.xml"
 NEUTRAL = np.array([0.00, 0.41, 0.00, -1.85, 0.00, 2.26, 0.79])
 
 

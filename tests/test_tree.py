@@ -4,7 +4,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import ASSET, NEUTRAL, REFERENCE_XML, tree_fk
+from conftest import ASSET, GOLDEN, NEUTRAL, tree_fk
 from mujoco_panda_pnp_b200 import KinematicData, KinematicModel, KinematicTree
 from mujoco_panda_pnp_b200.mjcf import JNT_FREE, JNT_HINGE, JNT_SLIDE
 from oracle import ik_oracle, mj_oracle
@@ -38,17 +38,19 @@ def test_model_layout_matches_reference_scene(kin_model):
         m.site("nope")
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE_XML), reason="reference checkout not present")
 def test_packaged_asset_equals_reference_mjcf():
+    """tests/golden/reference_scene_golden.npz holds what the loader reads from the reference's
+    assets/shelf_pnp.xml (+ panda_mocap.xml): the model fields, the names and the canonical tree.  They were
+    recorded from the packaged asset, which had been checked field for field equal to the reference's MJCF and
+    whose bodies, joints and sites have not changed since."""
     ours = KinematicModel.from_xml_path(ASSET)
-    ref = KinematicModel.from_xml_path(REFERENCE_XML)
+    ref = np.load(os.path.join(GOLDEN, "reference_scene_golden.npz"))
     for f in ("body_parentid", "body_pos", "body_quat", "body_jntadr", "body_jntnum", "jnt_type", "jnt_axis",
               "jnt_pos", "jnt_qposadr", "jnt_dofadr", "jnt_range", "qpos0", "site_bodyid", "site_pos", "site_quat"):
-        np.testing.assert_array_equal(getattr(ours, f), getattr(ref, f), err_msg=f)
-    assert ours.body_names == ref.body_names and ours.joint_names == ref.joint_names
-    assert ours.site_names == ref.site_names
-    t1, t2 = KinematicTree.from_mjmodel(ours), KinematicTree.from_mjmodel(ref)
-    assert bytes(t1.to_struct()) == bytes(t2.to_struct())
+        np.testing.assert_array_equal(getattr(ours, f), ref[f], err_msg=f)
+    assert ours.body_names == ref["body_names"].tolist() and ours.joint_names == ref["joint_names"].tolist()
+    assert ours.site_names == ref["site_names"].tolist()
+    assert bytes(KinematicTree.from_mjmodel(ours).to_struct()) == ref["tree_struct"].tobytes()
 
 
 def test_from_mjmodel_accepts_foreign_model_objects(oracle_model):

@@ -277,3 +277,53 @@ def test_pose_ik_statement_agrees_with_an_independent_formulation(oracle_model):
         np.testing.assert_allclose(p, want["final_pos"], atol=1e-9)
         n_conv += converged
     assert n_conv >= 10
+
+
+def test_batched_pose_statement_walks_the_scalar_iterates(oracle_model, oracle_chain):
+    """pose_ik_oracle.solve_pose_batch (N queries at once on c_oracle's FK, NumPy mat2Quat / mulQuat / quat2vel, one
+    batched 6x6 solve) against the scalar statement solve_pose, query by query: the GPU pose tests run thousands of
+    queries against the batched form, so it has to be the same statement.  Half the queries start near their target,
+    half at NEUTRAL; the targets span all four mju_mat2Quat cases and a third of the quaternions are given as -q or
+    scaled (the statement normalises them and the angle fold makes -q the same rotation)."""
+    from oracle import pose_ik_oracle
+
+    rng = np.random.default_rng(5)
+    lo, hi = oracle_model.jnt_range[:7, 0], oracle_model.jnt_range[:7, 1]
+    # draw from the workspace until each mat2Quat case has 16 targets
+    qs = rng.uniform(lo, hi, (400, 7))
+    ev = pose_ik_oracle.pose_eval_batch(oracle_chain, qs, np.zeros(3), np.array([1.0, 0.0, 0.0, 0.0]))
+    pick = np.concatenate([np.nonzero(ev["case"] == c)[0][:16] for c in range(4)])
+    assert len(pick) == 64
+    q_star = qs[pick]
+    pos, quat = ev["final_pos"][pick], ev["final_quat"][pick].copy()
+    quat[1::3] *= -1.0
+    quat[2::6] *= 7.5
+    quat[5::6] *= 1e-3
+    near = np.arange(64) % 2 == 0
+    q_init = np.where(near[:, None], np.clip(q_star + rng.uniform(-0.3, 0.3, (64, 7)), lo, hi), NEUTRAL)
+    got = pose_ik_oracle.solve_pose_batch(oracle_chain, pos, quat, q_init)
+    d = mj_oracle.MjData(oracle_model)
+    ties = 0
+    for k in range(64):
+        w = pose_ik_oracle.solve_pose(oracle_model, d, pos[k], quat[k], q_init[k])
+        if got["iterations"][k] != w["iterations"]:
+            ties += 1  # FK rounding of the two restatements put one of them exactly on a threshold
+            continue
+        assert bool(got["converged"][k]) == w["converged"] and bool(got["success"][k]) == w["success"], k
+        if w["converged"]:
+            np.testing.assert_allclose(got["q"][k], w["q"], atol=1e-9, err_msg=str(k))
+            np.testing.assert_allclose(got["final_pos"][k], w["final_pos"], atol=1e-9, err_msg=str(k))
+            np.testing.assert_allclose(got["final_quat"][k], w["final_quat"], atol=1e-9, err_msg=str(k))
+            assert abs(got["pos_error"][k] - w["pos_error"]) < 1e-9 and abs(got["rot_error"][k] - w["rot_error"]) < 1e-9
+    assert ties <= 1, ties
+    assert got["converged"][near].all() and got["converged"][~near].mean() > 0.4
+    # the single evaluation is the pass the loop makes: at q_init with max_iters = 0
+    e0 = pose_ik_oracle.pose_eval_batch(oracle_chain, q_init, pos, quat)
+    z = pose_ik_oracle.solve_pose_batch(oracle_chain, pos, quat, q_init, max_iters=0)
+    assert (z["iterations"] == 0).all() and not z["converged"].any() and np.array_equal(z["q"], q_init)
+    for key in ("final_pos", "final_quat", "pos_error", "rot_error"):
+        np.testing.assert_array_equal(z[key], e0[key])
+    # both hemispheres of the error quaternion occur, and -q gives the same rotation error as q
+    assert (e0["err_w"] < 0).any() and (e0["err_w"] > 0).any()
+    e1 = pose_ik_oracle.pose_eval_batch(oracle_chain, q_init, pos, -quat)
+    np.testing.assert_allclose(e1["rot_error"], e0["rot_error"], atol=1e-12)

@@ -153,7 +153,9 @@ int pnp_ik_solve_f32(const float* targets, const float* q_init, int32_t q_init_s
  * or overwrites memory of the first (the library compares the byte ranges and falls back to plain stream order); from
  * 16384 queries per SM up a launch is followed by a small resume launch that finishes its last stragglers.  Neither
  * changes a result bit.  The first such launch on a stream allocates 6 MB of device scratch (cudaMalloc: one device
- * synchronisation).  Captured launches (CUDA graphs) keep plain stream order.  See INTEGRATION.md section 4. */
+ * synchronisation).  Captured launches (CUDA graphs) keep plain stream order.  The restart kernels of
+ * pnp_ik_solve_multistart_* are plain launches (no programmatic-serialization attribute, no early trigger): an IK launch
+ * queued after a multistart call cannot start before the call's last kernel has completed.  See INTEGRATION.md section 4. */
 /* Same solve with PACKED outputs (the fast path: 3 x 128-bit stores per query instead of 13):
  *   out_q8  [n][8] float = q0..q6, pos_error
  *   out_aux4[n][4] float = final_pos xyz, then a 32-bit word (iterations | flags << 24)
@@ -171,6 +173,37 @@ int pnp_ik_solve_compact_f32(const float* targets, const float* q_init, int32_t 
 int pnp_ik_solve_f64(const double* targets, const double* q_init, int32_t q_init_stride, int64_t n,
                      const PnpIkParams* params, double* q_out, double* final_pos, double* pos_err,
                      int32_t* iters, uint8_t* flags, unsigned long long* counters, void* stream);
+/* ---- multi-start solve: restart the queries that attempt 0 did not solve from a shared seed table ---------------- */
+/* Attempt 0 is the plain solve of the same layout (pnp_ik_solve_f32 / _packed_f32 / _f64) from q_init, same params,
+ * same kernel choice.  For every query whose attempt 0 is not a success, attempts 1..n_seeds solve the same target from
+ * seeds[k - 1] (seeds[n_seeds][7], q_init semantics: may lie outside the limits), same params.  A query returns the
+ * record of its FIRST successful attempt in the order 0, 1, ..., n_seeds, or attempt 0's when none succeeds; every output
+ * field is bit-identical to the plain entry point's result for that target from that start.  0 <= n_seeds <= 255;
+ * n_seeds = 0 is the plain solve (no extra kernel launch).
+ *   attempt[n]        uint8 (nullable): the attempt returned
+ *   counters[4]       (nullable, accumulated): as pnp_ik_solve_*, over the RETURNED records
+ *   restart_stats[3]  (nullable, accumulated): queries that entered restarts, queries rescued, DLS passes run by restart
+ *                     attempts (the cost; >= the iterations of the returned restart attempts)
+ *   scratch           device memory, 16-byte aligned, pnp_ik_multistart_scratch_bytes(n) bytes; required
+ * The separate layouts need flags (non-null: the restarts read attempt 0's success from it).  seeds and scratch must not
+ * overlap an output.  The call never synchronises the host (it can be captured in a CUDA graph): the restarts run in
+ * ceil(n_seeds / G) waves that read their list lengths on the device.  They are plain launches, so a library IK launch
+ * queued after a multistart call on the same stream starts only once the multistart has completed. */
+int pnp_ik_multistart_scratch_bytes(int64_t n, int64_t* bytes);
+int pnp_ik_solve_multistart_f32(const float* targets, const float* q_init, int32_t q_init_stride, int64_t n,
+                                const float* seeds, int32_t n_seeds, const PnpIkParams* params, float* q_out,
+                                float* final_pos, float* pos_err, int32_t* iters, uint8_t* flags, uint8_t* attempt,
+                                unsigned long long* counters, unsigned long long* restart_stats, void* scratch,
+                                void* stream);
+int pnp_ik_solve_multistart_packed_f32(const float* targets, const float* q_init, int32_t q_init_stride, int64_t n,
+                                       const float* seeds, int32_t n_seeds, const PnpIkParams* params, float* out_q8,
+                                       float* out_aux4, uint8_t* attempt, unsigned long long* counters,
+                                       unsigned long long* restart_stats, void* scratch, void* stream);
+int pnp_ik_solve_multistart_f64(const double* targets, const double* q_init, int32_t q_init_stride, int64_t n,
+                                const double* seeds, int32_t n_seeds, const PnpIkParams* params, double* q_out,
+                                double* final_pos, double* pos_err, int32_t* iters, uint8_t* flags, uint8_t* attempt,
+                                unsigned long long* counters, unsigned long long* restart_stats, void* scratch,
+                                void* stream);
 /* Launch scratch (the refill ticket of the IK / waypoint / pose / planner kernels, the plan-order histograms) is kept
  * per STREAM: any number of launches may be queued on a stream, and up to 64 distinct streams per device may have
  * library launches in flight at the same time.  A captured CUDA graph keeps the scratch of its capture stream - do

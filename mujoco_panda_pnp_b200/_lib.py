@@ -85,6 +85,13 @@ SIGNATURES = {
     "pnp_ik_solve_packed_f32": (c_int, [_P, _P, c_int32, c_int64, POINTER(PnpIkParams), _P, _P, _P, _P]),
     "pnp_ik_solve_compact_f32": (c_int, [_P, _P, c_int32, c_int64, POINTER(PnpIkParams), _P, _P, _P]),
     "pnp_ik_solve_f64": (c_int, [_P, _P, c_int32, c_int64, POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_ik_multistart_scratch_bytes": (c_int, [c_int64, POINTER(c_int64)]),
+    "pnp_ik_solve_multistart_f32": (c_int, [_P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams), _P, _P, _P, _P, _P,
+                                            _P, _P, _P, _P, _P]),
+    "pnp_ik_solve_multistart_packed_f32": (c_int, [_P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams), _P, _P, _P,
+                                                   _P, _P, _P, _P]),
+    "pnp_ik_solve_multistart_f64": (c_int, [_P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams), _P, _P, _P, _P, _P,
+                                            _P, _P, _P, _P, _P]),
     "pnp_ik_waypoints_f32": (c_int, [_P, _P, c_int64, c_int32, c_double, POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P]),
     "pnp_ik_pose_solve_f32": (c_int, [_P, _P, _P, c_int32, c_int64, POINTER(PnpIkParams), c_double, c_double,
                                       _P, _P, _P, _P, _P, _P, _P, _P, _P]),

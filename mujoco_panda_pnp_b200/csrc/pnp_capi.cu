@@ -61,6 +61,7 @@ struct DeviceState {
   bool slot_used[kStreamSlots] = {};
   unsigned slot_clock = 0;
   int occ_ik[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  int occ_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // restart wave kernels of the multistart solve
   bool obs_smem_set = false;
   bool fk_smem_set = false;
   bool plan_smem_set = false;
@@ -571,6 +572,115 @@ int ik_solve_impl(const T* targets, const T* q_init, int32_t q_init_stride, int6
   return launch_ik<T, pnp::GenericKin, kOut>(s, a, small, st);
 }
 
+// ---- multistart (see ms_collect_kernel / ms_wave_* in pnp_kernels.cuh) ----------------------------------------------
+// Lanes per restarted query: the seeds a wave runs in parallel.  A wave lasts as long as its slowest attempt (up to
+// max_iters passes) whatever its width, so fewer, wider waves cost less until the lanes no longer fit the SMs at once;
+// see DESIGN.md 4.1 for the measurement.  PNP_MS_GROUP overrides it (1, 2, 4 or 8), for measurements.
+constexpr int kMsGroup = 4;
+constexpr size_t kMsHdrBytes = pnp::MS_HDR_WORDS * sizeof(unsigned);
+size_t ms_list_bytes(int64_t n) { return ((size_t)n * sizeof(unsigned) + 15u) & ~(size_t)15u; }
+// header | list A | list B | iterations of attempt 0 (separate layout without an iters output)
+size_t ms_scratch_bytes(int64_t n) { return kMsHdrBytes + 3 * ms_list_bytes(n); }
+
+template <typename K, typename T>
+int launch_ms_wave(DeviceState* s, K kernel, int occ_slot, const pnp::MsArgs<T>& m, cudaStream_t st) {
+  if (s->occ_ms[occ_slot] == 0) {
+    int occ = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, pnp::MS_BLOCK, 0);
+    s->occ_ms[occ_slot] = (e == cudaSuccess && occ > 0) ? occ : 1;
+  }
+  kernel<<<s->sm_count * s->occ_ms[occ_slot], pnp::MS_BLOCK, 0, st>>>(m);
+  ++g_launches;
+  CUDA_TRY(cudaGetLastError());
+  return PNP_OK;
+}
+
+template <typename T, int kOut>
+int ik_multistart_impl(const T* targets, const T* q_init, int32_t q_init_stride, int64_t n, const T* seeds, int32_t n_seeds,
+                       const PnpIkParams* params, T* q_out, T* final_pos, T* pos_err, int32_t* iters, uint8_t* flags,
+                       uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats, void* scratch,
+                       void* stream) {
+  if (n_seeds < 0 || n_seeds > pnp::MS_MAX_SEEDS) return fail(PNP_EINVAL, "ik_multistart: n_seeds must be in [0, 255]");
+  if (n_seeds > 0 && !seeds) return fail(PNP_EINVAL, "ik_multistart: seeds is NULL");
+  if (!scratch || !aligned16(scratch)) return fail(PNP_EINVAL, "ik_multistart: scratch must be non-null and 16-byte aligned");
+  if (kOut == pnp::IK_OUT_SEPARATE && n > 0 && !flags)
+    return fail(PNP_EINVAL, "ik_multistart: flags must be non-null (the restarts read attempt 0's success from it)");
+  if (n > 0) {
+    // seeds (read by every wave) and scratch (written) must not share memory with an output
+    auto range = [](const void* p, size_t bytes) { ByteRange r; if (p) { r.b = (const char*)p; r.e = r.b + bytes; } return r; };
+    const size_t m = (size_t)n;
+    const ByteRange in[2] = {range(seeds, (size_t)n_seeds * PNP_NJOINT * sizeof(T)), range(scratch, ms_scratch_bytes(n))};
+    ByteRange out[8];
+    if (kOut == pnp::IK_OUT_SEPARATE) {
+      out[0] = range(q_out, m * PNP_NJOINT * sizeof(T)); out[1] = range(final_pos, m * 3 * sizeof(T));
+      out[2] = range(pos_err, m * sizeof(T)); out[3] = range(iters, m * sizeof(int32_t)); out[4] = range(flags, m);
+    } else {
+      out[0] = range(q_out, m * 8 * sizeof(float)); out[1] = range(final_pos, m * 4 * sizeof(float));
+    }
+    out[5] = range(attempt, m);
+    out[6] = range(counters, 4 * sizeof(unsigned long long));
+    out[7] = range(restart_stats, 3 * sizeof(unsigned long long));
+    for (const ByteRange& o : out)
+      if (ranges_overlap(o, in[0]) || ranges_overlap(o, in[1]))
+        return fail(PNP_EINVAL, "ik_multistart: seeds and scratch must not overlap an output");
+    if (ranges_overlap(in[0], in[1])) return fail(PNP_EINVAL, "ik_multistart: seeds and scratch must not overlap");
+  }
+  unsigned* hdr = static_cast<unsigned*>(scratch);
+  unsigned* list[2] = {reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes),
+                       reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes + ms_list_bytes(n))};
+  int32_t* iters0 = iters;
+  if (kOut == pnp::IK_OUT_SEPARATE && !iters0 && n_seeds > 0)  // the restarts need attempt 0's iterations for the counters
+    iters0 = reinterpret_cast<int32_t*>((char*)scratch + kMsHdrBytes + 2 * ms_list_bytes(n));
+  // attempt 0: the plain entry point, unchanged
+  int rc = ik_solve_impl<T, kOut>(targets, q_init, q_init_stride, n, params, q_out, final_pos, pos_err, iters0, flags, counters,
+                                  stream);
+  if (rc || n == 0) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (attempt) CUDA_TRY(cudaMemsetAsync(attempt, 0, (size_t)n, st));
+  if (n_seeds == 0) return PNP_OK;
+  DeviceState* s;
+  if ((rc = current_state(&s))) return rc;
+  bool spec;
+  if ((rc = pick_kin(s, params->kinematics, &spec))) return rc;
+
+  CUDA_TRY(cudaMemsetAsync(hdr, 0, kMsHdrBytes, st));
+  {
+    const int grid = grid_for(n, pnp::MS_COLLECT_BLOCK, s->sm_count, 8);
+    pnp::ms_collect_kernel<kOut><<<grid, pnp::MS_COLLECT_BLOCK, 0, st>>>(
+        flags, reinterpret_cast<const unsigned*>(final_pos), (unsigned)n, list[0], hdr, restart_stats);
+    ++g_launches;
+    CUDA_TRY(cudaGetLastError());
+  }
+  static const int env_group = env_int("PNP_MS_GROUP", 0);
+  const int G = (env_group == 1 || env_group == 2 || env_group == 4 || env_group == 8) ? env_group : kMsGroup;
+  pnp::MsArgs<T> m;
+  pnp::IkArgs<T>& a = m.a;
+  memset(&a, 0, sizeof a);
+  a.targets = targets; a.q_init = q_init; a.q_init_stride = q_init_stride; a.n = (unsigned)n;
+  a.k = make_ik_const<T>(params);
+  a.q_out = q_out; a.final_pos = final_pos; a.pos_err = pos_err; a.iters = iters0; a.flags = flags; a.counters = counters;
+  a.thresh2 = a.k.pos_thresh * a.k.pos_thresh;
+  m.seeds = seeds; m.n_seeds = n_seeds; m.group = (unsigned)G;
+  m.iters0 = iters0; m.attempt = attempt; m.restart_stats = restart_stats;
+  const int waves = (n_seeds + G - 1) / G;
+  for (int w = 0; w < waves; ++w) {
+    m.wave = w;
+    m.list_in = list[w & 1]; m.cnt_in = hdr + w;
+    m.list_out = w + 1 < waves ? list[(w + 1) & 1] : nullptr; m.cnt_out = hdr + w + 1;
+    if constexpr (std::is_same<T, float>::value) {
+      if (spec && params->kinematics != PNP_KIN_GENERIC)
+        rc = launch_ms_wave(s, pnp::ms_wave_v_kernel<kOut>, kOut == pnp::IK_OUT_SEPARATE ? 0 : 1, m, st);
+      else
+        rc = launch_ms_wave(s, pnp::ms_wave_kernel<float, pnp::GenericKin, kOut>, kOut == pnp::IK_OUT_SEPARATE ? 2 : 3, m, st);
+    } else {
+      rc = spec ? launch_ms_wave(s, pnp::ms_wave_kernel<double, pnp::SpecKin, kOut>, 4, m, st)
+                : launch_ms_wave(s, pnp::ms_wave_kernel<double, pnp::GenericKin, kOut>, 5, m, st);
+    }
+    if (rc) return rc;
+  }
+  return PNP_OK;
+}
+
 // Smallest double s >= 0 with sqrt(s) >= t (sqrt is correctly rounded, hence monotone): the
 // reference's `sqrt(s) < t` is exactly `s < sqrt_preimage(t)`.
 double sqrt_preimage(double t) {
@@ -756,6 +866,36 @@ int pnp_ik_solve_f64(const double* targets, const double* q_init, int32_t q_init
                      uint8_t* flags, unsigned long long* counters, void* stream) {
   return ik_solve_impl<double, pnp::IK_OUT_SEPARATE>(targets, q_init, q_init_stride, n, params, q_out, final_pos, pos_err, iters,
                                       flags, counters, stream);
+}
+
+int pnp_ik_multistart_scratch_bytes(int64_t n, int64_t* bytes) {
+  if (n < 0 || !bytes) return fail(PNP_EINVAL, "ik_multistart_scratch_bytes: negative n or NULL bytes");
+  *bytes = (int64_t)ms_scratch_bytes(n);
+  return PNP_OK;
+}
+int pnp_ik_solve_multistart_f32(const float* targets, const float* q_init, int32_t q_init_stride, int64_t n, const float* seeds,
+                                int32_t n_seeds, const PnpIkParams* params, float* q_out, float* final_pos, float* pos_err,
+                                int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                unsigned long long* restart_stats, void* scratch, void* stream) {
+  return ik_multistart_impl<float, pnp::IK_OUT_SEPARATE>(targets, q_init, q_init_stride, n, seeds, n_seeds, params, q_out,
+                                                         final_pos, pos_err, iters, flags, attempt, counters, restart_stats,
+                                                         scratch, stream);
+}
+int pnp_ik_solve_multistart_packed_f32(const float* targets, const float* q_init, int32_t q_init_stride, int64_t n,
+                                       const float* seeds, int32_t n_seeds, const PnpIkParams* params, float* out_q8,
+                                       float* out_aux4, uint8_t* attempt, unsigned long long* counters,
+                                       unsigned long long* restart_stats, void* scratch, void* stream) {
+  return ik_multistart_impl<float, pnp::IK_OUT_PACKED>(targets, q_init, q_init_stride, n, seeds, n_seeds, params, out_q8,
+                                                       out_aux4, nullptr, nullptr, nullptr, attempt, counters, restart_stats,
+                                                       scratch, stream);
+}
+int pnp_ik_solve_multistart_f64(const double* targets, const double* q_init, int32_t q_init_stride, int64_t n,
+                                const double* seeds, int32_t n_seeds, const PnpIkParams* params, double* q_out,
+                                double* final_pos, double* pos_err, int32_t* iters, uint8_t* flags, uint8_t* attempt,
+                                unsigned long long* counters, unsigned long long* restart_stats, void* scratch, void* stream) {
+  return ik_multistart_impl<double, pnp::IK_OUT_SEPARATE>(targets, q_init, q_init_stride, n, seeds, n_seeds, params, q_out,
+                                                          final_pos, pos_err, iters, flags, attempt, counters, restart_stats,
+                                                          scratch, stream);
 }
 
 int pnp_ik_waypoints_f32(const float* q_start, const float* goal, int64_t n, int32_t n_steps, double step_size,

@@ -1007,6 +1007,238 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_solve_one_kernel(const float* __r
 }
 
 // =============================================================================================
+// Multi-start position IK (pnp_ik_solve_multistart_*): attempt 0 is the plain solve above, written to the outputs by
+// the plain launch path.  For the queries it did not solve, attempts 1..K restart the same target from a shared seed
+// table; a query returns the record of its first successful attempt (attempt 0's when none succeeds).
+//
+//   ms_collect_kernel   appends the index of every query whose attempt 0 failed to a list (one atomic per warp)
+//   ms_wave_*_kernel    wave w: each listed query gets a group of G consecutive lanes of one warp that run the seeds
+//                       [w G, w G + G) in parallel, each a plain solve from its seed (lane_solve on the specialised tree,
+//                       the ik_solve_kernel pass everywhere else: the same arithmetic as the plain entry points, so a
+//                       returned attempt is bit-identical to the plain solve from that start).  The lowest lane of the
+//                       group that succeeds overwrites the query's record; a query without a success goes onto the
+//                       next wave's list.
+// Every wave is launched whether or not its list is empty: it reads the list length on the device and its blocks leave at
+// once when they have nothing to do, so the host never reads a count.  The order of a list is not deterministic, the
+// outputs are: each query depends on its own attempts only.
+// =============================================================================================
+constexpr int MS_BLOCK = 128;
+constexpr int MS_COLLECT_BLOCK = 256;
+constexpr int MS_MAX_SEEDS = 255;
+constexpr int MS_HDR_WORDS = 256;  // list lengths: [0] = failures of attempt 0, [w + 1] = queries still failed after wave w
+
+template <typename T>
+struct MsArgs {
+  IkArgs<T> a;             // targets and the outputs of attempt 0 (its layout), solver constants
+  const T* seeds;          // [n_seeds][7]
+  int n_seeds;
+  int wave;                // this launch runs seeds [wave * group, wave * group + group)
+  unsigned group;          // lanes per query: a power of two <= 32
+  const unsigned* list_in;
+  const unsigned* cnt_in;
+  unsigned* list_out;      // nullptr: last wave
+  unsigned* cnt_out;
+  const int32_t* iters0;   // separate layout: iterations of attempt 0 (the iters output or scratch)
+  uint8_t* attempt;        // nullable
+  unsigned long long* restart_stats;  // nullable: restarted, rescued, DLS passes of restart attempts
+};
+
+// success bit of attempt 0: flags[] (separate layout) or the flag byte of the packed word
+template <int kOut>
+__global__ void __launch_bounds__(MS_COLLECT_BLOCK) ms_collect_kernel(const uint8_t* __restrict__ flags,
+                                                                      const unsigned* __restrict__ aux_words, unsigned n,
+                                                                      unsigned* __restrict__ list, unsigned* __restrict__ cnt,
+                                                                      unsigned long long* __restrict__ restart_stats) {
+  const unsigned lane = threadIdx.x & 31u;
+  const unsigned stride = gridDim.x * MS_COLLECT_BLOCK;
+  unsigned long long c_fail = 0;
+  for (unsigned base = blockIdx.x * MS_COLLECT_BLOCK + (threadIdx.x & ~31u); base < n; base += stride) {  // warp-uniform
+    const unsigned i = base + lane;
+    bool failed = false;
+    if (i < n) {
+      const unsigned fl = kOut == IK_OUT_SEPARATE ? (unsigned)flags[i] : aux_words[(size_t)i * 4u + 3u] >> 24;
+      failed = (fl & PNP_IK_SUCCESS) == 0u;
+    }
+    const unsigned fb = __ballot_sync(FULL, failed);
+    if (fb) {
+      unsigned at = 0;
+      if (lane == 0) at = atomicAdd(cnt, (unsigned)__popc(fb));
+      at = __shfl_sync(FULL, at, 0);
+      if (failed) list[at + (unsigned)__popc(fb & ((1u << lane) - 1u))] = i;
+      c_fail += (unsigned)__popc(fb);
+    }
+  }
+  if (restart_stats && lane == 0 && c_fail) atomicAdd(restart_stats + 0, c_fail);
+}
+
+// The part of a wave both lane mappings share: pick the group's first success, store it, queue the unsolved queries.
+// `solve(valid, id, seed, out...)` runs one attempt per lane and stores nothing.
+template <typename T, int kOut, typename Solve, typename Store>
+__device__ __forceinline__ void ms_wave(const MsArgs<T>& m, unsigned cnt, Solve solve, Store store) {
+  const unsigned lane = threadIdx.x & 31u;
+  const unsigned G = m.group;
+  const unsigned gl = lane & (G - 1u);
+  const unsigned gmask = (G == 32u ? FULL : ((1u << G) - 1u)) << (lane & ~(G - 1u));
+  const unsigned long long lanes_total = (unsigned long long)cnt * G;
+  // warps interleaved over the blocks: a short list spreads over as many SMs as possible
+  const unsigned warps_total = gridDim.x * (MS_BLOCK / 32);
+  const unsigned warp_id = (threadIdx.x >> 5) * gridDim.x + blockIdx.x;
+  unsigned long long c_conv = 0, c_iter = 0, c_rescued = 0, c_passes = 0;
+  bool worked = false;
+  for (unsigned long long base = (unsigned long long)warp_id * 32u; base < lanes_total; base += (unsigned long long)warps_total * 32u) {
+    worked = true;
+    const unsigned long long L = base + lane;
+    const bool listed = L < lanes_total;
+    const unsigned id = listed ? m.list_in[L / G] : 0u;
+    const int seed = m.wave * (int)G + (int)gl;
+    const bool valid = listed && seed < m.n_seeds;
+    bool succ;
+    int iterations;
+    solve(valid, id, valid ? seed : 0, succ, iterations);
+    succ = succ && valid;
+    c_passes += valid ? (unsigned)iterations : 0u;
+    const unsigned sb = __ballot_sync(FULL, succ) & gmask;
+    if (sb && lane == (unsigned)(__ffs(sb) - 1)) {
+      // the record of attempt 0 leaves the returned set: correct the counters (which counted it) by the difference
+      unsigned old_fl, old_it;
+      if (kOut == IK_OUT_SEPARATE) {
+        old_fl = m.a.flags[id];
+        old_it = (unsigned)m.iters0[id];
+      } else {
+        const unsigned w = reinterpret_cast<const unsigned*>(m.a.final_pos)[(size_t)id * 4u + 3u];
+        old_fl = w >> 24;
+        old_it = w & 0xFFFFFFu;
+      }
+      store(id);
+      if (m.attempt) m.attempt[id] = (uint8_t)(seed + 1);
+      c_conv += 1ull - (unsigned long long)(old_fl & PNP_IK_CONVERGED);
+      c_iter += (unsigned long long)(unsigned)iterations - (unsigned long long)old_it;  // mod 2^64
+      c_rescued += 1u;
+    }
+    const bool push = m.list_out && listed && gl == 0u && !sb;
+    const unsigned pb = __ballot_sync(FULL, push);
+    if (pb) {
+      unsigned at = 0;
+      if (lane == 0) at = atomicAdd(m.cnt_out, (unsigned)__popc(pb));
+      at = __shfl_sync(FULL, at, 0);
+      if (push) m.list_out[at + (unsigned)__popc(pb & ((1u << lane) - 1u))] = id;
+    }
+  }
+  if (!worked) return;
+  if (m.a.counters) {
+    const unsigned long long w_conv = warp_sum(c_conv), w_iter = warp_sum(c_iter);
+    if (lane == 0) {
+      atomicAdd(m.a.counters + PNP_IK_CNT_CONVERGED, w_conv);
+      atomicAdd(m.a.counters + PNP_IK_CNT_SUCCESS, w_conv);  // success == converged, as the plain kernels count it
+      atomicAdd(m.a.counters + PNP_IK_CNT_ITERATIONS, w_iter);
+    }
+  }
+  if (m.restart_stats) {
+    const unsigned long long w_res = warp_sum(c_rescued), w_pass = warp_sum(c_passes);
+    if (lane == 0) {
+      atomicAdd(m.restart_stats + 1, w_res);
+      atomicAdd(m.restart_stats + 2, w_pass);
+    }
+  }
+}
+
+// FP32 on the specialised tree: lane_solve + store_lane_result, i.e. ik_solve_small_kernel's arithmetic per lane
+template <int kOut>
+__global__ void __launch_bounds__(MS_BLOCK) ms_wave_v_kernel(const MsArgs<float> m) {
+  const unsigned cnt = *m.cnt_in;
+  if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;  // no work for any warp of this block
+  __shared__ __align__(16) float s_trig[kTrigVWords];
+  load_trigv_table(s_trig);
+  __syncthreads();
+  const TrigV trig{s_trig};
+  float q[NJ], pf[3], n2f;
+  bool conv;
+  int it_kept = 0;
+  auto solve = [&](bool valid, unsigned id, int seed, bool& succ, int& iterations) {
+    float q0[NJ], tgt[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) tgt[i] = m.a.targets[(size_t)id * 3u + i];
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) q[i] = q0[i] = m.seeds[seed * NJ + i];
+    lane_solve(m.a.k, trig, valid, 0, q, q0, tgt, pf, n2f, iterations, conv);
+    succ = conv && (finish_sqrt(n2f) < m.a.k.pos_thresh * 2.0f);  // store_lane_result's success
+    it_kept = iterations;
+  };
+  auto store = [&](unsigned id) { store_lane_result<kOut>(m.a, id, q, pf, n2f, it_kept, conv); };
+  ms_wave<float, kOut>(m, cnt, solve, store);
+}
+
+// FP32 on other trees and FP64: per lane the pass of ik_solve_kernel (ik_eval_and_step), no refill
+template <typename T, typename Kin, int kOut>
+__global__ void __launch_bounds__(MS_BLOCK) ms_wave_kernel(const MsArgs<T> m) {
+  const unsigned cnt = *m.cnt_in;
+  if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  const Trig<T> trig{s_tab};
+  T q[NJ], p[3], n2;
+  bool conv;
+  int it_kept = 0;
+  auto solve = [&](bool valid, unsigned id, int seed, bool& succ, int& iterations) {
+    T tgt[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) tgt[i] = m.a.targets[(size_t)id * 3u + i];
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) q[i] = m.seeds[seed * NJ + i];
+    bool active = valid;
+    conv = false;
+    iterations = 0;
+    p[0] = p[1] = p[2] = T(0);
+    n2 = T(0);
+    for (int it = 0; __any_sync(FULL, active); ++it) {
+      T pp[3], nn2, qn[NJ];
+      ik_eval_and_step<T, Kin>(q, tgt, m.a.k, trig, pp, nn2, qn);
+      const bool last = it >= m.a.k.max_iters;             // loop ran out (ik_solver.py:57)
+      const bool cv = !last && below_thresh(nn2, m.a.k);   // :61-64
+      if (active) {
+        if (cv || last) {
+          conv = cv;
+          iterations = cv ? it + 1 : it;                   // :66 / :85
+          p[0] = pp[0]; p[1] = pp[1]; p[2] = pp[2];
+          n2 = nn2;
+          active = false;
+        } else {
+#pragma unroll
+          for (int i = 0; i < NJ; ++i) q[i] = qn[i];       // :81-85
+        }
+      }
+    }
+    succ = conv && (finish_sqrt(n2) < m.a.k.pos_thresh * T(2));
+    it_kept = iterations;
+  };
+  auto store = [&](unsigned id) {  // ik_solve_kernel's store block
+    const T err = finish_sqrt(n2);
+    const bool success = conv && (err < m.a.k.pos_thresh * T(2));
+    const unsigned fl = (conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u);
+    if (kOut == IK_OUT_PACKED) {
+      float4* oq = reinterpret_cast<float4*>(m.a.q_out) + (size_t)id * 2u;
+      oq[0] = make_float4((float)q[0], (float)q[1], (float)q[2], (float)q[3]);
+      oq[1] = make_float4((float)q[4], (float)q[5], (float)q[6], (float)err);
+      reinterpret_cast<float4*>(m.a.final_pos)[id] =
+          make_float4((float)p[0], (float)p[1], (float)p[2], __int_as_float((int)((unsigned)it_kept | (fl << 24))));
+    } else {
+      T* qo = m.a.q_out + (size_t)id * NJ;
+#pragma unroll
+      for (int i = 0; i < NJ; ++i) qo[i] = q[i];
+      if (m.a.final_pos) {
+        T* fp = m.a.final_pos + (size_t)id * 3u;
+        fp[0] = p[0]; fp[1] = p[1]; fp[2] = p[2];
+      }
+      if (m.a.pos_err) m.a.pos_err[id] = err;
+      if (m.a.iters) m.a.iters[id] = it_kept;
+      m.a.flags[id] = (uint8_t)fl;
+    }
+  };
+  ms_wave<T, kOut>(m, cnt, solve, store);
+}
+
+// =============================================================================================
 // Warm-started waypoint sequences (MoveIKSkill.reset inner loop, skills/move.py:106-137):
 // one lane per env, q carried in registers across the n_steps solves.
 // =============================================================================================

@@ -145,8 +145,9 @@ class BatchIKResult:
     word (iterations | flags << 24) on first access, so a solve launches exactly one kernel."""
 
     def __init__(self, success=None, q=None, final_pos=None, pos_error=None, iterations=None, converged=None,
-                 counters=None, word=None):
+                 counters=None, word=None, attempt=None):
         self.q, self.final_pos, self.pos_error, self.counters = q, final_pos, pos_error, counters
+        self.attempt = attempt  # ik_solve_multistart: uint8[N], the attempt each row is the result of (0 = from q_init)
         self._success, self._iterations, self._converged, self._word = success, iterations, converged, word
 
     @property
@@ -270,6 +271,93 @@ def ik_solve(targets: torch.Tensor, q_init: torch.Tensor, params: PnpIkParams, c
     return BatchIKResult(
         success=(flags & 2) != 0, q=q, final_pos=fpos, pos_error=err, iterations=iters,
         converged=(flags & 1) != 0, counters=counters,
+    )
+
+
+def ik_restart_seeds(k: int, lower=None, upper=None, seed: int = 0, dtype=torch.float32, device="cuda") -> torch.Tensor:
+    """A seed table for ik_solve_multistart: k joint configurations ~ U(lower, upper), shape (k, 7).
+
+    Drawn from a CPU ``torch.Generator`` and then moved to ``device``, so a seed gives the same table on every device.
+    ``lower`` / ``upper`` default to the joint limits of the packaged kinematic tree."""
+    if lower is None or upper is None:
+        t = KinematicTree.from_mjcf()
+        lower = t.lower if lower is None else lower
+        upper = t.upper if upper is None else upper
+    from .synthetic import random_joint_configs
+
+    return random_joint_configs(int(k), lower, upper, seed=seed, device="cpu", dtype=torch.float64).to(
+        device=device, dtype=dtype).contiguous()
+
+
+def ik_solve_multistart(targets: torch.Tensor, q_init: torch.Tensor, seeds: torch.Tensor, params: PnpIkParams,
+                        counters: Optional[torch.Tensor] = None, restart_stats: Optional[torch.Tensor] = None,
+                        packed: Optional[bool] = None) -> BatchIKResult:
+    """ik_solve, then every query it did not solve is solved again from the rows of ``seeds`` (K, 7), in order, until
+    one succeeds (pnp_ik_solve_multistart_*).  Each row of the result is, bit for bit, the plain ik_solve of that target
+    from the start ``result.attempt`` names (0 = q_init, k = seeds[k - 1]); rows no attempt solves keep attempt 0.
+
+    ``counters`` (int64[4]) accumulates over the returned rows like ik_solve's; ``restart_stats`` (int64[3])
+    accumulates queries restarted, queries rescued and DLS passes spent on restarts.  Same layouts as ik_solve
+    (packed float32 by default, ``packed=False`` / float64: separate arrays).  Never synchronises."""
+    lib = _lib.load()
+    dt = targets.dtype
+    if dt not in (torch.float32, torch.float64):
+        raise ValueError("targets must be float32 or float64")
+    targets = _check_cuda("targets", targets, dt, (3,))
+    n = targets.shape[0]
+    dev = targets.device
+    if q_init.dim() == 1:
+        if q_init.shape != (7,):
+            raise ValueError("broadcast q_init must have shape (7,)")
+        stride = 0
+        q_init = q_init.to(device=dev, dtype=dt).contiguous()
+    else:
+        q_init = _check_cuda("q_init", q_init, dt, (7,))
+        if q_init.shape[0] != n:
+            raise ValueError("q_init and targets disagree on N")
+        stride = 7
+    seeds = torch.as_tensor(seeds).to(device=dev, dtype=dt).reshape(-1, 7).contiguous()
+    k = seeds.shape[0]
+    if k > 255:
+        raise ValueError(f"at most 255 seeds, got {k}")
+    for name, t, m in (("counters", counters, 4), ("restart_stats", restart_stats, 3)):
+        if t is not None and (t.dtype != torch.int64 or t.numel() < m or not t.is_cuda):
+            raise ValueError(f"{name} must be a CUDA int64 tensor with >= {m} elements")
+    if packed is None:
+        packed = dt == torch.float32
+    if packed and dt != torch.float32:
+        raise ValueError("packed outputs exist for float32 only")
+    nbytes = ctypes.c_int64()
+    _lib.check(lib.pnp_ik_multistart_scratch_bytes(n, ctypes.byref(nbytes)), "pnp_ik_multistart_scratch_bytes")
+    with torch.cuda.device(dev):
+        scratch = torch.empty(((nbytes.value + 15) // 16, 4), dtype=torch.int32, device=dev)
+        attempt = torch.empty((n,), dtype=torch.uint8, device=dev)
+        if packed:
+            q8 = torch.empty((n, 8), dtype=dt, device=dev)
+            aux = torch.empty((n, 4), dtype=dt, device=dev)
+            _lib.check(
+                lib.pnp_ik_solve_multistart_packed_f32(_ptr(targets), _ptr(q_init), stride, n, _ptr(seeds), k,
+                                                       ctypes.byref(params), _ptr(q8), _ptr(aux), _ptr(attempt),
+                                                       _ptr(counters), _ptr(restart_stats), _ptr(scratch), _stream()),
+                "pnp_ik_solve_multistart_packed",
+            )
+            q, err, fpos, word = unpack_ik(q8, aux)
+            return BatchIKResult(q=q, final_pos=fpos, pos_error=err, word=word, counters=counters, attempt=attempt)
+        q = torch.empty((n, 7), dtype=dt, device=dev)
+        fpos = torch.empty((n, 3), dtype=dt, device=dev)
+        err = torch.empty((n,), dtype=dt, device=dev)
+        iters = torch.empty((n,), dtype=torch.int32, device=dev)
+        flags = torch.empty((n,), dtype=torch.uint8, device=dev)
+        fn = lib.pnp_ik_solve_multistart_f32 if dt == torch.float32 else lib.pnp_ik_solve_multistart_f64
+        _lib.check(
+            fn(_ptr(targets), _ptr(q_init), stride, n, _ptr(seeds), k, ctypes.byref(params), _ptr(q), _ptr(fpos),
+               _ptr(err), _ptr(iters), _ptr(flags), _ptr(attempt), _ptr(counters), _ptr(restart_stats), _ptr(scratch),
+               _stream()),
+            "pnp_ik_solve_multistart",
+        )
+    return BatchIKResult(
+        success=(flags & 2) != 0, q=q, final_pos=fpos, pos_error=err, iterations=iters,
+        converged=(flags & 1) != 0, counters=counters, attempt=attempt,
     )
 
 

@@ -79,14 +79,17 @@ class JacobianIKController:
 
     def solve(self, target_pos: np.ndarray, q_init: np.ndarray,
               max_iters: int = 100, pos_thresh: float = 1e-3,
-              damping: float = 1e-2, step_limit: float = 0.1) -> IKResult:
+              damping: float = 1e-2, step_limit: float = 0.1, seeds=None) -> IKResult:
         """Same contract as the reference (ik_solver.py:35-101).  Side effect kept: on return
-        ``data.qpos[:7] == result.q`` and ``data.site_xpos[site_id] == result.final_pos``."""
+        ``data.qpos[:7] == result.q`` and ``data.site_xpos[site_id] == result.final_pos``.
+
+        ``seeds`` (K, 7), an extension: when the solve from ``q_init`` fails, retry from each seed in turn and return
+        the first success (see solve_batch); the call then goes through the batch path."""
         target_pos = np.asarray(target_pos, dtype=np.float64)
         q_init = np.asarray(q_init, dtype=np.float64)
         if target_pos.shape != (3,) or q_init.shape != (7,):
             raise ValueError("solve expects target_pos (3,) and q_init (7,)")
-        if self.precision == "fp32":
+        if self.precision == "fp32" and seeds is None:
             # one C call, no memcpy: the kernel reads the query from and writes the result to a mapped
             # pinned mailbox (pnp_ik_solve_one_host_f32)
             key = (max_iters, pos_thresh, damping, step_limit)
@@ -109,7 +112,7 @@ class JacobianIKController:
             self._write_back(q, final_pos)
             return IKResult(success=bool(word & (2 << 24)), q=q, final_pos=final_pos, pos_error=float(o[7]),
                             iterations=word & 0xFFFFFF, converged=bool(word & (1 << 24)))
-        r = self.solve_batch(target_pos[None], q_init[None], max_iters, pos_thresh, damping, step_limit)
+        r = self.solve_batch(target_pos[None], q_init[None], max_iters, pos_thresh, damping, step_limit, seeds=seeds)
         q = r.q[0].double().cpu().numpy()
         final_pos = r.final_pos[0].double().cpu().numpy()
         self._write_back(q, final_pos)
@@ -119,10 +122,14 @@ class JacobianIKController:
         )
 
     def solve_batch(self, targets, q_init, max_iters: int = 100, pos_thresh: float = 1e-3,
-                    damping: float = 1e-2, step_limit: float = 0.1, counters=None) -> BatchIKResult:
+                    damping: float = 1e-2, step_limit: float = 0.1, counters=None, seeds=None) -> BatchIKResult:
         """N independent solves in one launch.  targets (N,3); q_init (N,7) or (7,) broadcast.
         NumPy / CPU inputs are copied to ``self.device``; CUDA tensors are used in place.
-        Returns device tensors (BatchIKResult)."""
+        Returns device tensors (BatchIKResult).
+
+        ``seeds`` (K, 7), K <= 255 (e.g. ``engine.ik_restart_seeds(8)``): every query the solve from ``q_init`` does not
+        solve is solved again from seeds[0], seeds[1], ... until one succeeds (engine.ik_solve_multistart); the result
+        then carries ``attempt`` (0 = from q_init, k = from seeds[k - 1])."""
         dt = self._dtype()
         with torch.cuda.device(self.device):
             engine.set_tree(self.tree)
@@ -131,7 +138,11 @@ class JacobianIKController:
                 raise ValueError(f"targets must have shape (N, 3), got {tuple(t.shape)}")
             t = t.to(device=self.device, dtype=dt)
             qi = qi.to(device=self.device, dtype=dt)
-            return engine.ik_solve(t, qi, self._params(max_iters, pos_thresh, damping, step_limit), counters=counters)
+            params = self._params(max_iters, pos_thresh, damping, step_limit)
+            if seeds is not None:
+                sd = _to_tensor(seeds).to(device=self.device, dtype=dt)
+                return engine.ik_solve_multistart(t, qi, sd, params, counters=counters)
+            return engine.ik_solve(t, qi, params, counters=counters)
 
     def fk(self, q):
         """EE-site position, wxyz quaternion and 6x7 Jacobian [jacp; jacr] at q (N,7)."""

@@ -239,6 +239,32 @@ int pnp_ik_pose_solve_f64(const double* target_pos, const double* target_quat, c
                           double rot_weight, double* q_out, double* final_pos, double* final_quat,
                           double* pos_err, double* rot_err, int32_t* iters, uint8_t* flags,
                           unsigned long long* counters, void* stream);
+/* Multi-start pose solve: pnp_ik_pose_solve_* from q_init (attempt 0, unchanged), then, for every query whose attempt 0
+ * is not a success, attempts 1..n_seeds solve the same pose from seeds[k - 1] (seeds[n_seeds][7], q_init semantics),
+ * same params.  A query returns the record of its FIRST successful attempt in the order 0, 1, ..., n_seeds, or attempt
+ * 0's when none succeeds; every output (q_out, final_pos, final_quat, pos_err, rot_err, iters, flags; nullable as in
+ * pnp_ik_pose_solve_*) is bit-identical to the plain entry point's for that target from that start.  0 <= n_seeds <= 255;
+ * n_seeds = 0 is the plain pose solve plus attempt zeroed (no extra kernel launch).
+ *   flags             required (the restarts read attempt 0's success from it)
+ *   attempt[n]        uint8 (nullable): the attempt returned
+ *   counters[4]       (nullable, accumulated): as pnp_ik_pose_solve_*, over the RETURNED records
+ *   restart_stats[3]  (nullable, accumulated): queries that entered restarts, queries rescued, DLS passes run by restart
+ *                     attempts (>= the iterations of the returned restart attempts)
+ *   scratch           device memory, 16-byte aligned, pnp_ik_multistart_scratch_bytes(n) bytes; required
+ * seeds and scratch must not overlap an output or each other.  Like pnp_ik_solve_multistart_*, the call never
+ * synchronises the host (it can be captured in a CUDA graph) and its restart waves are plain launches. */
+int pnp_ik_pose_solve_multistart_f32(const float* target_pos, const float* target_quat, const float* q_init,
+                                     int32_t q_init_stride, int64_t n, const float* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, double rot_thresh, double rot_weight, float* q_out,
+                                     float* final_pos, float* final_quat, float* pos_err, float* rot_err, int32_t* iters,
+                                     uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                     unsigned long long* restart_stats, void* scratch, void* stream);
+int pnp_ik_pose_solve_multistart_f64(const double* target_pos, const double* target_quat, const double* q_init,
+                                     int32_t q_init_stride, int64_t n, const double* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, double rot_thresh, double rot_weight, double* q_out,
+                                     double* final_pos, double* final_quat, double* pos_err, double* rot_err,
+                                     int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                     unsigned long long* restart_stats, void* scratch, void* stream);
 
 /* ---- full MoveIKSkill.reset trajectory planner (skills/move.py:76-191) -------------------- */
 typedef struct PnpMoveParams {

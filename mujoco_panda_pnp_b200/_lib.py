@@ -97,6 +97,10 @@ SIGNATURES = {
                                       _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "pnp_ik_pose_solve_f64": (c_int, [_P, _P, _P, c_int32, c_int64, POINTER(PnpIkParams), c_double, c_double,
                                       _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_ik_pose_solve_multistart_f32": (c_int, [_P, _P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams),
+                                                 c_double, c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_ik_pose_solve_multistart_f64": (c_int, [_P, _P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams),
+                                                 c_double, c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_ik_plan_f32": (c_int, [_P, _P, c_int64, POINTER(PnpMoveParams), POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_ik_plan_f64": (c_int, [_P, _P, c_int64, POINTER(PnpMoveParams), POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_plan_order_f32": (c_int, [_P, _P, c_int64, _P, c_int32, _P]),

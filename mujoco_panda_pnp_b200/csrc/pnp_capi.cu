@@ -61,7 +61,7 @@ struct DeviceState {
   bool slot_used[kStreamSlots] = {};
   unsigned slot_clock = 0;
   int occ_ik[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  int occ_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // restart wave kernels of the multistart solve
+  int occ_ms[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};  // restart wave kernels of the multistart solves (position, pose)
   bool obs_smem_set = false;
   bool fk_smem_set = false;
   bool plan_smem_set = false;
@@ -582,8 +582,8 @@ size_t ms_list_bytes(int64_t n) { return ((size_t)n * sizeof(unsigned) + 15u) & 
 // header | list A | list B | iterations of attempt 0 (separate layout without an iters output)
 size_t ms_scratch_bytes(int64_t n) { return kMsHdrBytes + 3 * ms_list_bytes(n); }
 
-template <typename K, typename T>
-int launch_ms_wave(DeviceState* s, K kernel, int occ_slot, const pnp::MsArgs<T>& m, cudaStream_t st) {
+template <typename K, typename M>
+int launch_ms_wave(DeviceState* s, K kernel, int occ_slot, const M& m, cudaStream_t st) {
   if (s->occ_ms[occ_slot] == 0) {
     int occ = 0;
     cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, pnp::MS_BLOCK, 0);
@@ -1009,6 +1009,92 @@ int pose_solve_impl(const T* tpos, const T* tquat, const T* q_init, int32_t q_in
   return PNP_OK;
 }
 
+// Multi-start pose solve: pose_solve_impl, then the restart waves of ms_pose_wave_kernel (see ik_multistart_impl).
+// Lanes per restarted query.  About a quarter of a cold workspace batch enters the first wave, and a failing attempt
+// runs all max_iters passes, so a wave costs about its lane count times max_iters: the narrowest group, which spends
+// no attempt on a query an earlier seed already rescues, measured fastest (DESIGN.md 4.6: 2^22 W-cold poses with 8
+// seeds in 14.7 ms at G = 1, 16.0 / 20.3 / 30.8 ms at G = 2 / 4 / 8).  PNP_MS_POSE_GROUP overrides it (1, 2, 4 or 8), for
+// measurements.
+constexpr int kMsPoseGroup = 1;
+
+template <typename T>
+int pose_multistart_impl(const T* tpos, const T* tquat, const T* q_init, int32_t q_init_stride, int64_t n, const T* seeds,
+                         int32_t n_seeds, const PnpIkParams* params, double rot_thresh, double rot_weight, T* q_out,
+                         T* final_pos, T* final_quat, T* pos_err, T* rot_err, int32_t* iters, uint8_t* flags,
+                         uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats, void* scratch,
+                         void* stream) {
+  if (n_seeds < 0 || n_seeds > pnp::MS_MAX_SEEDS) return fail(PNP_EINVAL, "ik_pose_multistart: n_seeds must be in [0, 255]");
+  if (n_seeds > 0 && !seeds) return fail(PNP_EINVAL, "ik_pose_multistart: seeds is NULL");
+  if (!scratch || !aligned16(scratch))
+    return fail(PNP_EINVAL, "ik_pose_multistart: scratch must be non-null and 16-byte aligned");
+  if (n > 0 && !flags)
+    return fail(PNP_EINVAL, "ik_pose_multistart: flags must be non-null (the restarts read attempt 0's success from it)");
+  if (n > 0) {
+    // seeds (read by every wave) and scratch (written) must not share memory with an output or with each other
+    auto range = [](const void* p, size_t bytes) { ByteRange r; if (p) { r.b = (const char*)p; r.e = r.b + bytes; } return r; };
+    const size_t m = (size_t)n;
+    const ByteRange in[2] = {range(seeds, (size_t)n_seeds * PNP_NJOINT * sizeof(T)), range(scratch, ms_scratch_bytes(n))};
+    const ByteRange out[10] = {range(q_out, m * PNP_NJOINT * sizeof(T)), range(final_pos, m * 3 * sizeof(T)),
+                               range(final_quat, m * 4 * sizeof(T)), range(pos_err, m * sizeof(T)),
+                               range(rot_err, m * sizeof(T)), range(iters, m * sizeof(int32_t)), range(flags, m),
+                               range(attempt, m), range(counters, 4 * sizeof(unsigned long long)),
+                               range(restart_stats, 3 * sizeof(unsigned long long))};
+    for (const ByteRange& o : out)
+      if (ranges_overlap(o, in[0]) || ranges_overlap(o, in[1]))
+        return fail(PNP_EINVAL, "ik_pose_multistart: seeds and scratch must not overlap an output");
+    if (ranges_overlap(in[0], in[1])) return fail(PNP_EINVAL, "ik_pose_multistart: seeds and scratch must not overlap");
+  }
+  unsigned* hdr = static_cast<unsigned*>(scratch);
+  unsigned* list[2] = {reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes),
+                       reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes + ms_list_bytes(n))};
+  int32_t* iters0 = iters;
+  if (!iters0 && n_seeds > 0)  // the restarts need attempt 0's iterations for the counters
+    iters0 = reinterpret_cast<int32_t*>((char*)scratch + kMsHdrBytes + 2 * ms_list_bytes(n));
+  // attempt 0: the plain entry point, unchanged
+  int rc = pose_solve_impl<T>(tpos, tquat, q_init, q_init_stride, n, params, rot_thresh, rot_weight, q_out, final_pos,
+                              final_quat, pos_err, rot_err, iters0, flags, counters, stream);
+  if (rc || n == 0) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (attempt) CUDA_TRY(cudaMemsetAsync(attempt, 0, (size_t)n, st));
+  if (n_seeds == 0) return PNP_OK;
+  DeviceState* s;
+  if ((rc = current_state(&s))) return rc;
+  bool spec;
+  if ((rc = pick_kin(s, params->kinematics, &spec))) return rc;
+
+  CUDA_TRY(cudaMemsetAsync(hdr, 0, kMsHdrBytes, st));
+  {
+    const int grid = grid_for(n, pnp::MS_COLLECT_BLOCK, s->sm_count, 8);
+    pnp::ms_collect_kernel<pnp::IK_OUT_SEPARATE><<<grid, pnp::MS_COLLECT_BLOCK, 0, st>>>(
+        flags, nullptr, (unsigned)n, list[0], hdr, restart_stats);
+    ++g_launches;
+    CUDA_TRY(cudaGetLastError());
+  }
+  static const int env_group = env_int("PNP_MS_POSE_GROUP", 0);
+  const int G = (env_group == 1 || env_group == 2 || env_group == 4 || env_group == 8) ? env_group : kMsPoseGroup;
+  pnp::MsPoseArgs<T> m;
+  pnp::PoseIkArgs<T>& a = m.a;
+  memset(&a, 0, sizeof a);
+  a.target_pos = tpos; a.target_quat = tquat; a.q_init = q_init; a.q_init_stride = q_init_stride; a.n = (unsigned)n;
+  a.k = make_ik_const<T>(params);
+  a.rot_thresh = (T)rot_thresh; a.rot_weight = (T)rot_weight;
+  a.q_out = q_out; a.final_pos = final_pos; a.final_quat = final_quat; a.pos_err = pos_err; a.rot_err = rot_err;
+  a.iters = iters0; a.flags = flags; a.counters = counters;
+  m.seeds = seeds; m.n_seeds = n_seeds; m.group = (unsigned)G;
+  m.iters0 = iters0; m.attempt = attempt; m.restart_stats = restart_stats;
+  const int waves = (n_seeds + G - 1) / G;
+  for (int w = 0; w < waves; ++w) {
+    m.wave = w;
+    m.list_in = list[w & 1]; m.cnt_in = hdr + w;
+    m.list_out = w + 1 < waves ? list[(w + 1) & 1] : nullptr; m.cnt_out = hdr + w + 1;
+    const int slot = 6 + (std::is_same<T, float>::value ? 0 : 2) + (spec ? 0 : 1);
+    rc = spec ? launch_ms_wave(s, pnp::ms_pose_wave_kernel<T, pnp::SpecKin>, slot, m, st)
+              : launch_ms_wave(s, pnp::ms_pose_wave_kernel<T, pnp::GenericKin>, slot, m, st);
+    if (rc) return rc;
+  }
+  return PNP_OK;
+}
+
 template <typename T>
 int plan_order_impl(const T* q_start, const T* target, int64_t n, uint32_t* order, int32_t kinematics, void* stream,
                     float4* records = nullptr) {
@@ -1164,6 +1250,27 @@ int pnp_ik_pose_solve_f64(const double* target_pos, const double* target_quat, c
                           double* rot_err, int32_t* iters, uint8_t* flags, unsigned long long* counters, void* stream) {
   return pose_solve_impl<double>(target_pos, target_quat, q_init, q_init_stride, n, params, rot_thresh, rot_weight, q_out,
                                  final_pos, final_quat, pos_err, rot_err, iters, flags, counters, stream);
+}
+
+int pnp_ik_pose_solve_multistart_f32(const float* target_pos, const float* target_quat, const float* q_init,
+                                     int32_t q_init_stride, int64_t n, const float* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, double rot_thresh, double rot_weight, float* q_out,
+                                     float* final_pos, float* final_quat, float* pos_err, float* rot_err, int32_t* iters,
+                                     uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                     unsigned long long* restart_stats, void* scratch, void* stream) {
+  return pose_multistart_impl<float>(target_pos, target_quat, q_init, q_init_stride, n, seeds, n_seeds, params, rot_thresh,
+                                     rot_weight, q_out, final_pos, final_quat, pos_err, rot_err, iters, flags, attempt,
+                                     counters, restart_stats, scratch, stream);
+}
+int pnp_ik_pose_solve_multistart_f64(const double* target_pos, const double* target_quat, const double* q_init,
+                                     int32_t q_init_stride, int64_t n, const double* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, double rot_thresh, double rot_weight, double* q_out,
+                                     double* final_pos, double* final_quat, double* pos_err, double* rot_err,
+                                     int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                     unsigned long long* restart_stats, void* scratch, void* stream) {
+  return pose_multistart_impl<double>(target_pos, target_quat, q_init, q_init_stride, n, seeds, n_seeds, params,
+                                      rot_thresh, rot_weight, q_out, final_pos, final_quat, pos_err, rot_err, iters, flags,
+                                      attempt, counters, restart_stats, scratch, stream);
 }
 
 int pnp_move_plan_order_f32(const float* q_start, const float* target, int64_t n, uint32_t* order, int32_t kinematics,

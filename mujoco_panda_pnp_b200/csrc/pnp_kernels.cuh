@@ -1071,10 +1071,14 @@ __global__ void __launch_bounds__(MS_COLLECT_BLOCK) ms_collect_kernel(const uint
   if (restart_stats && lane == 0 && c_fail) atomicAdd(restart_stats + 0, c_fail);
 }
 
-// The part of a wave both lane mappings share: pick the group's first success, store it, queue the unsolved queries.
-// `solve(valid, id, seed, out...)` runs one attempt per lane and stores nothing.
-template <typename T, int kOut, typename Solve, typename Store>
-__device__ __forceinline__ void ms_wave(const MsArgs<T>& m, unsigned cnt, Solve solve, Store store) {
+// The part of a wave every restart kernel shares (position: both lane mappings and layouts; pose): pick the group's
+// first success, store it, queue the unsolved queries.  `solve(valid, id, seed, out...)` runs one attempt per lane and
+// stores nothing; `prev(id, fl, it)` reads the flags and iteration count of the record being replaced (attempt 0's),
+// `store(id)` writes the lane's record.  M is MsArgs or MsPoseArgs: any argument block with the wave fields and the
+// attempt-0 arguments `a` (for a.counters).  Every solver counts success == converged, so the counter correction is
+// the same for all.
+template <typename M, typename Solve, typename Prev, typename Store>
+__device__ __forceinline__ void ms_wave(const M& m, unsigned cnt, Solve solve, Prev prev, Store store) {
   const unsigned lane = threadIdx.x & 31u;
   const unsigned G = m.group;
   const unsigned gl = lane & (G - 1u);
@@ -1101,14 +1105,7 @@ __device__ __forceinline__ void ms_wave(const MsArgs<T>& m, unsigned cnt, Solve 
     if (sb && lane == (unsigned)(__ffs(sb) - 1)) {
       // the record of attempt 0 leaves the returned set: correct the counters (which counted it) by the difference
       unsigned old_fl, old_it;
-      if (kOut == IK_OUT_SEPARATE) {
-        old_fl = m.a.flags[id];
-        old_it = (unsigned)m.iters0[id];
-      } else {
-        const unsigned w = reinterpret_cast<const unsigned*>(m.a.final_pos)[(size_t)id * 4u + 3u];
-        old_fl = w >> 24;
-        old_it = w & 0xFFFFFFu;
-      }
+      prev(id, old_fl, old_it);
       store(id);
       if (m.attempt) m.attempt[id] = (uint8_t)(seed + 1);
       c_conv += 1ull - (unsigned long long)(old_fl & PNP_IK_CONVERGED);
@@ -1142,6 +1139,19 @@ __device__ __forceinline__ void ms_wave(const MsArgs<T>& m, unsigned cnt, Solve 
   }
 }
 
+// flags and iterations of attempt 0's position record: flags[] / iters0[] (separate layout) or the packed word
+template <int kOut, typename T>
+__device__ __forceinline__ void ms_ik_prev(const MsArgs<T>& m, unsigned id, unsigned& fl, unsigned& it) {
+  if (kOut == IK_OUT_SEPARATE) {
+    fl = m.a.flags[id];
+    it = (unsigned)m.iters0[id];
+  } else {
+    const unsigned w = reinterpret_cast<const unsigned*>(m.a.final_pos)[(size_t)id * 4u + 3u];
+    fl = w >> 24;
+    it = w & 0xFFFFFFu;
+  }
+}
+
 // FP32 on the specialised tree: lane_solve + store_lane_result, i.e. ik_solve_small_kernel's arithmetic per lane
 template <int kOut>
 __global__ void __launch_bounds__(MS_BLOCK) ms_wave_v_kernel(const MsArgs<float> m) {
@@ -1165,7 +1175,7 @@ __global__ void __launch_bounds__(MS_BLOCK) ms_wave_v_kernel(const MsArgs<float>
     it_kept = iterations;
   };
   auto store = [&](unsigned id) { store_lane_result<kOut>(m.a, id, q, pf, n2f, it_kept, conv); };
-  ms_wave<float, kOut>(m, cnt, solve, store);
+  ms_wave(m, cnt, solve, [&](unsigned id, unsigned& fl, unsigned& it) { ms_ik_prev<kOut>(m, id, fl, it); }, store);
 }
 
 // FP32 on other trees and FP64: per lane the pass of ik_solve_kernel (ik_eval_and_step), no refill
@@ -1235,7 +1245,7 @@ __global__ void __launch_bounds__(MS_BLOCK) ms_wave_kernel(const MsArgs<T> m) {
       m.a.flags[id] = (uint8_t)fl;
     }
   };
-  ms_wave<T, kOut>(m, cnt, solve, store);
+  ms_wave(m, cnt, solve, [&](unsigned id, unsigned& fl, unsigned& it) { ms_ik_prev<kOut>(m, id, fl, it); }, store);
 }
 
 // =============================================================================================
@@ -1722,6 +1732,94 @@ __device__ __forceinline__ void ldlt_solve(T (&A)[N][N], T (&b)[N]) {
     for (int k = i + 1; k < N; ++k) b[i] -= A[k][i] * b[k];
 }
 
+// The three pieces of a pose solve that ik_pose_solve_kernel and the multistart restarts (ms_pose_wave_kernel) share,
+// so that a restart attempt runs the plain kernel's arithmetic bit for bit.
+// Target of query e: its position and its quaternion normalised on load.
+template <typename T>
+__device__ __forceinline__ void pose_load_target(const PoseIkArgs<T>& a, unsigned e, T (&tp)[3], T (&tq)[4]) {
+#pragma unroll
+  for (int i = 0; i < 3; ++i) tp[i] = a.target_pos[(size_t)e * 3 + i];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) tq[i] = a.target_quat[(size_t)e * 4 + i];
+  const T nq = sqrt_t(tq[0] * tq[0] + tq[1] * tq[1] + tq[2] * tq[2] + tq[3] * tq[3]);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) tq[i] = tq[i] / nq;
+}
+
+// One 6-row DLS pass at q (pass number `it`): evaluate the pose error and test convergence; a lane that is `active` and
+// finishes in this pass calls done(pp, qcur, pe, re, iterations, conv) with the pose and errors at the q it finished
+// at (q is still that q during the call).  Then q takes the DLS step - unconditionally: the caller discards the q of a
+// lane that has finished.
+template <typename T, typename Kin, typename Done>
+__device__ __forceinline__ void pose_pass(const PoseIkArgs<T>& a, const Trig<T>& trig, T (&q)[NJ], const T (&tp)[3],
+                                          const T (&tq)[4], int it, bool active, Done done) {
+  T s[NJ], c[NJ];
+#pragma unroll
+  for (int i = 0; i < NJ; ++i) trig(q[i] - Kin::template qref<T>(i), &s[i], &c[i]);
+  T pp[3], J[42], R[9], qcur[4];
+  Kin::template fk_full<T>(s, c, pp, J, R);
+  mat2quat_fast(R, qcur);
+  // err_quat = target (x) conj(current); rotation vector in the world frame
+  const T eq[4] = {tq[0] * qcur[0] + tq[1] * qcur[1] + tq[2] * qcur[2] + tq[3] * qcur[3],
+                   -tq[0] * qcur[1] + tq[1] * qcur[0] - tq[2] * qcur[3] + tq[3] * qcur[2],
+                   -tq[0] * qcur[2] + tq[1] * qcur[3] + tq[2] * qcur[0] - tq[3] * qcur[1],
+                   -tq[0] * qcur[3] - tq[1] * qcur[2] + tq[2] * qcur[1] + tq[3] * qcur[0]};
+  T rv[3];
+  quat2vel_fast(eq, rv);
+  T err[6] = {tp[0] - pp[0], tp[1] - pp[1], tp[2] - pp[2], rv[0] * a.rot_weight, rv[1] * a.rot_weight,
+              rv[2] * a.rot_weight};
+  const T pe = finish_sqrt((err[0] * err[0] + err[1] * err[1]) + err[2] * err[2]);
+  const T re = finish_sqrt((rv[0] * rv[0] + rv[1] * rv[1]) + rv[2] * rv[2]);
+  const bool last = it >= a.k.max_iters;
+  const bool conv = !last && (pe < a.k.pos_thresh) && (re < a.rot_thresh);
+  if (active && (conv || last)) done(pp, qcur, pe, re, conv ? it + 1 : it, conv);
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) { J[21 + j] *= a.rot_weight; J[28 + j] *= a.rot_weight; J[35 + j] *= a.rot_weight; }
+  T A[6][6];
+#pragma unroll
+  for (int r = 0; r < 6; ++r)
+#pragma unroll
+    for (int c2 = 0; c2 <= r; ++c2) {
+      T acc = T(0);
+#pragma unroll
+      for (int j = 0; j < NJ; ++j) acc = acc + J[r * 7 + j] * J[c2 * 7 + j];
+      A[r][c2] = acc + (r == c2 ? a.k.damping : T(0));
+    }
+  ldlt_solve<T, 6>(A, err);
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) {
+    T dq = T(0);
+#pragma unroll
+    for (int r = 0; r < 6; ++r) dq = dq + J[r * 7 + j] * err[r];
+    dq = clamp_t(dq, -a.k.step_limit, a.k.step_limit);
+    q[j] = clamp_t(q[j] + dq, Kin::template lower<T>(j), Kin::template upper<T>(j));
+  }
+}
+
+// the success rule of a finished pose solve
+template <typename T>
+__device__ __forceinline__ bool pose_success(const PoseIkArgs<T>& a, T pe, T re, bool conv) {
+  return conv && (pe < a.k.pos_thresh * T(2)) && (re < a.rot_thresh * T(2));
+}
+
+// Store the record of query e (every output but q_out nullable)
+template <typename T>
+__device__ __forceinline__ void pose_store(const PoseIkArgs<T>& a, unsigned e, const T (&q)[NJ], const T* pp,
+                                           const T* qcur, T pe, T re, int iterations, bool conv) {
+  const bool success = pose_success(a, pe, re, conv);
+#pragma unroll
+  for (int i = 0; i < NJ; ++i) a.q_out[(size_t)e * NJ + i] = q[i];
+  if (a.final_pos) { a.final_pos[(size_t)e * 3] = pp[0]; a.final_pos[(size_t)e * 3 + 1] = pp[1]; a.final_pos[(size_t)e * 3 + 2] = pp[2]; }
+  if (a.final_quat) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) a.final_quat[(size_t)e * 4 + i] = qcur[i];
+  }
+  if (a.pos_err) a.pos_err[e] = pe;
+  if (a.rot_err) a.rot_err[e] = re;
+  if (a.iters) a.iters[e] = iterations;
+  if (a.flags) a.flags[e] = (uint8_t)((conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u));
+}
+
 // Persistent warps with lane refill, like ik_solve_kernel: pose solves take 4-30 passes, and a grid of
 // one-shot lanes ran every warp at the pace of its slowest query (25.9 of 32 lanes active per
 // instruction, twice the mean pass count).  The FP32 instantiation uses the table trig.
@@ -1762,13 +1860,7 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArg
           const T* qi = a.q_init + (size_t)a.q_init_stride * e;
 #pragma unroll
           for (int i = 0; i < NJ; ++i) q[i] = qi[i];
-#pragma unroll
-          for (int i = 0; i < 3; ++i) tp[i] = a.target_pos[(size_t)e * 3 + i];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) tq[i] = a.target_quat[(size_t)e * 4 + i];
-          const T nq = sqrt_t(tq[0] * tq[0] + tq[1] * tq[1] + tq[2] * tq[2] + tq[3] * tq[3]);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) tq[i] = tq[i] / nq;
+          pose_load_target(a, e, tp, tq);
           it = 0;
           active = true;
         } else {
@@ -1780,65 +1872,13 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArg
     }
     if (!__any_sync(FULL, active)) break;
 
-    // ---- one 6-row DLS pass for all lanes --------------------------------------------------------
-    T s[NJ], c[NJ];
-#pragma unroll
-    for (int i = 0; i < NJ; ++i) trig(q[i] - Kin::template qref<T>(i), &s[i], &c[i]);
-    T pp[3], J[42], R[9], qcur[4];
-    Kin::template fk_full<T>(s, c, pp, J, R);
-    mat2quat_fast(R, qcur);
-    // err_quat = target (x) conj(current); rotation vector in the world frame
-    const T eq[4] = {tq[0] * qcur[0] + tq[1] * qcur[1] + tq[2] * qcur[2] + tq[3] * qcur[3],
-                     -tq[0] * qcur[1] + tq[1] * qcur[0] - tq[2] * qcur[3] + tq[3] * qcur[2],
-                     -tq[0] * qcur[2] + tq[1] * qcur[3] + tq[2] * qcur[0] - tq[3] * qcur[1],
-                     -tq[0] * qcur[3] - tq[1] * qcur[2] + tq[2] * qcur[1] + tq[3] * qcur[0]};
-    T rv[3];
-    quat2vel_fast(eq, rv);
-    T err[6] = {tp[0] - pp[0], tp[1] - pp[1], tp[2] - pp[2], rv[0] * a.rot_weight, rv[1] * a.rot_weight,
-                rv[2] * a.rot_weight};
-    const T pe = finish_sqrt((err[0] * err[0] + err[1] * err[1]) + err[2] * err[2]);
-    const T re = finish_sqrt((rv[0] * rv[0] + rv[1] * rv[1]) + rv[2] * rv[2]);
-    const bool last = it >= a.k.max_iters;
-    const bool conv = !last && (pe < a.k.pos_thresh) && (re < a.rot_thresh);
-    if (active && (conv || last)) {
-      const int iterations = conv ? it + 1 : it;
-      const bool success = conv && (pe < a.k.pos_thresh * T(2)) && (re < a.rot_thresh * T(2));
-#pragma unroll
-      for (int i = 0; i < NJ; ++i) a.q_out[(size_t)e * NJ + i] = q[i];
-      if (a.final_pos) { a.final_pos[(size_t)e * 3] = pp[0]; a.final_pos[(size_t)e * 3 + 1] = pp[1]; a.final_pos[(size_t)e * 3 + 2] = pp[2]; }
-      if (a.final_quat) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) a.final_quat[(size_t)e * 4 + i] = qcur[i];
-      }
-      if (a.pos_err) a.pos_err[e] = pe;
-      if (a.rot_err) a.rot_err[e] = re;
-      if (a.iters) a.iters[e] = iterations;
-      if (a.flags) a.flags[e] = (uint8_t)((conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u));
-      c_n += 1; c_conv += conv ? 1 : 0; c_iter += (unsigned long long)iterations;
-      active = false;
-    }
-    // unconditional update (a lane that just finished is idle and is overwritten by the next refill)
-#pragma unroll
-    for (int j = 0; j < NJ; ++j) { J[21 + j] *= a.rot_weight; J[28 + j] *= a.rot_weight; J[35 + j] *= a.rot_weight; }
-    T A[6][6];
-#pragma unroll
-    for (int r = 0; r < 6; ++r)
-#pragma unroll
-      for (int c2 = 0; c2 <= r; ++c2) {
-        T acc = T(0);
-#pragma unroll
-        for (int j = 0; j < NJ; ++j) acc = acc + J[r * 7 + j] * J[c2 * 7 + j];
-        A[r][c2] = acc + (r == c2 ? a.k.damping : T(0));
-      }
-    ldlt_solve<T, 6>(A, err);
-#pragma unroll
-    for (int j = 0; j < NJ; ++j) {
-      T dq = T(0);
-#pragma unroll
-      for (int r = 0; r < 6; ++r) dq = dq + J[r * 7 + j] * err[r];
-      dq = clamp_t(dq, -a.k.step_limit, a.k.step_limit);
-      q[j] = clamp_t(q[j] + dq, Kin::template lower<T>(j), Kin::template upper<T>(j));
-    }
+    // ---- one 6-row DLS pass for all lanes (a lane that just finished is idle and is overwritten by the next refill) --
+    pose_pass<T, Kin>(a, trig, q, tp, tq, it, active,
+                      [&](const T* pp, const T* qcur, T pe, T re, int iterations, bool conv) {
+                        pose_store(a, e, q, pp, qcur, pe, re, iterations, conv);
+                        c_n += 1; c_conv += conv ? 1 : 0; c_iter += (unsigned long long)iterations;
+                        active = false;
+                      });
     ++it;
   }
   if (a.counters) {
@@ -1850,6 +1890,71 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArg
       atomicAdd(a.counters + PNP_IK_CNT_ITERATIONS, c_iter);
     }
   }
+}
+
+// ---- multi-start pose IK (pnp_ik_pose_solve_multistart_*) ---------------------------------------------------------
+// The position multistart's machinery (ms_collect_kernel, ms_wave) on the pose solve: attempt 0 is
+// ik_pose_solve_kernel; the collect kernel lists the queries whose flags[] lack PNP_IK_SUCCESS; wave w gives each listed
+// query G lanes that run seeds [w G, w G + G) with pose_pass, the plain kernel's pass, from pose_load_target's target.
+// The lowest successful lane of a group stores the record with pose_store (every output the caller passed) and the
+// attempt; queries without a success go onto the next wave's list.
+template <typename T>
+struct MsPoseArgs {
+  PoseIkArgs<T> a;         // targets, solver constants and the outputs of attempt 0
+  const T* seeds;          // [n_seeds][7]
+  int n_seeds;
+  int wave;                // this launch runs seeds [wave * group, wave * group + group)
+  unsigned group;          // lanes per query: a power of two <= 32
+  const unsigned* list_in;
+  const unsigned* cnt_in;
+  unsigned* list_out;      // nullptr: last wave
+  unsigned* cnt_out;
+  const int32_t* iters0;   // iterations of attempt 0 (the iters output or scratch)
+  uint8_t* attempt;        // nullable
+  unsigned long long* restart_stats;  // nullable: restarted, rescued, DLS passes of restart attempts
+};
+
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(MS_BLOCK) ms_pose_wave_kernel(const MsPoseArgs<T> m) {
+  const unsigned cnt = *m.cnt_in;
+  if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;  // no work for any warp of this block
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  const Trig<T> trig{s_tab};
+  // the finished attempt of this lane: q, pose and errors at the pass it finished in
+  T qk[NJ], pk[3], qck[4], pek = T(0), rek = T(0);
+  bool conv = false;
+  int it_kept = 0;
+  auto solve = [&](bool valid, unsigned id, int seed, bool& succ, int& iterations) {
+    T q[NJ], tp[3], tq[4];
+    pose_load_target(m.a, id, tp, tq);
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) q[i] = m.seeds[seed * NJ + i];
+    bool active = valid;
+    conv = false;
+    it_kept = 0;
+    for (int it = 0; __any_sync(FULL, active); ++it)
+      pose_pass<T, Kin>(m.a, trig, q, tp, tq, it, active,
+                        [&](const T* pp, const T* qcur, T pe, T re, int its, bool cv) {
+#pragma unroll
+                          for (int i = 0; i < NJ; ++i) qk[i] = q[i];
+#pragma unroll
+                          for (int i = 0; i < 3; ++i) pk[i] = pp[i];
+#pragma unroll
+                          for (int i = 0; i < 4; ++i) qck[i] = qcur[i];
+                          pek = pe; rek = re; it_kept = its; conv = cv;
+                          active = false;
+                        });
+    iterations = it_kept;
+    succ = pose_success(m.a, pek, rek, conv);
+  };
+  auto prev = [&](unsigned id, unsigned& fl, unsigned& it) {
+    fl = m.a.flags[id];
+    it = (unsigned)m.iters0[id];
+  };
+  auto store = [&](unsigned id) { pose_store(m.a, id, qk, pk, qck, pek, rek, it_kept, conv); };
+  ms_wave(m, cnt, solve, prev, store);
 }
 
 // =============================================================================================

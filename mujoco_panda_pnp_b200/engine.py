@@ -425,6 +425,66 @@ def ik_pose_solve(target_pos: torch.Tensor, target_quat: torch.Tensor, q_init: t
                 converged=(flags & 1) != 0, success=(flags & 2) != 0)
 
 
+def ik_pose_solve_multistart(target_pos: torch.Tensor, target_quat: torch.Tensor, q_init: torch.Tensor,
+                             seeds: torch.Tensor, params: PnpIkParams, rot_thresh: float = 1e-2, rot_weight: float = 1.0,
+                             counters: Optional[torch.Tensor] = None,
+                             restart_stats: Optional[torch.Tensor] = None) -> dict:
+    """ik_pose_solve, then every query it did not solve is solved again from the rows of ``seeds`` (K, 7), in order,
+    until one succeeds (pnp_ik_pose_solve_multistart_*).  Each row of the result is, bit for bit, the plain
+    ik_pose_solve of that target from the start ``attempt`` names (0 = q_init, k = seeds[k - 1]); rows no attempt
+    solves keep attempt 0.  Returns ik_pose_solve's dict plus ``attempt`` (uint8[N]).
+
+    ``counters`` (int64[4]) accumulates over the returned rows like ik_pose_solve's; ``restart_stats`` (int64[3])
+    accumulates queries restarted, queries rescued and DLS passes spent on restarts.  Never synchronises."""
+    lib = _lib.load()
+    dt = target_pos.dtype
+    if dt not in (torch.float32, torch.float64):
+        raise ValueError("target_pos must be float32 or float64")
+    target_pos = _check_cuda("target_pos", target_pos, dt, (3,))
+    target_quat = _check_cuda("target_quat", target_quat, dt, (4,))
+    n = target_pos.shape[0]
+    if target_quat.shape[0] != n:
+        raise ValueError("target_pos and target_quat disagree on N")
+    dev = target_pos.device
+    if q_init.dim() == 1:
+        if q_init.shape != (7,):
+            raise ValueError("broadcast q_init must have shape (7,)")
+        q_init, stride = q_init.to(device=dev, dtype=dt).contiguous(), 0
+    else:
+        q_init, stride = _check_cuda("q_init", q_init, dt, (7,)), 7
+        if q_init.shape[0] != n:
+            raise ValueError("q_init disagrees with target_pos on N")
+    seeds = torch.as_tensor(seeds).to(device=dev, dtype=dt).reshape(-1, 7).contiguous()
+    k = seeds.shape[0]
+    if k > 255:
+        raise ValueError(f"at most 255 seeds, got {k}")
+    for name, t, m in (("counters", counters, 4), ("restart_stats", restart_stats, 3)):
+        if t is not None and (t.dtype != torch.int64 or t.numel() < m or not t.is_cuda):
+            raise ValueError(f"{name} must be a CUDA int64 tensor with >= {m} elements")
+    nbytes = ctypes.c_int64()
+    _lib.check(lib.pnp_ik_multistart_scratch_bytes(n, ctypes.byref(nbytes)), "pnp_ik_multistart_scratch_bytes")
+    fn = lib.pnp_ik_pose_solve_multistart_f32 if dt == torch.float32 else lib.pnp_ik_pose_solve_multistart_f64
+    with torch.cuda.device(dev):
+        scratch = torch.empty(((nbytes.value + 15) // 16, 4), dtype=torch.int32, device=dev)
+        attempt = torch.empty((n,), dtype=torch.uint8, device=dev)
+        q = torch.empty((n, 7), dtype=dt, device=dev)
+        fpos = torch.empty((n, 3), dtype=dt, device=dev)
+        fquat = torch.empty((n, 4), dtype=dt, device=dev)
+        perr = torch.empty((n,), dtype=dt, device=dev)
+        rerr = torch.empty((n,), dtype=dt, device=dev)
+        iters = torch.empty((n,), dtype=torch.int32, device=dev)
+        flags = torch.empty((n,), dtype=torch.uint8, device=dev)
+        _lib.check(
+            fn(_ptr(target_pos), _ptr(target_quat), _ptr(q_init), stride, n, _ptr(seeds), k, ctypes.byref(params),
+               float(rot_thresh), float(rot_weight), _ptr(q), _ptr(fpos), _ptr(fquat), _ptr(perr), _ptr(rerr),
+               _ptr(iters), _ptr(flags), _ptr(attempt), _ptr(counters), _ptr(restart_stats), _ptr(scratch),
+               _stream()),
+            "pnp_ik_pose_solve_multistart",
+        )
+    return dict(q=q, final_pos=fpos, final_quat=fquat, pos_error=perr, rot_error=rerr, iterations=iters,
+                converged=(flags & 1) != 0, success=(flags & 2) != 0, attempt=attempt)
+
+
 PLAN_ORDER_MIN = 1 << 16  # below this a launch has fewer envs than lanes: nothing to balance (2^14 measured slower)
 
 

@@ -153,19 +153,27 @@ class JacobianIKController:
 
     def solve_pose(self, target_pos, target_quat, q_init, max_iters: int = 100, pos_thresh: float = 1e-3,
                    rot_thresh: float = 1e-2, damping: float = 1e-2, step_limit: float = 0.1,
-                   rot_weight: float = 1.0) -> dict:
+                   rot_weight: float = 1.0, seeds=None) -> dict:
         """Pose-mode IK (EXTENSION, no reference counterpart: see pnp_ik_pose_solve_* in
         include/pnp_b200.h).  target_pos (3,)|(N,3), target_quat wxyz (4,)|(N,4), q_init (7,)|(N,7).
         Returns a dict of device tensors (batched) with q, final_pos, final_quat, pos_error,
-        rot_error, iterations, converged, success."""
+        rot_error, iterations, converged, success.
+
+        ``seeds`` (K, 7), K <= 255 (e.g. ``engine.ik_restart_seeds(8)``): every query the solve from ``q_init`` does not
+        solve is solved again from seeds[0], seeds[1], ... until one succeeds (engine.ik_pose_solve_multistart); the
+        dict then also holds ``attempt`` (0 = from q_init, k = from seeds[k - 1])."""
         dt = self._dtype()
         with torch.cuda.device(self.device):
             engine.set_tree(self.tree)
             tp = _to_tensor(target_pos).to(device=self.device, dtype=dt).reshape(-1, 3)
             tq = _to_tensor(target_quat).to(device=self.device, dtype=dt).reshape(-1, 4)
             qi = _to_tensor(q_init).to(device=self.device, dtype=dt)
-            return engine.ik_pose_solve(tp, tq, qi, self._params(max_iters, pos_thresh, damping, step_limit),
-                                        rot_thresh=rot_thresh, rot_weight=rot_weight)
+            params = self._params(max_iters, pos_thresh, damping, step_limit)
+            if seeds is not None:
+                sd = _to_tensor(seeds).to(device=self.device, dtype=dt)
+                return engine.ik_pose_solve_multistart(tp, tq, qi, sd, params, rot_thresh=rot_thresh,
+                                                       rot_weight=rot_weight)
+            return engine.ik_pose_solve(tp, tq, qi, params, rot_thresh=rot_thresh, rot_weight=rot_weight)
 
     def _write_back(self, q: np.ndarray, final_pos: np.ndarray) -> None:
         d = self.data
@@ -198,11 +206,15 @@ def _mujoco_module():
 IKSolver = JacobianIKController  # north_star calls the class IKSolver (SURVEY.md D1)
 
 
-def solve_ik(model, data, site_name, target_pos, target_quat, q_init):
+def solve_ik(model, data, site_name, target_pos, target_quat, q_init, seeds=None):
     """The function FrankaEnv.solve_ik tries to import (envs/panda_env.py:399-409) and the reference
-    never defined.  Pose-mode DLS IK on the GPU; returns an IKResult for the single query."""
+    never defined.  Pose-mode DLS IK on the GPU; returns an IKResult for the single query.
+
+    ``seeds`` (K, 7), an extension: when the solve from ``q_init`` fails, retry from each seed in turn and return the
+    first success (JacobianIKController.solve_pose)."""
     ctl = JacobianIKController(model, data, site_name)
-    r = ctl.solve_pose(np.asarray(target_pos, float), np.asarray(target_quat, float), np.asarray(q_init, float))
+    r = ctl.solve_pose(np.asarray(target_pos, float), np.asarray(target_quat, float), np.asarray(q_init, float),
+                       seeds=seeds)
     q = r["q"][0].double().cpu().numpy()
     final_pos = r["final_pos"][0].double().cpu().numpy()
     ctl._write_back(q, final_pos)

@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <mutex>
 #include <string>
 #include <type_traits>
@@ -61,7 +62,6 @@ struct DeviceState {
   bool slot_used[kStreamSlots] = {};
   unsigned slot_clock = 0;
   int occ_ik[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  int occ_ms[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};  // restart wave kernels of the multistart solves (position, pose)
   bool obs_smem_set = false;
   bool fk_smem_set = false;
   bool plan_smem_set = false;
@@ -91,6 +91,7 @@ int stream_slot(DeviceState* s, cudaStream_t st) {
   std::lock_guard<std::mutex> lk(g_mu);
   return stream_slot_locked(s, st);
 }
+ByteRange byte_range(const void* p, size_t bytes) { ByteRange r; if (p) { r.b = (const char*)p; r.e = r.b + bytes; } return r; }
 bool ranges_overlap(const ByteRange& x, const ByteRange& y) { return x.b && y.b && x.b < y.e && y.b < x.e; }
 
 int fail(int code, const char* fmt, ...) {
@@ -398,16 +399,15 @@ int launch_ik_v(DeviceState* s, const pnp::IkArgs<float>& a, bool small, cudaStr
   }
   // what this launch reads and writes
   ByteRange in[2], out[5];
-  auto range = [](const void* p, size_t bytes) { ByteRange r; if (p) { r.b = (const char*)p; r.e = r.b + bytes; } return r; };
   const size_t n = a.n;
-  in[0] = range(a.targets, n * 12);
-  in[1] = range(a.q_init, a.q_init_stride ? n * 28 : 28);
+  in[0] = byte_range(a.targets, n * 12);
+  in[1] = byte_range(a.q_init, a.q_init_stride ? n * 28 : 28);
   if (kOut == pnp::IK_OUT_SEPARATE) {
-    out[0] = range(a.q_out, n * 28); out[1] = range(a.final_pos, n * 12); out[2] = range(a.pos_err, n * 4);
-    out[3] = range(a.iters, n * 4); out[4] = range(a.flags, n);
+    out[0] = byte_range(a.q_out, n * 28); out[1] = byte_range(a.final_pos, n * 12); out[2] = byte_range(a.pos_err, n * 4);
+    out[3] = byte_range(a.iters, n * 4); out[4] = byte_range(a.flags, n);
   } else {
-    out[0] = range(a.q_out, n * 32);
-    if (kOut == pnp::IK_OUT_PACKED) out[1] = range(a.final_pos, n * 16);
+    out[0] = byte_range(a.q_out, n * 32);
+    if (kOut == pnp::IK_OUT_PACKED) out[1] = byte_range(a.final_pos, n * 16);
   }
   bool clash = false;  // with the previous launch of this stream, which may still be draining when this one starts
   if (ps.primed) {
@@ -526,7 +526,7 @@ int launch_ik_spec_f32(DeviceState* s, const pnp::IkArgs<float>& a, int kinemati
 template <typename T, int kOut>
 int ik_solve_impl(const T* targets, const T* q_init, int32_t q_init_stride, int64_t n, const PnpIkParams* params,
                   T* q_out, T* final_pos, T* pos_err, int32_t* iters, uint8_t* flags, unsigned long long* counters,
-                  void* stream) {
+                  void* stream, pnp::IkArgs<T>* args_out = nullptr) {
   int rc = check_ik_params(params);
   if (rc) return rc;
   if (n < 0 || (n > 0 && (!targets || !q_init || !q_out))) return fail(PNP_EINVAL, "ik_solve: null pointer or negative n");
@@ -552,6 +552,7 @@ int ik_solve_impl(const T* targets, const T* q_init, int32_t q_init_stride, int6
   a.park_dump = nullptr; a.park_list = nullptr; a.park_lanes = nullptr; a.park_slots = nullptr;
   a.zero_next[0] = a.zero_next[1] = a.zero_next[2] = nullptr;
   a.thresh2 = a.k.pos_thresh * a.k.pos_thresh;
+  if (args_out) *args_out = a;  // the multistart's restarts use this block
   const bool small = n <= (long long)s->sm_count * pnp::IK_BLOCK;
   if constexpr (std::is_same<T, float>::value) {
     // the latency kernel needs no ticket: skip the memset node as well
@@ -572,68 +573,75 @@ int ik_solve_impl(const T* targets, const T* q_init, int32_t q_init_stride, int6
   return launch_ik<T, pnp::GenericKin, kOut>(s, a, small, st);
 }
 
-// ---- multistart (see ms_collect_kernel / ms_wave_* in pnp_kernels.cuh) ----------------------------------------------
-// Lanes per restarted query: the seeds a wave runs in parallel.  A wave lasts as long as its slowest attempt (up to
-// max_iters passes) whatever its width, so fewer, wider waves cost less until the lanes no longer fit the SMs at once;
-// see DESIGN.md 4.1 for the measurement.  PNP_MS_GROUP overrides it (1, 2, 4 or 8), for measurements.
+// ---- multistart (see ms_collect_kernel / ms_wave* in pnp_kernels.cuh) ----------------------------------------------
+// Lanes per restarted query: the seeds a wave runs in parallel.
+// Position solver: a wave lasts as long as its slowest attempt (up to max_iters passes) whatever its width, so fewer,
+// wider waves cost less until the lanes no longer fit the SMs at once; see DESIGN.md 4.1 for the measurement.
+// PNP_MS_GROUP overrides it (1, 2, 4 or 8), for measurements.
 constexpr int kMsGroup = 4;
+// Pose solver: about a quarter of a cold workspace batch enters the first wave, and a failing attempt runs all
+// max_iters passes, so a wave costs about its lane count times max_iters: the narrowest group, which spends no attempt
+// on a query an earlier seed already rescues, measured fastest (DESIGN.md 4.6: 2^22 W-cold poses with 8 seeds in
+// 14.7 ms at G = 1, 16.0 / 20.3 / 30.8 ms at G = 2 / 4 / 8).  PNP_MS_POSE_GROUP overrides it (1, 2, 4 or 8), for
+// measurements.
+constexpr int kMsPoseGroup = 1;
 constexpr size_t kMsHdrBytes = pnp::MS_HDR_WORDS * sizeof(unsigned);
 size_t ms_list_bytes(int64_t n) { return ((size_t)n * sizeof(unsigned) + 15u) & ~(size_t)15u; }
 // header | list A | list B | iterations of attempt 0 (separate layout without an iters output)
 size_t ms_scratch_bytes(int64_t n) { return kMsHdrBytes + 3 * ms_list_bytes(n); }
 
-template <typename K, typename M>
-int launch_ms_wave(DeviceState* s, K kernel, int occ_slot, const M& m, cudaStream_t st) {
-  if (s->occ_ms[occ_slot] == 0) {
-    int occ = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, pnp::MS_BLOCK, 0);
-    s->occ_ms[occ_slot] = (e == cudaSuccess && occ > 0) ? occ : 1;
+// one restart wave; the occupancy of each wave kernel is queried once per device
+template <auto kKernel, typename M>
+int launch_ms_wave(DeviceState* s, const M& m, cudaStream_t st) {
+  static int occ_of_device[kMaxDevices] = {};
+  int& occ = occ_of_device[s - g_dev];
+  if (occ == 0) {
+    int o = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, kKernel, pnp::MS_BLOCK, 0);
+    occ = (e == cudaSuccess && o > 0) ? o : 1;
   }
-  kernel<<<s->sm_count * s->occ_ms[occ_slot], pnp::MS_BLOCK, 0, st>>>(m);
+  kKernel<<<s->sm_count * occ, pnp::MS_BLOCK, 0, st>>>(m);
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return PNP_OK;
 }
 
-template <typename T, int kOut>
-int ik_multistart_impl(const T* targets, const T* q_init, int32_t q_init_stride, int64_t n, const T* seeds, int32_t n_seeds,
-                       const PnpIkParams* params, T* q_out, T* final_pos, T* pos_err, int32_t* iters, uint8_t* flags,
-                       uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats, void* scratch,
-                       void* stream) {
-  if (n_seeds < 0 || n_seeds > pnp::MS_MAX_SEEDS) return fail(PNP_EINVAL, "ik_multistart: n_seeds must be in [0, 255]");
-  if (n_seeds > 0 && !seeds) return fail(PNP_EINVAL, "ik_multistart: seeds is NULL");
-  if (!scratch || !aligned16(scratch)) return fail(PNP_EINVAL, "ik_multistart: scratch must be non-null and 16-byte aligned");
-  if (kOut == pnp::IK_OUT_SEPARATE && n > 0 && !flags)
-    return fail(PNP_EINVAL, "ik_multistart: flags must be non-null (the restarts read attempt 0's success from it)");
+// The multistart of either solver; A is its argument block (IkArgs<T>, PoseIkArgs<T>), `who` names it in messages.
+// kCollect is where attempt 0's success and iterations are read: IK_OUT_SEPARATE (flags[] required, iterations from
+// iters or scratch) or IK_OUT_PACKED (the packed word of a.final_pos).  `outputs` are the byte ranges of the solver's
+// outputs.  attempt0(iters0, a) runs the plain solve with iters0 as its iterations output and leaves its argument
+// block in `a`; wave(s, spec, m, st) launches the restart kernel of one wave.  Every argument is checked before the
+// first launch.
+template <typename A, int kCollect, typename T, typename Attempt0, typename Wave>
+int multistart_impl(const char* who, int64_t n, const T* seeds, int32_t n_seeds, const PnpIkParams* params,
+                    const uint8_t* flags, int32_t* iters, uint8_t* attempt, unsigned long long* counters,
+                    unsigned long long* restart_stats, void* scratch, std::initializer_list<ByteRange> outputs,
+                    int group_default, const char* group_env, void* stream, Attempt0 attempt0, Wave wave) {
+  if (n_seeds < 0 || n_seeds > pnp::MS_MAX_SEEDS) return fail(PNP_EINVAL, "%s: n_seeds must be in [0, 255]", who);
+  if (n_seeds > 0 && !seeds) return fail(PNP_EINVAL, "%s: seeds is NULL", who);
+  if (!scratch || !aligned16(scratch)) return fail(PNP_EINVAL, "%s: scratch must be non-null and 16-byte aligned", who);
+  if (kCollect == pnp::IK_OUT_SEPARATE && n > 0 && !flags)
+    return fail(PNP_EINVAL, "%s: flags must be non-null (the restarts read attempt 0's success from it)", who);
   if (n > 0) {
-    // seeds (read by every wave) and scratch (written) must not share memory with an output
-    auto range = [](const void* p, size_t bytes) { ByteRange r; if (p) { r.b = (const char*)p; r.e = r.b + bytes; } return r; };
-    const size_t m = (size_t)n;
-    const ByteRange in[2] = {range(seeds, (size_t)n_seeds * PNP_NJOINT * sizeof(T)), range(scratch, ms_scratch_bytes(n))};
-    ByteRange out[8];
-    if (kOut == pnp::IK_OUT_SEPARATE) {
-      out[0] = range(q_out, m * PNP_NJOINT * sizeof(T)); out[1] = range(final_pos, m * 3 * sizeof(T));
-      out[2] = range(pos_err, m * sizeof(T)); out[3] = range(iters, m * sizeof(int32_t)); out[4] = range(flags, m);
-    } else {
-      out[0] = range(q_out, m * 8 * sizeof(float)); out[1] = range(final_pos, m * 4 * sizeof(float));
-    }
-    out[5] = range(attempt, m);
-    out[6] = range(counters, 4 * sizeof(unsigned long long));
-    out[7] = range(restart_stats, 3 * sizeof(unsigned long long));
-    for (const ByteRange& o : out)
-      if (ranges_overlap(o, in[0]) || ranges_overlap(o, in[1]))
-        return fail(PNP_EINVAL, "ik_multistart: seeds and scratch must not overlap an output");
-    if (ranges_overlap(in[0], in[1])) return fail(PNP_EINVAL, "ik_multistart: seeds and scratch must not overlap");
+    // seeds (read by every wave) and scratch (written) must not share memory with an output or with each other
+    const ByteRange in[2] = {byte_range(seeds, (size_t)n_seeds * PNP_NJOINT * sizeof(T)), byte_range(scratch, ms_scratch_bytes(n))};
+    const ByteRange more[3] = {byte_range(attempt, (size_t)n), byte_range(counters, 4 * sizeof(unsigned long long)),
+                               byte_range(restart_stats, 3 * sizeof(unsigned long long))};
+    bool clash = false;
+    for (const ByteRange& o : outputs) clash = clash || ranges_overlap(o, in[0]) || ranges_overlap(o, in[1]);
+    for (const ByteRange& o : more) clash = clash || ranges_overlap(o, in[0]) || ranges_overlap(o, in[1]);
+    if (clash) return fail(PNP_EINVAL, "%s: seeds and scratch must not overlap an output", who);
+    if (ranges_overlap(in[0], in[1])) return fail(PNP_EINVAL, "%s: seeds and scratch must not overlap", who);
   }
   unsigned* hdr = static_cast<unsigned*>(scratch);
   unsigned* list[2] = {reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes),
                        reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes + ms_list_bytes(n))};
   int32_t* iters0 = iters;
-  if (kOut == pnp::IK_OUT_SEPARATE && !iters0 && n_seeds > 0)  // the restarts need attempt 0's iterations for the counters
+  if (kCollect == pnp::IK_OUT_SEPARATE && !iters0 && n_seeds > 0)  // the restarts need attempt 0's iterations for the counters
     iters0 = reinterpret_cast<int32_t*>((char*)scratch + kMsHdrBytes + 2 * ms_list_bytes(n));
   // attempt 0: the plain entry point, unchanged
-  int rc = ik_solve_impl<T, kOut>(targets, q_init, q_init_stride, n, params, q_out, final_pos, pos_err, iters0, flags, counters,
-                                  stream);
+  pnp::MsArgs<A> m;
+  int rc = attempt0(iters0, m.a);
   if (rc || n == 0) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   if (attempt) CUDA_TRY(cudaMemsetAsync(attempt, 0, (size_t)n, st));
@@ -646,20 +654,14 @@ int ik_multistart_impl(const T* targets, const T* q_init, int32_t q_init_stride,
   CUDA_TRY(cudaMemsetAsync(hdr, 0, kMsHdrBytes, st));
   {
     const int grid = grid_for(n, pnp::MS_COLLECT_BLOCK, s->sm_count, 8);
-    pnp::ms_collect_kernel<kOut><<<grid, pnp::MS_COLLECT_BLOCK, 0, st>>>(
-        flags, reinterpret_cast<const unsigned*>(final_pos), (unsigned)n, list[0], hdr, restart_stats);
+    const unsigned* aux_words = kCollect == pnp::IK_OUT_SEPARATE ? nullptr : reinterpret_cast<const unsigned*>(m.a.final_pos);
+    pnp::ms_collect_kernel<kCollect><<<grid, pnp::MS_COLLECT_BLOCK, 0, st>>>(m.a.flags, aux_words, (unsigned)n, list[0],
+                                                                              hdr, restart_stats);
     ++g_launches;
     CUDA_TRY(cudaGetLastError());
   }
-  static const int env_group = env_int("PNP_MS_GROUP", 0);
-  const int G = (env_group == 1 || env_group == 2 || env_group == 4 || env_group == 8) ? env_group : kMsGroup;
-  pnp::MsArgs<T> m;
-  pnp::IkArgs<T>& a = m.a;
-  memset(&a, 0, sizeof a);
-  a.targets = targets; a.q_init = q_init; a.q_init_stride = q_init_stride; a.n = (unsigned)n;
-  a.k = make_ik_const<T>(params);
-  a.q_out = q_out; a.final_pos = final_pos; a.pos_err = pos_err; a.iters = iters0; a.flags = flags; a.counters = counters;
-  a.thresh2 = a.k.pos_thresh * a.k.pos_thresh;
+  static const int env_group = env_int(group_env, 0);  // (one instantiation per solver and layout: one variable each)
+  const int G = (env_group == 1 || env_group == 2 || env_group == 4 || env_group == 8) ? env_group : group_default;
   m.seeds = seeds; m.n_seeds = n_seeds; m.group = (unsigned)G;
   m.iters0 = iters0; m.attempt = attempt; m.restart_stats = restart_stats;
   const int waves = (n_seeds + G - 1) / G;
@@ -667,18 +669,37 @@ int ik_multistart_impl(const T* targets, const T* q_init, int32_t q_init_stride,
     m.wave = w;
     m.list_in = list[w & 1]; m.cnt_in = hdr + w;
     m.list_out = w + 1 < waves ? list[(w + 1) & 1] : nullptr; m.cnt_out = hdr + w + 1;
-    if constexpr (std::is_same<T, float>::value) {
-      if (spec && params->kinematics != PNP_KIN_GENERIC)
-        rc = launch_ms_wave(s, pnp::ms_wave_v_kernel<kOut>, kOut == pnp::IK_OUT_SEPARATE ? 0 : 1, m, st);
-      else
-        rc = launch_ms_wave(s, pnp::ms_wave_kernel<float, pnp::GenericKin, kOut>, kOut == pnp::IK_OUT_SEPARATE ? 2 : 3, m, st);
-    } else {
-      rc = spec ? launch_ms_wave(s, pnp::ms_wave_kernel<double, pnp::SpecKin, kOut>, 4, m, st)
-                : launch_ms_wave(s, pnp::ms_wave_kernel<double, pnp::GenericKin, kOut>, 5, m, st);
-    }
-    if (rc) return rc;
+    if ((rc = wave(s, spec, m, st))) return rc;
   }
   return PNP_OK;
+}
+
+template <typename T, int kOut>
+int ik_multistart_impl(const T* targets, const T* q_init, int32_t q_init_stride, int64_t n, const T* seeds, int32_t n_seeds,
+                       const PnpIkParams* params, T* q_out, T* final_pos, T* pos_err, int32_t* iters, uint8_t* flags,
+                       uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats, void* scratch,
+                       void* stream) {
+  const size_t m = (size_t)n;
+  const bool sep = kOut == pnp::IK_OUT_SEPARATE;  // else packed: out_q8 in q_out, out_aux4 in final_pos
+  return multistart_impl<pnp::IkArgs<T>, kOut>(
+      "ik_multistart", n, seeds, n_seeds, params, flags, iters, attempt, counters, restart_stats, scratch,
+      {byte_range(q_out, m * (sep ? PNP_NJOINT * sizeof(T) : 8 * sizeof(float))),
+       byte_range(final_pos, m * (sep ? 3 * sizeof(T) : 4 * sizeof(float))), byte_range(pos_err, m * sizeof(T)),
+       byte_range(iters, m * sizeof(int32_t)), byte_range(flags, m)},
+      kMsGroup, "PNP_MS_GROUP", stream,
+      [&](int32_t* iters0, pnp::IkArgs<T>& a) {
+        return ik_solve_impl<T, kOut>(targets, q_init, q_init_stride, n, params, q_out, final_pos, pos_err, iters0, flags,
+                                      counters, stream, &a);
+      },
+      [&](DeviceState* s, bool spec, const auto& m, cudaStream_t st) {
+        if constexpr (std::is_same<T, float>::value) {
+          if (spec && params->kinematics != PNP_KIN_GENERIC) return launch_ms_wave<pnp::ms_wave_v_kernel<kOut>>(s, m, st);
+          return launch_ms_wave<pnp::ms_wave_kernel<float, pnp::GenericKin, kOut>>(s, m, st);
+        } else {
+          return spec ? launch_ms_wave<pnp::ms_wave_kernel<double, pnp::SpecKin, kOut>>(s, m, st)
+                      : launch_ms_wave<pnp::ms_wave_kernel<double, pnp::GenericKin, kOut>>(s, m, st);
+        }
+      });
 }
 
 // Smallest double s >= 0 with sqrt(s) >= t (sqrt is correctly rounded, hence monotone): the
@@ -965,7 +986,7 @@ template <typename T>
 int pose_solve_impl(const T* tpos, const T* tquat, const T* q_init, int32_t q_init_stride, int64_t n,
                     const PnpIkParams* params, double rot_thresh, double rot_weight, T* q_out, T* final_pos,
                     T* final_quat, T* pos_err, T* rot_err, int32_t* iters, uint8_t* flags,
-                    unsigned long long* counters, void* stream) {
+                    unsigned long long* counters, void* stream, pnp::PoseIkArgs<T>* args_out = nullptr) {
   int rc = check_ik_params(params);
   if (rc) return rc;
   if (!(rot_thresh > 0.0) || !(rot_weight > 0.0)) return fail(PNP_EINVAL, "rot_thresh and rot_weight must be > 0");
@@ -1000,6 +1021,7 @@ int pose_solve_impl(const T* tpos, const T* tquat, const T* q_init, int32_t q_in
   chunk = chunk < 32 ? 32 : (chunk > 256 ? 256 : chunk);
   a.chunk = (unsigned)(chunk & ~31ll);
   a.solo_warp = small ? 1u : 0u;
+  if (args_out) *args_out = a;  // the multistart's restarts use this block
   if (spec)
     pnp::ik_pose_solve_kernel<T, pnp::SpecKin><<<grid, block, 0, st>>>(a);
   else
@@ -1009,90 +1031,28 @@ int pose_solve_impl(const T* tpos, const T* tquat, const T* q_init, int32_t q_in
   return PNP_OK;
 }
 
-// Multi-start pose solve: pose_solve_impl, then the restart waves of ms_pose_wave_kernel (see ik_multistart_impl).
-// Lanes per restarted query.  About a quarter of a cold workspace batch enters the first wave, and a failing attempt
-// runs all max_iters passes, so a wave costs about its lane count times max_iters: the narrowest group, which spends
-// no attempt on a query an earlier seed already rescues, measured fastest (DESIGN.md 4.6: 2^22 W-cold poses with 8
-// seeds in 14.7 ms at G = 1, 16.0 / 20.3 / 30.8 ms at G = 2 / 4 / 8).  PNP_MS_POSE_GROUP overrides it (1, 2, 4 or 8), for
-// measurements.
-constexpr int kMsPoseGroup = 1;
-
+// Multi-start pose solve: pose_solve_impl, then the restart waves of ms_pose_wave_kernel (see multistart_impl).
 template <typename T>
 int pose_multistart_impl(const T* tpos, const T* tquat, const T* q_init, int32_t q_init_stride, int64_t n, const T* seeds,
                          int32_t n_seeds, const PnpIkParams* params, double rot_thresh, double rot_weight, T* q_out,
                          T* final_pos, T* final_quat, T* pos_err, T* rot_err, int32_t* iters, uint8_t* flags,
                          uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats, void* scratch,
                          void* stream) {
-  if (n_seeds < 0 || n_seeds > pnp::MS_MAX_SEEDS) return fail(PNP_EINVAL, "ik_pose_multistart: n_seeds must be in [0, 255]");
-  if (n_seeds > 0 && !seeds) return fail(PNP_EINVAL, "ik_pose_multistart: seeds is NULL");
-  if (!scratch || !aligned16(scratch))
-    return fail(PNP_EINVAL, "ik_pose_multistart: scratch must be non-null and 16-byte aligned");
-  if (n > 0 && !flags)
-    return fail(PNP_EINVAL, "ik_pose_multistart: flags must be non-null (the restarts read attempt 0's success from it)");
-  if (n > 0) {
-    // seeds (read by every wave) and scratch (written) must not share memory with an output or with each other
-    auto range = [](const void* p, size_t bytes) { ByteRange r; if (p) { r.b = (const char*)p; r.e = r.b + bytes; } return r; };
-    const size_t m = (size_t)n;
-    const ByteRange in[2] = {range(seeds, (size_t)n_seeds * PNP_NJOINT * sizeof(T)), range(scratch, ms_scratch_bytes(n))};
-    const ByteRange out[10] = {range(q_out, m * PNP_NJOINT * sizeof(T)), range(final_pos, m * 3 * sizeof(T)),
-                               range(final_quat, m * 4 * sizeof(T)), range(pos_err, m * sizeof(T)),
-                               range(rot_err, m * sizeof(T)), range(iters, m * sizeof(int32_t)), range(flags, m),
-                               range(attempt, m), range(counters, 4 * sizeof(unsigned long long)),
-                               range(restart_stats, 3 * sizeof(unsigned long long))};
-    for (const ByteRange& o : out)
-      if (ranges_overlap(o, in[0]) || ranges_overlap(o, in[1]))
-        return fail(PNP_EINVAL, "ik_pose_multistart: seeds and scratch must not overlap an output");
-    if (ranges_overlap(in[0], in[1])) return fail(PNP_EINVAL, "ik_pose_multistart: seeds and scratch must not overlap");
-  }
-  unsigned* hdr = static_cast<unsigned*>(scratch);
-  unsigned* list[2] = {reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes),
-                       reinterpret_cast<unsigned*>((char*)scratch + kMsHdrBytes + ms_list_bytes(n))};
-  int32_t* iters0 = iters;
-  if (!iters0 && n_seeds > 0)  // the restarts need attempt 0's iterations for the counters
-    iters0 = reinterpret_cast<int32_t*>((char*)scratch + kMsHdrBytes + 2 * ms_list_bytes(n));
-  // attempt 0: the plain entry point, unchanged
-  int rc = pose_solve_impl<T>(tpos, tquat, q_init, q_init_stride, n, params, rot_thresh, rot_weight, q_out, final_pos,
-                              final_quat, pos_err, rot_err, iters0, flags, counters, stream);
-  if (rc || n == 0) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (attempt) CUDA_TRY(cudaMemsetAsync(attempt, 0, (size_t)n, st));
-  if (n_seeds == 0) return PNP_OK;
-  DeviceState* s;
-  if ((rc = current_state(&s))) return rc;
-  bool spec;
-  if ((rc = pick_kin(s, params->kinematics, &spec))) return rc;
-
-  CUDA_TRY(cudaMemsetAsync(hdr, 0, kMsHdrBytes, st));
-  {
-    const int grid = grid_for(n, pnp::MS_COLLECT_BLOCK, s->sm_count, 8);
-    pnp::ms_collect_kernel<pnp::IK_OUT_SEPARATE><<<grid, pnp::MS_COLLECT_BLOCK, 0, st>>>(
-        flags, nullptr, (unsigned)n, list[0], hdr, restart_stats);
-    ++g_launches;
-    CUDA_TRY(cudaGetLastError());
-  }
-  static const int env_group = env_int("PNP_MS_POSE_GROUP", 0);
-  const int G = (env_group == 1 || env_group == 2 || env_group == 4 || env_group == 8) ? env_group : kMsPoseGroup;
-  pnp::MsPoseArgs<T> m;
-  pnp::PoseIkArgs<T>& a = m.a;
-  memset(&a, 0, sizeof a);
-  a.target_pos = tpos; a.target_quat = tquat; a.q_init = q_init; a.q_init_stride = q_init_stride; a.n = (unsigned)n;
-  a.k = make_ik_const<T>(params);
-  a.rot_thresh = (T)rot_thresh; a.rot_weight = (T)rot_weight;
-  a.q_out = q_out; a.final_pos = final_pos; a.final_quat = final_quat; a.pos_err = pos_err; a.rot_err = rot_err;
-  a.iters = iters0; a.flags = flags; a.counters = counters;
-  m.seeds = seeds; m.n_seeds = n_seeds; m.group = (unsigned)G;
-  m.iters0 = iters0; m.attempt = attempt; m.restart_stats = restart_stats;
-  const int waves = (n_seeds + G - 1) / G;
-  for (int w = 0; w < waves; ++w) {
-    m.wave = w;
-    m.list_in = list[w & 1]; m.cnt_in = hdr + w;
-    m.list_out = w + 1 < waves ? list[(w + 1) & 1] : nullptr; m.cnt_out = hdr + w + 1;
-    const int slot = 6 + (std::is_same<T, float>::value ? 0 : 2) + (spec ? 0 : 1);
-    rc = spec ? launch_ms_wave(s, pnp::ms_pose_wave_kernel<T, pnp::SpecKin>, slot, m, st)
-              : launch_ms_wave(s, pnp::ms_pose_wave_kernel<T, pnp::GenericKin>, slot, m, st);
-    if (rc) return rc;
-  }
-  return PNP_OK;
+  const size_t m = (size_t)n;
+  return multistart_impl<pnp::PoseIkArgs<T>, pnp::IK_OUT_SEPARATE>(
+      "ik_pose_multistart", n, seeds, n_seeds, params, flags, iters, attempt, counters, restart_stats, scratch,
+      {byte_range(q_out, m * PNP_NJOINT * sizeof(T)), byte_range(final_pos, m * 3 * sizeof(T)),
+       byte_range(final_quat, m * 4 * sizeof(T)), byte_range(pos_err, m * sizeof(T)), byte_range(rot_err, m * sizeof(T)),
+       byte_range(iters, m * sizeof(int32_t)), byte_range(flags, m)},
+      kMsPoseGroup, "PNP_MS_POSE_GROUP", stream,
+      [&](int32_t* iters0, pnp::PoseIkArgs<T>& a) {
+        return pose_solve_impl<T>(tpos, tquat, q_init, q_init_stride, n, params, rot_thresh, rot_weight, q_out, final_pos,
+                                  final_quat, pos_err, rot_err, iters0, flags, counters, stream, &a);
+      },
+      [&](DeviceState* s, bool spec, const auto& m, cudaStream_t st) {
+        return spec ? launch_ms_wave<pnp::ms_pose_wave_kernel<T, pnp::SpecKin>>(s, m, st)
+                    : launch_ms_wave<pnp::ms_pose_wave_kernel<T, pnp::GenericKin>>(s, m, st);
+      });
 }
 
 template <typename T>

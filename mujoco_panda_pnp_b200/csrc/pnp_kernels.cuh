@@ -230,6 +230,53 @@ __device__ __forceinline__ float finish_sqrt(float n2) {
   return n2 * r;
 }
 
+// The two pieces of a position solve that ik_solve_kernel and the multistart restarts (ms_wave_kernel) share, so that a
+// restart attempt runs the plain kernel's arithmetic bit for bit.
+// One DLS pass at q (pass number `it`): a lane that is `active` and finishes in this pass calls
+// done(p, n2, iterations, conv) with FK(q) and the squared error at the q it finished at.  qn is the DLS step from q
+// (:81-85); the caller moves q there, for the lanes it keeps solving.
+template <typename T, typename Kin, typename Done>
+__device__ __forceinline__ void ik_pass(const IkConst<T>& k, const Trig<T>& trig, const T (&q)[NJ], const T (&tgt)[3],
+                                        int it, bool active, T (&qn)[NJ], Done done) {
+  T p[3], n2;
+  ik_eval_and_step<T, Kin>(q, tgt, k, trig, p, n2, qn);
+  const bool last = it >= k.max_iters;             // loop ran out (ik_solver.py:57)
+  const bool conv = !last && below_thresh(n2, k);  // :61-64
+  if (active && (conv || last)) done(p, n2, conv ? it + 1 : it, conv);  // iterations :66 / :85
+}
+
+// Store the record of query idx in layout kOut (:88-92: final_pos = FK(q) = p; final_error = err;
+// success = conv && err < 2*thresh).  Separate layout: every output but q_out nullable.
+template <int kOut, typename T>
+__device__ __forceinline__ void ik_store(const IkArgs<T>& a, unsigned idx, const T (&q)[NJ], const T* p, T n2,
+                                         int iterations, bool conv) {
+  const T err = finish_sqrt(n2);
+  const bool success = conv && (err < a.k.pos_thresh * T(2));
+  const unsigned fl = (conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u);
+  if (kOut == IK_OUT_PACKED) {
+    float4* oq = reinterpret_cast<float4*>(a.q_out) + (size_t)idx * 2u;
+    oq[0] = make_float4((float)q[0], (float)q[1], (float)q[2], (float)q[3]);
+    oq[1] = make_float4((float)q[4], (float)q[5], (float)q[6], (float)err);
+    reinterpret_cast<float4*>(a.final_pos)[idx] =
+        make_float4((float)p[0], (float)p[1], (float)p[2], __int_as_float((int)((unsigned)iterations | (fl << 24))));
+  } else if (kOut == IK_OUT_COMPACT) {
+    float4* oq = reinterpret_cast<float4*>(a.q_out) + (size_t)idx * 2u;
+    oq[0] = make_float4((float)q[0], (float)q[1], (float)q[2], (float)q[3]);
+    oq[1] = make_float4((float)q[4], (float)q[5], (float)q[6], __int_as_float((int)((unsigned)iterations | (fl << 24))));
+  } else {
+    T* qo = a.q_out + (size_t)idx * NJ;
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) qo[i] = q[i];
+    if (a.final_pos) {
+      T* fp = a.final_pos + (size_t)idx * 3u;
+      fp[0] = p[0]; fp[1] = p[1]; fp[2] = p[2];
+    }
+    if (a.pos_err) a.pos_err[idx] = err;
+    if (a.iters) a.iters[idx] = iterations;
+    if (a.flags) a.flags[idx] = (uint8_t)fl;
+  }
+}
+
 template <typename T, typename Kin, int kOut>
 __global__ void __launch_bounds__(IK_BLOCK) ik_solve_kernel(const IkArgs<T> a) {
   const unsigned lane = threadIdx.x & 31u;
@@ -299,43 +346,14 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_solve_kernel(const IkArgs<T> a) {
     if (!__any_sync(FULL, active)) break;
 
     // ---- one DLS pass for all lanes ----------------------------------------------------
-    T p[3], n2, qn[NJ];
-    ik_eval_and_step<T, Kin>(q, tgt, a.k, trig, p, n2, qn);
-    const bool last = it >= a.k.max_iters;                      // loop ran out (ik_solver.py:57)
-    const bool conv = !last && below_thresh(n2, a.k);           // :61-64
-    if (active && (conv || last)) {
-      const T err = finish_sqrt(n2);
-      const int iterations = conv ? it + 1 : it;                // :66 / :85
-      // :88-92  final_pos = FK(q) = p; final_error = err; success = conv && err < 2*thresh
-      const bool success = conv && (err < a.k.pos_thresh * T(2));
-      const unsigned fl = (conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u);
-      if (kOut == IK_OUT_PACKED) {
-        float4* oq = reinterpret_cast<float4*>(a.q_out) + (size_t)idx * 2u;
-        oq[0] = make_float4((float)q[0], (float)q[1], (float)q[2], (float)q[3]);
-        oq[1] = make_float4((float)q[4], (float)q[5], (float)q[6], (float)err);
-        reinterpret_cast<float4*>(a.final_pos)[idx] =
-            make_float4((float)p[0], (float)p[1], (float)p[2], __int_as_float((int)((unsigned)iterations | (fl << 24))));
-      } else if (kOut == IK_OUT_COMPACT) {
-        float4* oq = reinterpret_cast<float4*>(a.q_out) + (size_t)idx * 2u;
-        oq[0] = make_float4((float)q[0], (float)q[1], (float)q[2], (float)q[3]);
-        oq[1] = make_float4((float)q[4], (float)q[5], (float)q[6], __int_as_float((int)((unsigned)iterations | (fl << 24))));
-      } else {
-        T* qo = a.q_out + (size_t)idx * NJ;
-#pragma unroll
-        for (int i = 0; i < NJ; ++i) qo[i] = q[i];
-        if (a.final_pos) {
-          T* fp = a.final_pos + (size_t)idx * 3u;
-          fp[0] = p[0]; fp[1] = p[1]; fp[2] = p[2];
-        }
-        if (a.pos_err) a.pos_err[idx] = err;
-        if (a.iters) a.iters[idx] = iterations;
-        if (a.flags) a.flags[idx] = (uint8_t)fl;
-      }
+    T qn[NJ];
+    ik_pass<T, Kin>(a.k, trig, q, tgt, it, active, qn, [&](const T* p, T n2, int iterations, bool conv) {
+      ik_store<kOut>(a, idx, q, p, n2, iterations, conv);
       c_n += 1u;
       c_conv += conv ? 1u : 0u;
       c_iter += (unsigned)iterations;
       active = false;
-    }
+    });
     // unconditional update: a lane that just finished is idle and gets overwritten by the
     // refill at the top of the next pass (:81-85)
 #pragma unroll
@@ -1014,8 +1032,8 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_solve_one_kernel(const float* __r
 //   ms_collect_kernel   appends the index of every query whose attempt 0 failed to a list (one atomic per warp)
 //   ms_wave_*_kernel    wave w: each listed query gets a group of G consecutive lanes of one warp that run the seeds
 //                       [w G, w G + G) in parallel, each a plain solve from its seed (lane_solve on the specialised tree,
-//                       the ik_solve_kernel pass everywhere else: the same arithmetic as the plain entry points, so a
-//                       returned attempt is bit-identical to the plain solve from that start).  The lowest lane of the
+//                       ik_pass everywhere else: the same arithmetic as the plain entry points, so a returned attempt
+//                       is bit-identical to the plain solve from that start).  The lowest lane of the
 //                       group that succeeds overwrites the query's record; a query without a success goes onto the
 //                       next wave's list.
 // Every wave is launched whether or not its list is empty: it reads the list length on the device and its blocks leave at
@@ -1027,10 +1045,11 @@ constexpr int MS_COLLECT_BLOCK = 256;
 constexpr int MS_MAX_SEEDS = 255;
 constexpr int MS_HDR_WORDS = 256;  // list lengths: [0] = failures of attempt 0, [w + 1] = queries still failed after wave w
 
-template <typename T>
+// The argument block of a restart wave, for either solver: A is attempt 0's argument block (IkArgs<T>, PoseIkArgs<T>)
+template <typename A>
 struct MsArgs {
-  IkArgs<T> a;             // targets and the outputs of attempt 0 (its layout), solver constants
-  const T* seeds;          // [n_seeds][7]
+  A a;                     // targets and the outputs of attempt 0 (its layout), solver constants
+  const std::remove_pointer_t<decltype(A::q_out)>* seeds;  // [n_seeds][7], in the solver's float type
   int n_seeds;
   int wave;                // this launch runs seeds [wave * group, wave * group + group)
   unsigned group;          // lanes per query: a power of two <= 32
@@ -1038,7 +1057,7 @@ struct MsArgs {
   const unsigned* cnt_in;
   unsigned* list_out;      // nullptr: last wave
   unsigned* cnt_out;
-  const int32_t* iters0;   // separate layout: iterations of attempt 0 (the iters output or scratch)
+  const int32_t* iters0;   // separate layouts: iterations of attempt 0 (the iters output or scratch)
   uint8_t* attempt;        // nullable
   unsigned long long* restart_stats;  // nullable: restarted, rescued, DLS passes of restart attempts
 };
@@ -1074,11 +1093,10 @@ __global__ void __launch_bounds__(MS_COLLECT_BLOCK) ms_collect_kernel(const uint
 // The part of a wave every restart kernel shares (position: both lane mappings and layouts; pose): pick the group's
 // first success, store it, queue the unsolved queries.  `solve(valid, id, seed, out...)` runs one attempt per lane and
 // stores nothing; `prev(id, fl, it)` reads the flags and iteration count of the record being replaced (attempt 0's),
-// `store(id)` writes the lane's record.  M is MsArgs or MsPoseArgs: any argument block with the wave fields and the
-// attempt-0 arguments `a` (for a.counters).  Every solver counts success == converged, so the counter correction is
-// the same for all.
-template <typename M, typename Solve, typename Prev, typename Store>
-__device__ __forceinline__ void ms_wave(const M& m, unsigned cnt, Solve solve, Prev prev, Store store) {
+// `store(id)` writes the lane's record.  Every solver counts success == converged, so the counter correction is the
+// same for all.
+template <typename A, typename Solve, typename Prev, typename Store>
+__device__ __forceinline__ void ms_wave(const MsArgs<A>& m, unsigned cnt, Solve solve, Prev prev, Store store) {
   const unsigned lane = threadIdx.x & 31u;
   const unsigned G = m.group;
   const unsigned gl = lane & (G - 1u);
@@ -1140,8 +1158,8 @@ __device__ __forceinline__ void ms_wave(const M& m, unsigned cnt, Solve solve, P
 }
 
 // flags and iterations of attempt 0's position record: flags[] / iters0[] (separate layout) or the packed word
-template <int kOut, typename T>
-__device__ __forceinline__ void ms_ik_prev(const MsArgs<T>& m, unsigned id, unsigned& fl, unsigned& it) {
+template <int kOut, typename A>
+__device__ __forceinline__ void ms_ik_prev(const MsArgs<A>& m, unsigned id, unsigned& fl, unsigned& it) {
   if (kOut == IK_OUT_SEPARATE) {
     fl = m.a.flags[id];
     it = (unsigned)m.iters0[id];
@@ -1154,7 +1172,7 @@ __device__ __forceinline__ void ms_ik_prev(const MsArgs<T>& m, unsigned id, unsi
 
 // FP32 on the specialised tree: lane_solve + store_lane_result, i.e. ik_solve_small_kernel's arithmetic per lane
 template <int kOut>
-__global__ void __launch_bounds__(MS_BLOCK) ms_wave_v_kernel(const MsArgs<float> m) {
+__global__ void __launch_bounds__(MS_BLOCK) ms_wave_v_kernel(const MsArgs<IkArgs<float>> m) {
   const unsigned cnt = *m.cnt_in;
   if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;  // no work for any warp of this block
   __shared__ __align__(16) float s_trig[kTrigVWords];
@@ -1178,15 +1196,16 @@ __global__ void __launch_bounds__(MS_BLOCK) ms_wave_v_kernel(const MsArgs<float>
   ms_wave(m, cnt, solve, [&](unsigned id, unsigned& fl, unsigned& it) { ms_ik_prev<kOut>(m, id, fl, it); }, store);
 }
 
-// FP32 on other trees and FP64: per lane the pass of ik_solve_kernel (ik_eval_and_step), no refill
+// FP32 on other trees and FP64: per lane ik_pass and ik_store, ik_solve_kernel's pass and store block, no refill
 template <typename T, typename Kin, int kOut>
-__global__ void __launch_bounds__(MS_BLOCK) ms_wave_kernel(const MsArgs<T> m) {
+__global__ void __launch_bounds__(MS_BLOCK) ms_wave_kernel(const MsArgs<IkArgs<T>> m) {
   const unsigned cnt = *m.cnt_in;
   if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;
   __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
   if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
   __syncthreads();
   const Trig<T> trig{s_tab};
+  // the finished attempt of this lane: q (which stops moving when the lane finishes), FK(q) and the squared error
   T q[NJ], p[3], n2;
   bool conv;
   int it_kept = 0;
@@ -1202,49 +1221,23 @@ __global__ void __launch_bounds__(MS_BLOCK) ms_wave_kernel(const MsArgs<T> m) {
     p[0] = p[1] = p[2] = T(0);
     n2 = T(0);
     for (int it = 0; __any_sync(FULL, active); ++it) {
-      T pp[3], nn2, qn[NJ];
-      ik_eval_and_step<T, Kin>(q, tgt, m.a.k, trig, pp, nn2, qn);
-      const bool last = it >= m.a.k.max_iters;             // loop ran out (ik_solver.py:57)
-      const bool cv = !last && below_thresh(nn2, m.a.k);   // :61-64
+      T qn[NJ];
+      ik_pass<T, Kin>(m.a.k, trig, q, tgt, it, active, qn, [&](const T* pp, T nn2, int its, bool cv) {
+        conv = cv;
+        iterations = its;
+        p[0] = pp[0]; p[1] = pp[1]; p[2] = pp[2];
+        n2 = nn2;
+        active = false;
+      });
       if (active) {
-        if (cv || last) {
-          conv = cv;
-          iterations = cv ? it + 1 : it;                   // :66 / :85
-          p[0] = pp[0]; p[1] = pp[1]; p[2] = pp[2];
-          n2 = nn2;
-          active = false;
-        } else {
 #pragma unroll
-          for (int i = 0; i < NJ; ++i) q[i] = qn[i];       // :81-85
-        }
+        for (int i = 0; i < NJ; ++i) q[i] = qn[i];
       }
     }
     succ = conv && (finish_sqrt(n2) < m.a.k.pos_thresh * T(2));
     it_kept = iterations;
   };
-  auto store = [&](unsigned id) {  // ik_solve_kernel's store block
-    const T err = finish_sqrt(n2);
-    const bool success = conv && (err < m.a.k.pos_thresh * T(2));
-    const unsigned fl = (conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u);
-    if (kOut == IK_OUT_PACKED) {
-      float4* oq = reinterpret_cast<float4*>(m.a.q_out) + (size_t)id * 2u;
-      oq[0] = make_float4((float)q[0], (float)q[1], (float)q[2], (float)q[3]);
-      oq[1] = make_float4((float)q[4], (float)q[5], (float)q[6], (float)err);
-      reinterpret_cast<float4*>(m.a.final_pos)[id] =
-          make_float4((float)p[0], (float)p[1], (float)p[2], __int_as_float((int)((unsigned)it_kept | (fl << 24))));
-    } else {
-      T* qo = m.a.q_out + (size_t)id * NJ;
-#pragma unroll
-      for (int i = 0; i < NJ; ++i) qo[i] = q[i];
-      if (m.a.final_pos) {
-        T* fp = m.a.final_pos + (size_t)id * 3u;
-        fp[0] = p[0]; fp[1] = p[1]; fp[2] = p[2];
-      }
-      if (m.a.pos_err) m.a.pos_err[id] = err;
-      if (m.a.iters) m.a.iters[id] = it_kept;
-      m.a.flags[id] = (uint8_t)fl;
-    }
-  };
+  auto store = [&](unsigned id) { ik_store<kOut>(m.a, id, q, p, n2, it_kept, conv); };
   ms_wave(m, cnt, solve, [&](unsigned id, unsigned& fl, unsigned& it) { ms_ik_prev<kOut>(m, id, fl, it); }, store);
 }
 
@@ -1897,25 +1890,10 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArg
 // ik_pose_solve_kernel; the collect kernel lists the queries whose flags[] lack PNP_IK_SUCCESS; wave w gives each listed
 // query G lanes that run seeds [w G, w G + G) with pose_pass, the plain kernel's pass, from pose_load_target's target.
 // The lowest successful lane of a group stores the record with pose_store (every output the caller passed) and the
-// attempt; queries without a success go onto the next wave's list.
-template <typename T>
-struct MsPoseArgs {
-  PoseIkArgs<T> a;         // targets, solver constants and the outputs of attempt 0
-  const T* seeds;          // [n_seeds][7]
-  int n_seeds;
-  int wave;                // this launch runs seeds [wave * group, wave * group + group)
-  unsigned group;          // lanes per query: a power of two <= 32
-  const unsigned* list_in;
-  const unsigned* cnt_in;
-  unsigned* list_out;      // nullptr: last wave
-  unsigned* cnt_out;
-  const int32_t* iters0;   // iterations of attempt 0 (the iters output or scratch)
-  uint8_t* attempt;        // nullable
-  unsigned long long* restart_stats;  // nullable: restarted, rescued, DLS passes of restart attempts
-};
-
+// attempt; queries without a success go onto the next wave's list.  Attempt 0's flags and iterations are read as in the
+// position solver's separate layout (ms_ik_prev).
 template <typename T, typename Kin>
-__global__ void __launch_bounds__(MS_BLOCK) ms_pose_wave_kernel(const MsPoseArgs<T> m) {
+__global__ void __launch_bounds__(MS_BLOCK) ms_pose_wave_kernel(const MsArgs<PoseIkArgs<T>> m) {
   const unsigned cnt = *m.cnt_in;
   if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;  // no work for any warp of this block
   __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
@@ -1949,10 +1927,7 @@ __global__ void __launch_bounds__(MS_BLOCK) ms_pose_wave_kernel(const MsPoseArgs
     iterations = it_kept;
     succ = pose_success(m.a, pek, rek, conv);
   };
-  auto prev = [&](unsigned id, unsigned& fl, unsigned& it) {
-    fl = m.a.flags[id];
-    it = (unsigned)m.iters0[id];
-  };
+  auto prev = [&](unsigned id, unsigned& fl, unsigned& it) { ms_ik_prev<IK_OUT_SEPARATE>(m, id, fl, it); };
   auto store = [&](unsigned id) { pose_store(m.a, id, qk, pk, qck, pek, rek, it_kept, conv); };
   ms_wave(m, cnt, solve, prev, store);
 }

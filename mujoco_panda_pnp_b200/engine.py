@@ -115,6 +115,35 @@ def _check_out_np(name: str, a, shape, dtype) -> np.ndarray:
     return a
 
 
+def _q_init_arg(q_init: torch.Tensor, n: int, dt, dev) -> Tuple[torch.Tensor, int]:
+    """q_init of the device IK entry points and its row stride: (7,) is broadcast to every query (stride 0), (N, 7)
+    gives one start per query (stride 7)."""
+    if q_init.dim() == 1:
+        if q_init.shape != (7,):
+            raise ValueError("broadcast q_init must have shape (7,)")
+        return q_init.to(device=dev, dtype=dt).contiguous(), 0
+    q_init = _check_cuda("q_init", q_init, dt, (7,))
+    if q_init.shape[0] != n:
+        raise ValueError("q_init and the targets disagree on N")
+    return q_init, 7
+
+
+def _multistart_inputs(seeds, n: int, dt, dev, counters, restart_stats):
+    """The seed table (K, 7) of a multistart call in dt on dev, its scratch and its attempt output (uint8[N])."""
+    seeds = torch.as_tensor(seeds).to(device=dev, dtype=dt).reshape(-1, 7).contiguous()
+    if seeds.shape[0] > 255:
+        raise ValueError(f"at most 255 seeds, got {seeds.shape[0]}")
+    for name, t, m in (("counters", counters, 4), ("restart_stats", restart_stats, 3)):
+        if t is not None and (t.dtype != torch.int64 or t.numel() < m or not t.is_cuda):
+            raise ValueError(f"{name} must be a CUDA int64 tensor with >= {m} elements")
+    nbytes = ctypes.c_int64()
+    _lib.check(_lib.load().pnp_ik_multistart_scratch_bytes(n, ctypes.byref(nbytes)), "pnp_ik_multistart_scratch_bytes")
+    with torch.cuda.device(dev):
+        scratch = torch.empty(((nbytes.value + 15) // 16, 4), dtype=torch.int32, device=dev)
+        attempt = torch.empty((n,), dtype=torch.uint8, device=dev)
+    return seeds, scratch, attempt
+
+
 # ---------------------------------------------------------------------------------------------
 # FK + Jacobian
 # ---------------------------------------------------------------------------------------------
@@ -217,17 +246,8 @@ def ik_solve(targets: torch.Tensor, q_init: torch.Tensor, params: PnpIkParams, c
         raise ValueError("targets must be float32 or float64")
     targets = _check_cuda("targets", targets, dt, (3,))
     n = targets.shape[0]
-    if q_init.dim() == 1:
-        if q_init.shape != (7,):
-            raise ValueError("broadcast q_init must have shape (7,)")
-        stride = 0
-        q_init = q_init.to(device=targets.device, dtype=dt).contiguous()
-    else:
-        q_init = _check_cuda("q_init", q_init, dt, (7,))
-        if q_init.shape[0] != n:
-            raise ValueError("q_init and targets disagree on N")
-        stride = 7
     dev = targets.device
+    q_init, stride = _q_init_arg(q_init, n, dt, dev)
     if counters is not None and (counters.dtype != torch.int64 or counters.numel() < 4 or not counters.is_cuda):
         raise ValueError("counters must be a CUDA int64 tensor with >= 4 elements")
     if compact:
@@ -306,32 +326,14 @@ def ik_solve_multistart(targets: torch.Tensor, q_init: torch.Tensor, seeds: torc
     targets = _check_cuda("targets", targets, dt, (3,))
     n = targets.shape[0]
     dev = targets.device
-    if q_init.dim() == 1:
-        if q_init.shape != (7,):
-            raise ValueError("broadcast q_init must have shape (7,)")
-        stride = 0
-        q_init = q_init.to(device=dev, dtype=dt).contiguous()
-    else:
-        q_init = _check_cuda("q_init", q_init, dt, (7,))
-        if q_init.shape[0] != n:
-            raise ValueError("q_init and targets disagree on N")
-        stride = 7
-    seeds = torch.as_tensor(seeds).to(device=dev, dtype=dt).reshape(-1, 7).contiguous()
-    k = seeds.shape[0]
-    if k > 255:
-        raise ValueError(f"at most 255 seeds, got {k}")
-    for name, t, m in (("counters", counters, 4), ("restart_stats", restart_stats, 3)):
-        if t is not None and (t.dtype != torch.int64 or t.numel() < m or not t.is_cuda):
-            raise ValueError(f"{name} must be a CUDA int64 tensor with >= {m} elements")
+    q_init, stride = _q_init_arg(q_init, n, dt, dev)
     if packed is None:
         packed = dt == torch.float32
     if packed and dt != torch.float32:
         raise ValueError("packed outputs exist for float32 only")
-    nbytes = ctypes.c_int64()
-    _lib.check(lib.pnp_ik_multistart_scratch_bytes(n, ctypes.byref(nbytes)), "pnp_ik_multistart_scratch_bytes")
+    seeds, scratch, attempt = _multistart_inputs(seeds, n, dt, dev, counters, restart_stats)
+    k = seeds.shape[0]
     with torch.cuda.device(dev):
-        scratch = torch.empty(((nbytes.value + 15) // 16, 4), dtype=torch.int32, device=dev)
-        attempt = torch.empty((n,), dtype=torch.uint8, device=dev)
         if packed:
             q8 = torch.empty((n, 8), dtype=dt, device=dev)
             aux = torch.empty((n, 4), dtype=dt, device=dev)
@@ -397,15 +399,8 @@ def ik_pose_solve(target_pos: torch.Tensor, target_quat: torch.Tensor, q_init: t
     n = target_pos.shape[0]
     if target_quat.shape[0] != n:
         raise ValueError("target_pos and target_quat disagree on N")
-    if q_init.dim() == 1:
-        if q_init.shape != (7,):
-            raise ValueError("broadcast q_init must have shape (7,)")
-        q_init, stride = q_init.to(device=target_pos.device, dtype=dt).contiguous(), 0
-    else:
-        q_init, stride = _check_cuda("q_init", q_init, dt, (7,)), 7
-        if q_init.shape[0] != n:
-            raise ValueError("q_init disagrees with target_pos on N")
     dev = target_pos.device
+    q_init, stride = _q_init_arg(q_init, n, dt, dev)
     q = torch.empty((n, 7), dtype=dt, device=dev)
     fpos = torch.empty((n, 3), dtype=dt, device=dev)
     fquat = torch.empty((n, 4), dtype=dt, device=dev)
@@ -446,27 +441,11 @@ def ik_pose_solve_multistart(target_pos: torch.Tensor, target_quat: torch.Tensor
     if target_quat.shape[0] != n:
         raise ValueError("target_pos and target_quat disagree on N")
     dev = target_pos.device
-    if q_init.dim() == 1:
-        if q_init.shape != (7,):
-            raise ValueError("broadcast q_init must have shape (7,)")
-        q_init, stride = q_init.to(device=dev, dtype=dt).contiguous(), 0
-    else:
-        q_init, stride = _check_cuda("q_init", q_init, dt, (7,)), 7
-        if q_init.shape[0] != n:
-            raise ValueError("q_init disagrees with target_pos on N")
-    seeds = torch.as_tensor(seeds).to(device=dev, dtype=dt).reshape(-1, 7).contiguous()
+    q_init, stride = _q_init_arg(q_init, n, dt, dev)
+    seeds, scratch, attempt = _multistart_inputs(seeds, n, dt, dev, counters, restart_stats)
     k = seeds.shape[0]
-    if k > 255:
-        raise ValueError(f"at most 255 seeds, got {k}")
-    for name, t, m in (("counters", counters, 4), ("restart_stats", restart_stats, 3)):
-        if t is not None and (t.dtype != torch.int64 or t.numel() < m or not t.is_cuda):
-            raise ValueError(f"{name} must be a CUDA int64 tensor with >= {m} elements")
-    nbytes = ctypes.c_int64()
-    _lib.check(lib.pnp_ik_multistart_scratch_bytes(n, ctypes.byref(nbytes)), "pnp_ik_multistart_scratch_bytes")
     fn = lib.pnp_ik_pose_solve_multistart_f32 if dt == torch.float32 else lib.pnp_ik_pose_solve_multistart_f64
     with torch.cuda.device(dev):
-        scratch = torch.empty(((nbytes.value + 15) // 16, 4), dtype=torch.int32, device=dev)
-        attempt = torch.empty((n,), dtype=torch.uint8, device=dev)
         q = torch.empty((n, 7), dtype=dt, device=dev)
         fpos = torch.empty((n, 3), dtype=dt, device=dev)
         fquat = torch.empty((n, 4), dtype=dt, device=dev)

@@ -61,10 +61,6 @@ struct DeviceState {
   cudaStream_t slot_stream[kStreamSlots] = {};
   bool slot_used[kStreamSlots] = {};
   unsigned slot_clock = 0;
-  int occ_ik[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  bool obs_smem_set = false;
-  bool fk_smem_set = false;
-  bool plan_smem_set = false;
 };
 DeviceState g_dev[kMaxDevices];
 std::mutex g_mu;
@@ -181,6 +177,62 @@ int grid_for(long long work_items, int block, int sm_count, int blocks_per_sm) {
   return (int)g;
 }
 
+// Raise a kernel's dynamic shared-memory cap above the default 48 KB, once per kernel and device.  Before the kernel's
+// occupancy query too: the query only sees the raised cap.
+template <auto kKernel>
+int max_dynamic_smem(DeviceState* s, size_t bytes) {
+  static bool set_on_device[kMaxDevices] = {};
+  bool& set = set_on_device[s - g_dev];
+  if (!set) {
+    CUDA_TRY(cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    set = true;
+  }
+  return PNP_OK;
+}
+
+// Resident blocks per SM of a kernel, queried once per kernel and device (every kernel is launched with one block size
+// and one dynamic shared-memory size).  A kernel of which no block fits an SM cannot be launched: an error.
+template <auto kKernel>
+int occupancy(DeviceState* s, int block, size_t smem, int* out) {
+  static int occ_of_device[kMaxDevices] = {};
+  int& occ = occ_of_device[s - g_dev];
+  if (occ == 0) {
+    int o = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, kKernel, block, smem));
+    if (o < 1) return cuda_fail(cudaErrorLaunchOutOfResources, "cudaOccupancyMaxActiveBlocksPerMultiprocessor: 0 blocks per SM");
+    occ = o;
+  }
+  *out = occ;
+  return PNP_OK;
+}
+
+// Launch geometry of a persistent-warp kernel of the IK family (lanes keep drawing queries from a ticket, S queries per
+// lane).  Small batches: one working warp per block - the block's other warps only load the trig table - so that the few
+// warps spread over as many SMs as possible.  Otherwise the lanes the batch needs, capped at occ blocks per SM.  A warp
+// reserves `chunk` queries per ticket atomic: about 1/div of its share, within [32 S, cap], a multiple of 32.  (For a
+// small batch, n <= 32 S grid and n / (warps div) < S: the chunk is the floor 32 S, whichever warp count divides.)
+struct PersistentGrid {
+  int grid;
+  unsigned chunk;
+};
+PersistentGrid persistent_grid(const DeviceState* s, long long n, int S, int block, int occ, bool small, int div, int cap) {
+  const long long lanes = (n + S - 1) / S;
+  PersistentGrid g;
+  g.grid = small ? (int)((lanes + 31) / 32) : grid_for(lanes, block, s->sm_count, occ);
+  long long chunk = n / ((long long)g.grid * (block / 32) * div);
+  chunk = chunk < 32 * S ? 32 * S : (chunk > cap ? cap : chunk);
+  g.chunk = (unsigned)(chunk & ~31ll);
+  return g;
+}
+
+// The refill ticket of the stream's scratch slot, zeroed on the stream.
+int stream_ticket(DeviceState* s, cudaStream_t st, unsigned** out) {
+  unsigned* ticket = s->tickets + stream_slot(s, st);
+  CUDA_TRY(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));
+  *out = ticket;
+  return PNP_OK;
+}
+
 template <typename T>
 pnp::IkConst<T> make_ik_const(const PnpIkParams* p) {
   pnp::IkConst<T> k;
@@ -216,11 +268,9 @@ int fk_jac_impl(const T* q, int64_t n, T* pos, T* quat, T* jac, int32_t kinemati
     // (position / quaternion only: 12-28 B out per configuration, the per-lane kernel at full occupancy is faster)
     const bool aligned = aligned16(pos) && (!quat || aligned16(quat)) && aligned16(jac);
     if (jac && aligned && n >= pnp::FK_TILE) {
-      if (!s->fk_smem_set) {
-        CUDA_TRY(cudaFuncSetAttribute(pnp::fk_jac_bulk_kernel<pnp::SpecKin>, cudaFuncAttributeMaxDynamicSharedMemorySize, pnp::FK_BULK_SMEM));
-        CUDA_TRY(cudaFuncSetAttribute(pnp::fk_jac_bulk_kernel<pnp::GenericKin>, cudaFuncAttributeMaxDynamicSharedMemorySize, pnp::FK_BULK_SMEM));
-        s->fk_smem_set = true;
-      }
+      rc = spec ? max_dynamic_smem<pnp::fk_jac_bulk_kernel<pnp::SpecKin>>(s, pnp::FK_BULK_SMEM)
+                : max_dynamic_smem<pnp::fk_jac_bulk_kernel<pnp::GenericKin>>(s, pnp::FK_BULK_SMEM);
+      if (rc) return rc;
       const int64_t tiles = n / pnp::FK_TILE;
       const int grid = (int)std::min<int64_t>(tiles, (int64_t)s->sm_count * 4);  // 4 x 49 KB of shared memory per SM
       if (spec)
@@ -272,11 +322,9 @@ int get_obs_impl(const T* q_arm, const T* qvel_arm, const T* fingers, const T* o
                          aligned16(obj_quat) && aligned16(obj_vel) && aligned16(out) && (goal_stride == 0 || aligned16(goal));
     static const bool bulk_enabled = [] { const char* e = getenv("PNP_OBS_BULK"); return !e || atoi(e) != 0; }();
     if (aligned && bulk_enabled && n >= pnp::OBS_TILE) {
-      if (!s->obs_smem_set) {
-        CUDA_TRY(cudaFuncSetAttribute(pnp::get_obs_bulk_kernel<pnp::SpecKin>, cudaFuncAttributeMaxDynamicSharedMemorySize, pnp::OBS_BULK_SMEM));
-        CUDA_TRY(cudaFuncSetAttribute(pnp::get_obs_bulk_kernel<pnp::GenericKin>, cudaFuncAttributeMaxDynamicSharedMemorySize, pnp::OBS_BULK_SMEM));
-        s->obs_smem_set = true;
-      }
+      rc = spec ? max_dynamic_smem<pnp::get_obs_bulk_kernel<pnp::SpecKin>>(s, pnp::OBS_BULK_SMEM)
+                : max_dynamic_smem<pnp::get_obs_bulk_kernel<pnp::GenericKin>>(s, pnp::OBS_BULK_SMEM);
+      if (rc) return rc;
       const int64_t tiles = n / pnp::OBS_TILE;
       const int grid = (int)std::min<int64_t>(tiles, (int64_t)s->sm_count * 3);  // 3 x 72 KB of shared memory per SM
       if (spec)
@@ -309,25 +357,15 @@ int env_int(const char* name, int dflt) {
 
 template <typename T, typename Kin, int kOut>
 int launch_ik(DeviceState* s, const pnp::IkArgs<T>& a, bool small, cudaStream_t st) {
-  const int slot = (sizeof(T) == 8 ? 4 : 0) + (Kin::kSpecialized ? 2 : 0) + (kOut != pnp::IK_OUT_SEPARATE ? 1 : 0);
-  if (s->occ_ik[slot] == 0) {
-    int occ = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::ik_solve_kernel<T, Kin, kOut>,
-                                                                  pnp::IK_BLOCK, 0);
-    s->occ_ik[slot] = (e == cudaSuccess && occ > 0) ? occ : 1;
-  }
-  // Persistent grid: every resident lane keeps pulling queries.  Small batches use one working warp
-  // per block so the few warps spread over as many SMs as possible (latency bound).
-  const int block = pnp::IK_BLOCK;  // small: one working warp + three table-loading helper warps per block
-  const int grid = small ? (int)((a.n + 31u) / 32u) : grid_for(a.n, block, s->sm_count, s->occ_ik[slot]);
+  int occ;
+  const int rc = occupancy<pnp::ik_solve_kernel<T, Kin, kOut>>(s, pnp::IK_BLOCK, 0, &occ);
+  if (rc) return rc;
   // queries reserved per ticket atomic: ~1/16 of a warp's share, within [32, 256]
+  const PersistentGrid g = persistent_grid(s, a.n, 1, pnp::IK_BLOCK, occ, small, 16, 256);
   pnp::IkArgs<T> args = a;
-  const long long warps = (long long)grid * (block / 32);
-  long long chunk = (long long)a.n / (warps * 16);
-  chunk = chunk < 32 ? 32 : (chunk > 256 ? 256 : chunk);
-  args.chunk = (unsigned)(chunk & ~31ll);
+  args.chunk = g.chunk;
   args.solo_warp = small ? 1u : 0u;
-  pnp::ik_solve_kernel<T, Kin, kOut><<<grid, block, 0, st>>>(args);
+  pnp::ik_solve_kernel<T, Kin, kOut><<<g.grid, pnp::IK_BLOCK, 0, st>>>(args);
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return PNP_OK;
@@ -337,26 +375,22 @@ int launch_ik(DeviceState* s, const pnp::IkArgs<T>& a, bool small, cudaStream_t 
 template <typename V, int kOut>
 int launch_ik_v(DeviceState* s, const pnp::IkArgs<float>& a, bool small, cudaStream_t st) {
   constexpr int S = pnp::Slots<V>::kN;
-  const int slot = 8 + (S - 1) * 2 + (kOut != pnp::IK_OUT_SEPARATE ? 1 : 0);
-  if (s->occ_ik[slot] == 0) {
-    int occ = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::ik_solve_v_kernel<V, kOut, true>,
-                                                                  pnp::IK_BLOCK, 0);
-    s->occ_ik[slot] = (e == cudaSuccess && occ > 0) ? occ : 1;
-  }
-  // small batches: one solving warp per block (spreads the batch over all SMs), plus three helper warps that
-  // only load the trig table (a lone warp needs ~5 us for its 40 KB)
+  // (small batches: a lone warp would need ~5 us to load the 40 KB trig table, hence the helper warps)
   const int block = pnp::IK_BLOCK;
-  const long long lanes_needed = ((long long)a.n + S - 1) / S;
+  // the grid of all four variants below follows the instantiation with counters, and the compact layout's follows the
+  // packed one's: those use fewer registers, and 5 blocks per SM measured slower than 4 (DESIGN.md 4.1)
+  constexpr int kOccOut = kOut == pnp::IK_OUT_SEPARATE ? pnp::IK_OUT_SEPARATE : pnp::IK_OUT_PACKED;
+  int occ;
+  const int rc = occupancy<pnp::ik_solve_v_kernel<V, kOccOut, true>>(s, block, 0, &occ);
+  if (rc) return rc;
   static const int env_occ = env_int("PNP_IK_OCC", 0);
-  const int occ_use = env_occ > 0 && env_occ < s->occ_ik[slot] ? env_occ : s->occ_ik[slot];
-  const int grid = small ? (int)((lanes_needed + 31) / 32) : grid_for(lanes_needed, block, s->sm_count, occ_use);
+  const int occ_use = env_occ > 0 && env_occ < occ ? env_occ : occ;
+  const PersistentGrid g = persistent_grid(s, a.n, S, block, occ_use, small, 16, 256);
+  const int grid = g.grid;
+  const long long warps = (long long)grid * (block / 32);
   pnp::IkArgs<float> args = a;
   args.solo_warp = small ? 1u : 0u;
-  const long long warps = small ? (long long)grid : (long long)grid * (block / 32);
-  long long chunk = (long long)a.n / (warps * 16);
-  chunk = chunk < 32 * S ? 32 * S : (chunk > 256 ? 256 : chunk);
-  args.chunk = (unsigned)(chunk & ~31ll);
+  args.chunk = g.chunk;
   {
     // lanes with a finished slot that trigger a store + refill (PNP_IK_FLUSH_MIN overrides, for tuning)
     static const int env_flush = env_int("PNP_IK_FLUSH_MIN", 0);
@@ -563,8 +597,7 @@ int ik_solve_impl(const T* targets, const T* q_init, int32_t q_init_stride, int6
   if (spec) {
     if constexpr (std::is_same<T, float>::value) return launch_ik_spec_f32<kOut>(s, a, params->kinematics, small, st);  // own tickets
   }
-  a.ticket = s->tickets + stream_slot(s, st);
-  CUDA_TRY(cudaMemsetAsync(a.ticket, 0, sizeof(unsigned), st));
+  if ((rc = stream_ticket(s, st, &a.ticket))) return rc;
   if (spec) {
     if constexpr (!std::is_same<T, float>::value) {
       return launch_ik<T, pnp::SpecKin, kOut>(s, a, small, st);
@@ -590,16 +623,12 @@ size_t ms_list_bytes(int64_t n) { return ((size_t)n * sizeof(unsigned) + 15u) & 
 // header | list A | list B | iterations of attempt 0 (separate layout without an iters output)
 size_t ms_scratch_bytes(int64_t n) { return kMsHdrBytes + 3 * ms_list_bytes(n); }
 
-// one restart wave; the occupancy of each wave kernel is queried once per device
+// one restart wave
 template <auto kKernel, typename M>
 int launch_ms_wave(DeviceState* s, const M& m, cudaStream_t st) {
-  static int occ_of_device[kMaxDevices] = {};
-  int& occ = occ_of_device[s - g_dev];
-  if (occ == 0) {
-    int o = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, kKernel, pnp::MS_BLOCK, 0);
-    occ = (e == cudaSuccess && o > 0) ? o : 1;
-  }
+  int occ;
+  const int rc = occupancy<kKernel>(s, pnp::MS_BLOCK, 0, &occ);
+  if (rc) return rc;
   kKernel<<<s->sm_count * occ, pnp::MS_BLOCK, 0, st>>>(m);
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
@@ -933,34 +962,28 @@ int pnp_ik_waypoints_f32(const float* q_start, const float* goal, int64_t n, int
   if (n == 0) return PNP_OK;
   if (n >= (int64_t(1) << 31)) return fail(PNP_EINVAL, "ik_waypoints: n must be < 2^31 per call");
   cudaStream_t st = (cudaStream_t)stream;
-  unsigned* ticket = s->tickets + stream_slot(s, st);
-  CUDA_TRY(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));
   pnp::WaypointArgs<float> a;
-  a.q_start = q_start; a.goal = goal; a.n = (unsigned)n; a.n_steps = n_steps; a.ticket = ticket;
+  if ((rc = stream_ticket(s, st, &a.ticket))) return rc;
+  a.q_start = q_start; a.goal = goal; a.n = (unsigned)n; a.n_steps = n_steps;
   a.step_size = (float)step_size; a.reach_thresh = 0.01f;
   a.k = make_ik_const<float>(params);
   a.q_out = q_out; a.pos_out = pos_out; a.n_accepted = n_accepted; a.iters_total = iters_total;
   a.counters = counters;
   const bool small = n <= (long long)s->sm_count * pnp::IK_BLOCK;
-  const int block = pnp::IK_BLOCK;  // small: one working warp + three table-loading helper warps per block
+  const int block = pnp::IK_BLOCK;
   // specialised tree: the value-type kernels (same arithmetic in both), one env per lane unless two are asked
   // for (with the fused accept / first-iteration pass the bookkeeping weighs more than the packed arithmetic
   // saves: 2^20 envs x 50, 0.81 ms against 0.87); other trees: the scalar-template kernel
   const bool pair = spec && params->kinematics == PNP_KIN_SPEC_PAIR;
-  const int S = pair ? 2 : 1;
-  int occ = 4;
-  if (!small) {
-    cudaError_t e = !spec ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::ik_waypoints_kernel<float, pnp::GenericKin>, pnp::IK_BLOCK, 0)
-                    : pair ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::ik_waypoints_v_kernel<pnp::F2, true>, pnp::IK_BLOCK, 0)
-                           : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::ik_waypoints_v_kernel<float, true>, pnp::IK_BLOCK, 0);
-    if (e != cudaSuccess || occ < 1) occ = 4;
-  }
-  const long long lanes_needed = (n + S - 1) / S;
-  const int grid = small ? (int)((lanes_needed + 31) / 32) : grid_for(lanes_needed, block, s->sm_count, occ);
+  int occ;  // (the fused instantiation's, for both)
+  rc = !spec ? occupancy<pnp::ik_waypoints_kernel<float, pnp::GenericKin>>(s, block, 0, &occ)
+       : pair ? occupancy<pnp::ik_waypoints_v_kernel<pnp::F2, true>>(s, block, 0, &occ)
+              : occupancy<pnp::ik_waypoints_v_kernel<float, true>>(s, block, 0, &occ);
+  if (rc) return rc;
   // envs reserved per ticket atomic: ~1/8 of a warp's share within [32 S, 128] (keeps the tail short)
-  long long chunk = n / ((long long)grid * (block / 32) * 8);
-  chunk = chunk < 32 * S ? 32 * S : (chunk > 128 ? 128 : chunk);
-  a.chunk = (unsigned)(chunk & ~31ll);
+  const PersistentGrid g = persistent_grid(s, n, pair ? 2 : 1, block, occ, small, 8, 128);
+  const int grid = g.grid;
+  a.chunk = g.chunk;
   a.solo_warp = small ? 1u : 0u;
   if (!spec)
     pnp::ik_waypoints_kernel<float, pnp::GenericKin><<<grid, block, 0, st>>>(a);
@@ -1000,32 +1023,27 @@ int pose_solve_impl(const T* tpos, const T* tquat, const T* q_init, int32_t q_in
   if (n == 0) return PNP_OK;
   if (n >= (int64_t(1) << 31)) return fail(PNP_EINVAL, "ik_pose_solve: n must be < 2^31 per call");
   cudaStream_t st = (cudaStream_t)stream;
-  unsigned* ticket = s->tickets + stream_slot(s, st);
-  CUDA_TRY(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));
   pnp::PoseIkArgs<T> a;
+  if ((rc = stream_ticket(s, st, &a.ticket))) return rc;
   a.target_pos = tpos; a.target_quat = tquat; a.q_init = q_init; a.q_init_stride = q_init_stride; a.n = (unsigned)n;
   a.k = make_ik_const<T>(params);
   a.rot_thresh = (T)rot_thresh; a.rot_weight = (T)rot_weight;
   a.q_out = q_out; a.final_pos = final_pos; a.final_quat = final_quat; a.pos_err = pos_err; a.rot_err = rot_err;
-  a.iters = iters; a.flags = flags; a.counters = counters; a.ticket = ticket;
+  a.iters = iters; a.flags = flags; a.counters = counters;
   const bool small = n <= (long long)s->sm_count * pnp::IK_BLOCK;
-  const int block = pnp::IK_BLOCK;  // small: one working warp + three table-loading helper warps per block
-  int occ = 4;
-  if (!small) {
-    cudaError_t e = spec ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::ik_pose_solve_kernel<T, pnp::SpecKin>, pnp::IK_BLOCK, 0)
-                         : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::ik_pose_solve_kernel<T, pnp::GenericKin>, pnp::IK_BLOCK, 0);
-    if (e != cudaSuccess || occ < 1) occ = 4;
-  }
-  const int grid = small ? (int)((n + 31) / 32) : grid_for(n, block, s->sm_count, occ);
-  long long chunk = n / ((long long)grid * (block / 32) * 16);
-  chunk = chunk < 32 ? 32 : (chunk > 256 ? 256 : chunk);
-  a.chunk = (unsigned)(chunk & ~31ll);
+  const int block = pnp::IK_BLOCK;
+  int occ;
+  rc = spec ? occupancy<pnp::ik_pose_solve_kernel<T, pnp::SpecKin>>(s, block, 0, &occ)
+            : occupancy<pnp::ik_pose_solve_kernel<T, pnp::GenericKin>>(s, block, 0, &occ);
+  if (rc) return rc;
+  const PersistentGrid g = persistent_grid(s, n, 1, block, occ, small, 16, 256);
+  a.chunk = g.chunk;
   a.solo_warp = small ? 1u : 0u;
   if (args_out) *args_out = a;  // the multistart's restarts use this block
   if (spec)
-    pnp::ik_pose_solve_kernel<T, pnp::SpecKin><<<grid, block, 0, st>>>(a);
+    pnp::ik_pose_solve_kernel<T, pnp::SpecKin><<<g.grid, block, 0, st>>>(a);
   else
-    pnp::ik_pose_solve_kernel<T, pnp::GenericKin><<<grid, block, 0, st>>>(a);
+    pnp::ik_pose_solve_kernel<T, pnp::GenericKin><<<g.grid, block, 0, st>>>(a);
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return PNP_OK;
@@ -1113,10 +1131,9 @@ int move_plan_impl(const T* q_start, const T* target, int64_t n, const PnpMovePa
   if (n == 0) return PNP_OK;
   if (n >= (int64_t(1) << 31)) return fail(PNP_EINVAL, "move_ik_plan: n must be < 2^31 per call");
   cudaStream_t st = (cudaStream_t)stream;
-  unsigned* ticket = s->tickets + stream_slot(s, st);
-  CUDA_TRY(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));
   pnp::MoveArgs<T> a;
-  a.q_start = q_start; a.target = target; a.n = (unsigned)n; a.ticket = ticket;
+  if ((rc = stream_ticket(s, st, &a.ticket))) return rc;
+  a.q_start = q_start; a.target = target; a.n = (unsigned)n;
   a.pos_thresh = (T)mp->pos_thresh; a.step_size = (T)mp->step_size;
   a.max_traj_points = mp->max_traj_points;
   a.max_outer = mp->max_outer > 0 ? mp->max_outer : 4 * mp->max_traj_points + 64;
@@ -1127,7 +1144,8 @@ int move_plan_impl(const T* q_start, const T* target, int64_t n, const PnpMovePa
   a.order = order;
   a.records = records;
   const bool small = n <= (long long)s->sm_count * pnp::IK_BLOCK;
-  int block = pnp::IK_BLOCK;  // small: one working warp + three table-loading helper warps per block
+  int block = pnp::IK_BLOCK;
+  int occ;
   if constexpr (std::is_same<T, float>::value) {
     if (spec) {
       // specialised tree, FP32: the value-type kernels (same arithmetic in both, branch-free common path)
@@ -1142,25 +1160,19 @@ int move_plan_impl(const T* q_start, const T* target, int64_t n, const PnpMovePa
       const bool stage = env_stage && !pair && !small && mp->traj_cap % 4 == 0 && aligned16(traj);
       if (stage) block = pnp::PLAN_BLOCK;
       const size_t smem = pnp::plan_smem_bytes(S, block, stage);
-      if (stage && !s->plan_smem_set) {  // 53 KB of dynamic shared memory: above the default 48 KB cap
-        CUDA_TRY(cudaFuncSetAttribute(pnp::move_ik_plan_v_kernel<float, true, pnp::PLAN_BLOCK, true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CUDA_TRY(cudaFuncSetAttribute(pnp::move_ik_plan_v_kernel<float, false, pnp::PLAN_BLOCK, true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        s->plan_smem_set = true;
+      // (the fused instantiation's occupancy, for both; the staged kernels need 53 KB of dynamic shared memory)
+      if (stage) {
+        if ((rc = max_dynamic_smem<pnp::move_ik_plan_v_kernel<float, true, pnp::PLAN_BLOCK, true>>(s, smem)) ||
+            (rc = max_dynamic_smem<pnp::move_ik_plan_v_kernel<float, false, pnp::PLAN_BLOCK, true>>(s, smem)))
+          return rc;
       }
-      int occv = 4;
-      if (!small) {
-        cudaError_t e = pair    ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occv, pnp::move_ik_plan_v_kernel<pnp::F2, true>, block, smem)
-                        : stage ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occv, pnp::move_ik_plan_v_kernel<float, true, pnp::PLAN_BLOCK, true>, block, smem)
-                                : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occv, pnp::move_ik_plan_v_kernel<float, true>, block, smem);
-        if (e != cudaSuccess || occv < 1) occv = 4;
-      }
-      const long long lanes_needed = (n + S - 1) / S;
-      const int gridv = small ? (int)((lanes_needed + 31) / 32) : grid_for(lanes_needed, block, s->sm_count, occv);
-      long long chunkv = n / ((long long)gridv * (block / 32) * 8);
-      chunkv = chunkv < 32 * S ? 32 * S : (chunkv > 128 ? 128 : chunkv);
-      a.chunk = (unsigned)(chunkv & ~31ll);
+      rc = pair    ? occupancy<pnp::move_ik_plan_v_kernel<pnp::F2, true>>(s, block, smem, &occ)
+           : stage ? occupancy<pnp::move_ik_plan_v_kernel<float, true, pnp::PLAN_BLOCK, true>>(s, block, smem, &occ)
+                   : occupancy<pnp::move_ik_plan_v_kernel<float, true>>(s, block, smem, &occ);
+      if (rc) return rc;
+      const PersistentGrid g = persistent_grid(s, n, S, block, occ, small, 8, 128);
+      const int gridv = g.grid;
+      a.chunk = g.chunk;
       a.solo_warp = small ? 1u : 0u;
       if (pair && fuse) pnp::move_ik_plan_v_kernel<pnp::F2, true><<<gridv, block, smem, st>>>(a);
       else if (pair) pnp::move_ik_plan_v_kernel<pnp::F2, false><<<gridv, block, smem, st>>>(a);
@@ -1173,22 +1185,17 @@ int move_plan_impl(const T* q_start, const T* target, int64_t n, const PnpMovePa
       return PNP_OK;
     }
   }
-  int occ = 4;
-  if (!small) {
-    cudaError_t e = spec ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::move_ik_plan_kernel<T, pnp::SpecKin>, pnp::IK_BLOCK, 0)
-                         : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pnp::move_ik_plan_kernel<T, pnp::GenericKin>, pnp::IK_BLOCK, 0);
-    if (e != cudaSuccess || occ < 1) occ = 4;
-  }
-  const int grid = small ? (int)((n + 31) / 32) : grid_for(n, block, s->sm_count, occ);
+  rc = spec ? occupancy<pnp::move_ik_plan_kernel<T, pnp::SpecKin>>(s, block, 0, &occ)
+            : occupancy<pnp::move_ik_plan_kernel<T, pnp::GenericKin>>(s, block, 0, &occ);
+  if (rc) return rc;
   // envs reserved per ticket atomic: ~1/8 of a warp's share within [32, 128] (keeps the tail short)
-  long long chunk = n / ((long long)grid * (block / 32) * 8);
-  chunk = chunk < 32 ? 32 : (chunk > 128 ? 128 : chunk);
-  a.chunk = (unsigned)(chunk & ~31ll);
+  const PersistentGrid g = persistent_grid(s, n, 1, block, occ, small, 8, 128);
+  a.chunk = g.chunk;
   a.solo_warp = small ? 1u : 0u;
   if (spec)
-    pnp::move_ik_plan_kernel<T, pnp::SpecKin><<<grid, block, 0, st>>>(a);
+    pnp::move_ik_plan_kernel<T, pnp::SpecKin><<<g.grid, block, 0, st>>>(a);
   else
-    pnp::move_ik_plan_kernel<T, pnp::GenericKin><<<grid, block, 0, st>>>(a);
+    pnp::move_ik_plan_kernel<T, pnp::GenericKin><<<g.grid, block, 0, st>>>(a);
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return PNP_OK;
@@ -1362,13 +1369,7 @@ int pnp_her_relabel_table_f32(const float* obs, const float* next_obs, const int
   }
   cudaStream_t st = (cudaStream_t)stream;
   const size_t smem_bulk = 2 * 2 * pnp::HER_TILE_BYTES, smem_plain = 2 * pnp::HER_TILE_BYTES;
-  static bool attr_set[kMaxDevices] = {};
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  if (!attr_set[dev]) {
-    CUDA_TRY(cudaFuncSetAttribute(pnp::her_relabel_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bulk));
-    attr_set[dev] = true;
-  }
+  if ((rc = max_dynamic_smem<pnp::her_relabel_kernel<true>>(s, smem_bulk))) return rc;
   const bool bulk_ok = aligned16(obs) && aligned16(next_obs) && aligned16(out_obs) && aligned16(out_next_obs);
   const int64_t full = bulk_ok ? (n / pnp::HER_TILE) * pnp::HER_TILE : 0;
   if (full > 0) {

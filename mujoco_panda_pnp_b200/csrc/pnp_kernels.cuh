@@ -174,8 +174,8 @@ struct IkArgs {
   unsigned* ticket;   // zeroed before launch
   unsigned chunk;     // queries a warp reserves per ticket atomic (>= 32)
   unsigned flush_min; // ik_solve_v_kernel: lanes with a finished slot that trigger a store + refill
-  unsigned solo_warp; // ik_solve_v_kernel, small batches: the block has 4 warps to load the 40 KB trig table quickly,
-                      // only warp 0 solves (one warp per block spreads a small batch over all SMs)
+  unsigned solo_warp; // small batches: the block has 4 warps to load the 40 KB trig table quickly, only warp 0 solves
+                      // (one warp per block spreads a small batch over all SMs); every persistent IK-family kernel
   unsigned tail;      // ik_solve_v_kernel<F2>: finish the block's last stragglers in the one-query-per-lane latency loop
   unsigned guided;    // ik_solve_v_kernel: 0 = fixed ticket chunks; else a reservation is (queries left) / guided, within [32 S, chunk]
   T thresh2;          // pos_thresh^2, squared on the host in T: read straight from the constant bank by the per-pass compare
@@ -192,6 +192,68 @@ struct IkArgs {
   unsigned* park_slots;   // slots written
   unsigned* zero_next[3]; // resume kernel: the counters the NEXT launch pair of this stream will use, zeroed by block 0
 };
+
+// Warp-local pool of reserved query indices [next, end) of the persistent IK-family kernels: one ticket atomic reserves
+// `chunk` consecutive queries, lanes then draw from the pool without touching global memory.  (A per-refill atomic on the
+// single ticket address serialises in L2 at ~1 op/clk and capped ik_solve_kernel at ~3.3 G solves/s regardless of its
+// instruction count.)  ik_solve_v_kernel keeps its own copy: guided chunks, the dry-pool hand-over.
+struct WarpPool {
+  unsigned next = 0, end = 0;
+
+  // Every slot k of this lane with want[k] draws the next index: ranks are slot-major over the warp (all slot-0 draws,
+  // then slot 1), and the warp reserves a fresh chunk when the pool holds fewer indices than it draws.  take(k, idx)
+  // runs for each draw below n.  A slot that draws an index >= n sets the lane's `exhausted` latch: the ticket is past
+  // the batch, and the caller's want[] stops asking for this lane.
+  template <int S, typename Take>
+  __device__ __forceinline__ void refill(const bool (&want)[S], bool& exhausted, unsigned n, unsigned* ticket, unsigned chunk,
+                                         Take take) {
+    const unsigned lane = threadIdx.x & 31u;
+    const unsigned lanemask_lt = (1u << lane) - 1u;
+    unsigned need[S], count = 0;
+#pragma unroll
+    for (int k = 0; k < S; ++k) {
+      need[k] = __ballot_sync(FULL, want[k]);
+      count += (unsigned)__popc(need[k]);
+    }
+    if (count) {
+      bool ran_out = false;
+      const unsigned avail = end - next;
+      unsigned fresh = 0;
+      if (count > avail) {  // warp-uniform
+        if (lane == 0) fresh = atomicAdd(ticket, chunk);
+        fresh = __shfl_sync(FULL, fresh, 0);
+      }
+      unsigned before = 0;
+#pragma unroll
+      for (int k = 0; k < S; ++k) {
+        if (want[k]) {
+          const unsigned rank = before + (unsigned)__popc(need[k] & lanemask_lt);
+          const unsigned idx = rank < avail ? next + rank : fresh + (rank - avail);
+          if (idx < n) take(k, idx);
+          else ran_out = true;
+        }
+        before += (unsigned)__popc(need[k]);
+      }
+      if (count > avail) { next = fresh + (count - avail); end = fresh + chunk; }
+      else next += count;
+      exhausted = exhausted || ran_out;
+    }
+  }
+};
+
+// End of a persistent IK-family kernel: the warp's query, convergence and iteration counts into counters[] (nullable).
+// Every solver here counts success == converged (SURVEY App. D.2).
+__device__ __forceinline__ void ik_counters_add(unsigned long long* counters, unsigned long long c_n,
+                                                unsigned long long c_conv, unsigned long long c_iter) {
+  if (!counters) return;
+  c_n = warp_sum(c_n); c_conv = warp_sum(c_conv); c_iter = warp_sum(c_iter);
+  if ((threadIdx.x & 31u) == 0) {
+    atomicAdd(counters + PNP_IK_CNT_N, c_n);
+    atomicAdd(counters + PNP_IK_CNT_CONVERGED, c_conv);
+    atomicAdd(counters + PNP_IK_CNT_SUCCESS, c_conv);
+    atomicAdd(counters + PNP_IK_CNT_ITERATIONS, c_iter);
+  }
+}
 
 // Back-to-back launches of ik_solve_v_kernel on one stream overlap the drain of launch k with the ramp of launch k+1
 // (programmatic dependent launch).  A launch's last ~0.09 ms are its drain: the ticket pool is dry and every block waits
@@ -279,7 +341,6 @@ __device__ __forceinline__ void ik_store(const IkArgs<T>& a, unsigned idx, const
 
 template <typename T, typename Kin, int kOut>
 __global__ void __launch_bounds__(IK_BLOCK) ik_solve_kernel(const IkArgs<T> a) {
-  const unsigned lane = threadIdx.x & 31u;
   __shared__ __align__(16) T s_q0[8];  // broadcast q_init: refills read it from shared memory
   __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
   if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
@@ -287,7 +348,6 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_solve_kernel(const IkArgs<T> a) {
   __syncthreads();
   if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
   const Trig<T> trig{s_tab};
-  const unsigned lanemask_lt = (1u << lane) - 1u;
 
   T q[NJ], tgt[3];
   int it = 0;
@@ -298,51 +358,26 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_solve_kernel(const IkArgs<T> a) {
 #pragma unroll
   for (int i = 0; i < NJ; ++i) q[i] = T(0);
   tgt[0] = tgt[1] = tgt[2] = T(0);
-
-  // Warp-local pool of reserved query indices [pool_next, pool_end): one ticket atomic reserves
-  // a.chunk consecutive queries, lanes then draw from the pool without touching global memory.
-  // (A per-refill atomic on the single ticket address serialises in L2 at ~1 op/clk and capped
-  // the whole kernel at ~3.3 G solves/s regardless of its instruction count.)
-  unsigned pool_next = 0, pool_end = 0;
+  WarpPool pool;
 
   while (true) {
     // ---- refill idle lanes -------------------------------------------------------------
-    const unsigned need = __ballot_sync(FULL, !active && !exhausted);
-    if (need) {
-      const unsigned count = (unsigned)__popc(need);
-      const unsigned avail = pool_end - pool_next;
-      unsigned fresh = 0;
-      if (count > avail) {  // warp-uniform
-        if (lane == 0) fresh = atomicAdd(a.ticket, a.chunk);
-        fresh = __shfl_sync(FULL, fresh, 0);
-      }
-      if (!active && !exhausted) {
-        const unsigned rank = (unsigned)__popc(need & lanemask_lt);
-        idx = rank < avail ? pool_next + rank : fresh + (rank - avail);
-        if (idx < a.n) {
+    const bool want[1] = {!active && !exhausted};
+    pool.refill(want, exhausted, a.n, a.ticket, a.chunk, [&](int, unsigned i) {
+          idx = i;
           const T* tp = a.targets + (size_t)idx * 3u;
           tgt[0] = tp[0]; tgt[1] = tp[1]; tgt[2] = tp[2];
           if (a.q_init_stride == 0) {
 #pragma unroll
-            for (int i = 0; i < NJ; ++i) q[i] = s_q0[i];
+            for (int j = 0; j < NJ; ++j) q[j] = s_q0[j];
           } else {
             const T* qi = a.q_init + (size_t)idx * NJ;
 #pragma unroll
-            for (int i = 0; i < NJ; ++i) q[i] = qi[i];
+            for (int j = 0; j < NJ; ++j) q[j] = qi[j];
           }
           it = 0;
           active = true;
-        } else {
-          exhausted = true;
-        }
-      }
-      if (count > avail) {
-        pool_next = fresh + (count - avail);
-        pool_end = fresh + a.chunk;
-      } else {
-        pool_next += count;
-      }
-    }
+        });
     if (!__any_sync(FULL, active)) break;
 
     // ---- one DLS pass for all lanes ----------------------------------------------------
@@ -360,17 +395,7 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_solve_kernel(const IkArgs<T> a) {
     for (int i = 0; i < NJ; ++i) q[i] = qn[i];
     ++it;
   }
-
-  if (a.counters) {
-    const unsigned long long w_n = warp_sum((unsigned long long)c_n), w_conv = warp_sum((unsigned long long)c_conv),
-                             w_iter = warp_sum(c_iter);
-    if (lane == 0) {
-      atomicAdd(a.counters + PNP_IK_CNT_N, w_n);
-      atomicAdd(a.counters + PNP_IK_CNT_CONVERGED, w_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_SUCCESS, w_conv);  // success == converged (SURVEY App. D.2)
-      atomicAdd(a.counters + PNP_IK_CNT_ITERATIONS, w_iter);
-    }
-  }
+  ik_counters_add(a.counters, c_n, c_conv, c_iter);
 }
 
 // =============================================================================================
@@ -1261,7 +1286,7 @@ struct WaypointArgs {
   unsigned long long* counters;
   unsigned* ticket; // zeroed before launch
   unsigned chunk;   // envs a warp reserves per ticket atomic
-  unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works (see IkArgs)
+  unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works
 };
 
 // The two loop levels (waypoints x DLS passes) are FLATTENED and the lanes are PERSISTENT: every pass
@@ -1274,16 +1299,14 @@ struct WaypointArgs {
 // some lane of nearly every warp, and envs need 10-50 waypoints, so lanes idled for 1/3 of the passes.)
 template <typename T, typename Kin>
 __global__ void __launch_bounds__(IK_BLOCK) ik_waypoints_kernel(const WaypointArgs<T> a) {
-  const unsigned lane = threadIdx.x & 31u;
   __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
   if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
   __syncthreads();
   if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
   const Trig<T> trig{s_tab};
-  const unsigned lanemask_lt = (1u << lane) - 1u;
   enum { IDLE = 0, INIT = 1, RUN = 2 };
   unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
-  unsigned pool_next = 0, pool_end = 0;
+  WarpPool pool;
   bool exhausted = false;
   unsigned e = 0;
   int state = IDLE;
@@ -1315,19 +1338,8 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_waypoints_kernel(const WaypointAr
 
   while (true) {
     // ---- refill idle lanes ------------------------------------------------------------------
-    const unsigned need = __ballot_sync(FULL, state == IDLE && !exhausted);
-    if (need) {
-      const unsigned count = (unsigned)__popc(need);
-      const unsigned avail = pool_end - pool_next;
-      unsigned fresh = 0;
-      if (count > avail) {
-        if (lane == 0) fresh = atomicAdd(a.ticket, a.chunk);
-        fresh = __shfl_sync(FULL, fresh, 0);
-      }
-      if (state == IDLE && !exhausted) {
-        const unsigned rank = (unsigned)__popc(need & lanemask_lt);
-        const unsigned idx = rank < avail ? pool_next + rank : fresh + (rank - avail);
-        if (idx < a.n) {
+    const bool want[1] = {state == IDLE && !exhausted};
+    pool.refill(want, exhausted, a.n, a.ticket, a.chunk, [&](int, unsigned idx) {
           e = idx;
 #pragma unroll
           for (int i = 0; i < NJ; ++i) q[i] = qs[i] = a.q_start[(size_t)e * NJ + i];
@@ -1335,13 +1347,7 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_waypoints_kernel(const WaypointAr
           for (int i = 0; i < 3; ++i) goal[i] = a.goal[(size_t)e * 3 + i];
           step = 0; accepted = 0; iters_sum = 0; fails = 0;
           state = INIT;
-        } else {
-          exhausted = true;
-        }
-      }
-      if (count > avail) { pool_next = fresh + (count - avail); pool_end = fresh + a.chunk; }
-      else pool_next += count;
-    }
+        });
     if (!__any_sync(FULL, state != IDLE)) break;
 
     // ---- one DLS pass for all lanes -------------------------------------------------------------
@@ -1389,15 +1395,7 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_waypoints_kernel(const WaypointAr
       state = IDLE;
     }
   }
-  if (a.counters) {
-    c_n = warp_sum(c_n); c_conv = warp_sum(c_conv); c_iter = warp_sum(c_iter);
-    if (lane == 0) {
-      atomicAdd(a.counters + PNP_IK_CNT_N, c_n);
-      atomicAdd(a.counters + PNP_IK_CNT_CONVERGED, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_SUCCESS, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_ITERATIONS, c_iter);
-    }
-  }
+  ik_counters_add(a.counters, c_n, c_conv, c_iter);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1413,14 +1411,12 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_waypoints_kernel(const WaypointAr
 template <typename V, bool kFuse>
 __global__ void __launch_bounds__(IK_BLOCK, Slots<V>::kN == 2 ? IK_PAIR_MIN_BLOCKS : 1) ik_waypoints_v_kernel(const WaypointArgs<float> a) {
   constexpr int S = Slots<V>::kN;
-  const unsigned lane = threadIdx.x & 31u;
   __shared__ __align__(16) float s_trig[kTrigVWords];
   __shared__ float s_qa[S * NJ * IK_BLOCK];  // accepted q of every slot: [(k * NJ + i) * IK_BLOCK + thread]
   load_trigv_table(s_trig);
   __syncthreads();
   if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
   const TrigV trig{s_trig};
-  const unsigned lanemask_lt = (1u << lane) - 1u;
   const float thresh2 = a.k.pos_thresh * a.k.pos_thresh;
   float* const qa = s_qa + threadIdx.x;
   enum { IDLE = 0, INIT = 1, RUN = 2 };
@@ -1430,7 +1426,7 @@ __global__ void __launch_bounds__(IK_BLOCK, Slots<V>::kN == 2 ? IK_PAIR_MIN_BLOC
   unsigned env[S];
   bool exhausted = false;
   unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
-  unsigned pool_next = 0, pool_end = 0;
+  WarpPool pool;
 #pragma unroll
   for (int i = 0; i < NJ; ++i) qs[i] = V(0.0f);
 #pragma unroll
@@ -1439,49 +1435,23 @@ __global__ void __launch_bounds__(IK_BLOCK, Slots<V>::kN == 2 ? IK_PAIR_MIN_BLOC
   for (int k = 0; k < S; ++k) { state[k] = IDLE; step[k] = it[k] = accepted[k] = iters_sum[k] = fails[k] = 0; env[k] = 0; }
 
   while (true) {
-    // ---- refill idle slots (slot-major ranks) ------------------------------------------------------
-    unsigned need[S], count = 0;
+    // ---- refill idle slots ---------------------------------------------------------------------------
+    bool want[S];
 #pragma unroll
-    for (int k = 0; k < S; ++k) {
-      need[k] = __ballot_sync(FULL, state[k] == IDLE && !exhausted);
-      count += (unsigned)__popc(need[k]);
-    }
-    if (count) {
-      const unsigned avail = pool_end - pool_next;
-      unsigned fresh = 0;
-      if (count > avail) {
-        if (lane == 0) fresh = atomicAdd(a.ticket, a.chunk);
-        fresh = __shfl_sync(FULL, fresh, 0);
-      }
-      unsigned before = 0;
-      bool ran_out = false;
+    for (int k = 0; k < S; ++k) want[k] = state[k] == IDLE && !exhausted;
+    pool.refill(want, exhausted, a.n, a.ticket, a.chunk, [&](int k, unsigned id) {
+          env[k] = id;
 #pragma unroll
-      for (int k = 0; k < S; ++k) {
-        if (state[k] == IDLE && !exhausted) {
-          const unsigned rank = before + (unsigned)__popc(need[k] & lanemask_lt);
-          const unsigned id = rank < avail ? pool_next + rank : fresh + (rank - avail);
-          if (id < a.n) {
-            env[k] = id;
-#pragma unroll
-            for (int i = 0; i < NJ; ++i) {
-              const float v = a.q_start[(size_t)id * NJ + i];
-              Slots<V>::set(qs[i], k, v);
-              qa[(k * NJ + i) * IK_BLOCK] = v;
-            }
-#pragma unroll
-            for (int i = 0; i < 3; ++i) Slots<V>::set(goal[i], k, a.goal[(size_t)id * 3 + i]);
-            step[k] = 0; accepted[k] = 0; iters_sum[k] = 0; fails[k] = 0; it[k] = 0;
-            state[k] = INIT;
-          } else {
-            ran_out = true;
+          for (int i = 0; i < NJ; ++i) {
+            const float v = a.q_start[(size_t)id * NJ + i];
+            Slots<V>::set(qs[i], k, v);
+            qa[(k * NJ + i) * IK_BLOCK] = v;
           }
-        }
-        before += (unsigned)__popc(need[k]);
-      }
-      exhausted = exhausted || ran_out;
-      if (count > avail) { pool_next = fresh + (count - avail); pool_end = fresh + a.chunk; }
-      else pool_next += count;
-    }
+#pragma unroll
+          for (int i = 0; i < 3; ++i) Slots<V>::set(goal[i], k, a.goal[(size_t)id * 3 + i]);
+          step[k] = 0; accepted[k] = 0; iters_sum[k] = 0; fails[k] = 0; it[k] = 0;
+          state[k] = INIT;
+        });
     bool any_live = false;
 #pragma unroll
     for (int k = 0; k < S; ++k) any_live = any_live || state[k] != IDLE;
@@ -1607,15 +1577,7 @@ __global__ void __launch_bounds__(IK_BLOCK, Slots<V>::kN == 2 ? IK_PAIR_MIN_BLOC
       }
     }
   }
-  if (a.counters) {
-    c_n = warp_sum(c_n); c_conv = warp_sum(c_conv); c_iter = warp_sum(c_iter);
-    if (lane == 0) {
-      atomicAdd(a.counters + PNP_IK_CNT_N, c_n);
-      atomicAdd(a.counters + PNP_IK_CNT_CONVERGED, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_SUCCESS, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_ITERATIONS, c_iter);
-    }
-  }
+  ik_counters_add(a.counters, c_n, c_conv, c_iter);
 }
 
 // =============================================================================================
@@ -1646,7 +1608,7 @@ struct PoseIkArgs {
   unsigned long long* counters;
   unsigned* ticket; // zeroed before launch
   unsigned chunk;   // queries a warp reserves per ticket atomic
-  unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works (see IkArgs)
+  unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works
 };
 
 // mju_quat2Vel(res, quat, 1): rotation vector of a unit quaternion, angle folded into (-pi, pi]
@@ -1818,15 +1780,13 @@ __device__ __forceinline__ void pose_store(const PoseIkArgs<T>& a, unsigned e, c
 // instruction, twice the mean pass count).  The FP32 instantiation uses the table trig.
 template <typename T, typename Kin>
 __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArgs<T> a) {
-  const unsigned lane = threadIdx.x & 31u;
   __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
   if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
   __syncthreads();
   if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
   const Trig<T> trig{s_tab};
-  const unsigned lanemask_lt = (1u << lane) - 1u;
   unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
-  unsigned pool_next = 0, pool_end = 0;
+  WarpPool pool;
   bool exhausted = false, active = false;
   unsigned e = 0;
   int it = 0;
@@ -1836,19 +1796,8 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArg
 
   while (true) {
     // ---- refill idle lanes -------------------------------------------------------------------
-    const unsigned need = __ballot_sync(FULL, !active && !exhausted);
-    if (need) {
-      const unsigned count = (unsigned)__popc(need);
-      const unsigned avail = pool_end - pool_next;
-      unsigned fresh = 0;
-      if (count > avail) {
-        if (lane == 0) fresh = atomicAdd(a.ticket, a.chunk);
-        fresh = __shfl_sync(FULL, fresh, 0);
-      }
-      if (!active && !exhausted) {
-        const unsigned rank = (unsigned)__popc(need & lanemask_lt);
-        const unsigned idx = rank < avail ? pool_next + rank : fresh + (rank - avail);
-        if (idx < a.n) {
+    const bool want[1] = {!active && !exhausted};
+    pool.refill(want, exhausted, a.n, a.ticket, a.chunk, [&](int, unsigned idx) {
           e = idx;
           const T* qi = a.q_init + (size_t)a.q_init_stride * e;
 #pragma unroll
@@ -1856,13 +1805,7 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArg
           pose_load_target(a, e, tp, tq);
           it = 0;
           active = true;
-        } else {
-          exhausted = true;
-        }
-      }
-      if (count > avail) { pool_next = fresh + (count - avail); pool_end = fresh + a.chunk; }
-      else pool_next += count;
-    }
+        });
     if (!__any_sync(FULL, active)) break;
 
     // ---- one 6-row DLS pass for all lanes (a lane that just finished is idle and is overwritten by the next refill) --
@@ -1874,15 +1817,7 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_pose_solve_kernel(const PoseIkArg
                       });
     ++it;
   }
-  if (a.counters) {
-    c_n = warp_sum(c_n); c_conv = warp_sum(c_conv); c_iter = warp_sum(c_iter);
-    if (lane == 0) {
-      atomicAdd(a.counters + PNP_IK_CNT_N, c_n);
-      atomicAdd(a.counters + PNP_IK_CNT_CONVERGED, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_SUCCESS, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_ITERATIONS, c_iter);
-    }
-  }
+  ik_counters_add(a.counters, c_n, c_conv, c_iter);
 }
 
 // ---- multi-start pose IK (pnp_ik_pose_solve_multistart_*) ---------------------------------------------------------
@@ -1964,7 +1899,7 @@ struct MoveArgs {
   unsigned long long* counters;
   unsigned* ticket; // zeroed before launch
   unsigned chunk;   // envs a warp reserves per ticket atomic
-  unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works (see IkArgs)
+  unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works
   const unsigned* order;  // nullable: env taken by the i-th ticket (longest plans first, plan_order_* kernels below)
   const float4* records;  // nullable (FP32 value-type kernel): the i-th ticket's inputs as one 48-byte record
                           // {q_start[7], target[3], env, -}, written in plan order by plan_order_scatter_kernel: a refill is
@@ -2099,16 +2034,14 @@ __device__ __forceinline__ float divmul(float a, float c, float b) { return a * 
 // and unreachable goals no longer runs at the pace of its capped envs.
 template <typename T, typename Kin>
 __global__ void __launch_bounds__(IK_BLOCK) move_ik_plan_kernel(const MoveArgs<T> a) {
-  const unsigned lane = threadIdx.x & 31u;
   __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
   if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
   __syncthreads();
   if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
   const Trig<T> trig{s_tab};
-  const unsigned lanemask_lt = (1u << lane) - 1u;
   enum { NORMAL = 0, FB1 = 1, FB2 = 2, DONE = 3, INIT = 4, IDLE = 5 };
   unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
-  unsigned pool_next = 0, pool_end = 0;
+  WarpPool pool;
   bool exhausted = false;
   unsigned e = 0;
   T q[NJ], qs[NJ], goal[3] = {T(0), T(0), T(0)}, pos[3] = {T(0), T(0), T(0)}, tgt[3] = {T(0), T(0), T(0)};
@@ -2134,19 +2067,8 @@ __global__ void __launch_bounds__(IK_BLOCK) move_ik_plan_kernel(const MoveArgs<T
       if (a.status) a.status[e] = st;
       state = IDLE;
     }
-    const unsigned need = __ballot_sync(FULL, state == IDLE && !exhausted);
-    if (need) {
-      const unsigned count = (unsigned)__popc(need);
-      const unsigned avail = pool_end - pool_next;
-      unsigned fresh = 0;
-      if (count > avail) {
-        if (lane == 0) fresh = atomicAdd(a.ticket, a.chunk);
-        fresh = __shfl_sync(FULL, fresh, 0);
-      }
-      if (state == IDLE && !exhausted) {
-        const unsigned rank = (unsigned)__popc(need & lanemask_lt);
-        const unsigned idx = rank < avail ? pool_next + rank : fresh + (rank - avail);
-        if (idx < a.n) {
+    const bool want[1] = {state == IDLE && !exhausted};
+    pool.refill(want, exhausted, a.n, a.ticket, a.chunk, [&](int, unsigned idx) {
           const unsigned eo = a.order ? a.order[idx] : idx;
           if (eo < a.n) {  // an out-of-range entry of a caller-made order is skipped: nothing is read or written for it
             e = eo;
@@ -2158,13 +2080,7 @@ __global__ void __launch_bounds__(IK_BLOCK) move_ik_plan_kernel(const MoveArgs<T
             len = 0; solves = 0; st = 0; point_count = 0; cf = 0; outer = 0; astep = T(0);
             state = INIT;
           }
-        } else {
-          exhausted = true;
-        }
-      }
-      if (count > avail) { pool_next = fresh + (count - avail); pool_end = fresh + a.chunk; }
-      else pool_next += count;
-    }
+        });
     if (!__any_sync(FULL, state != IDLE)) break;
 
     // ---- one DLS pass for all lanes (ik_solver.py:58-83); INIT lanes only take FK(q_start) from it ----
@@ -2267,15 +2183,7 @@ __global__ void __launch_bounds__(IK_BLOCK) move_ik_plan_kernel(const MoveArgs<T
       it = 0;
     }
   }
-  if (a.counters) {
-    c_n = warp_sum(c_n); c_conv = warp_sum(c_conv); c_iter = warp_sum(c_iter);
-    if (lane == 0) {
-      atomicAdd(a.counters + PNP_IK_CNT_N, c_n);
-      atomicAdd(a.counters + PNP_IK_CNT_CONVERGED, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_SUCCESS, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_ITERATIONS, c_iter);
-    }
-  }
+  ik_counters_add(a.counters, c_n, c_conv, c_iter);
 }
 
 // =============================================================================================
@@ -2540,7 +2448,6 @@ template <typename V, bool kFuse, int kBlock = IK_BLOCK, bool kStage = false>
 __global__ void __launch_bounds__(kBlock, (Slots<V>::kN == 2 || kBlock == PLAN_BLOCK) ? IK_PAIR_MIN_BLOCKS : 5) move_ik_plan_v_kernel(const MoveArgs<float> a) {
   constexpr int S = Slots<V>::kN;
   static_assert(!kStage || S == 1, "trajectory staging is written for one env per lane");
-  const unsigned lane = threadIdx.x & 31u;
   // dynamic shared memory (the staged variant needs 53 KB, above the 48 KB a kernel may declare statically): plan_smem_bytes()
   extern __shared__ __align__(16) unsigned char plan_smem[];
   float* const s_trig = reinterpret_cast<float*>(plan_smem);
@@ -2550,7 +2457,6 @@ __global__ void __launch_bounds__(kBlock, (Slots<V>::kN == 2 || kBlock == PLAN_B
   __syncthreads();
   if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
   const TrigV trig{s_trig};
-  const unsigned lanemask_lt = (1u << lane) - 1u;
   const float thresh2 = a.k.pos_thresh * a.k.pos_thresh;
   float* const qa = s_qa + threadIdx.x;
   enum { NORMAL = 0, FB1 = 1, FB2 = 2, DONE = 3, INIT = 4, IDLE = 5 };
@@ -2561,7 +2467,7 @@ __global__ void __launch_bounds__(kBlock, (Slots<V>::kN == 2 || kBlock == PLAN_B
   unsigned env[S];
   bool exhausted = false;
   unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
-  unsigned pool_next = 0, pool_end = 0;
+  WarpPool pool;
 #pragma unroll
   for (int i = 0; i < NJ; ++i) qs[i] = V(0.0f);
 #pragma unroll
@@ -2620,65 +2526,39 @@ __global__ void __launch_bounds__(kBlock, (Slots<V>::kN == 2 || kBlock == PLAN_B
         state[k] = IDLE;
       }
     }
-    unsigned need[S], count = 0;
+    bool want[S];
 #pragma unroll
-    for (int k = 0; k < S; ++k) {
-      need[k] = __ballot_sync(FULL, state[k] == IDLE && !exhausted);
-      count += (unsigned)__popc(need[k]);
-    }
-    if (count) {
-      const unsigned avail = pool_end - pool_next;
-      unsigned fresh = 0;
-      if (count > avail) {
-        if (lane == 0) fresh = atomicAdd(a.ticket, a.chunk);
-        fresh = __shfl_sync(FULL, fresh, 0);
-      }
-      unsigned before = 0;
-      bool ran_out = false;
-#pragma unroll
-      for (int k = 0; k < S; ++k) {
-        if (state[k] == IDLE && !exhausted) {
-          const unsigned rank = before + (unsigned)__popc(need[k] & lanemask_lt);
-          const unsigned id = rank < avail ? pool_next + rank : fresh + (rank - avail);
-          if (id < a.n) {
-            float rec[12];
-            unsigned e;
-            if (a.records) {  // warp-uniform
-              const float4 r0 = a.records[(size_t)id * 3u], r1 = a.records[(size_t)id * 3u + 1], r2 = a.records[(size_t)id * 3u + 2];
-              rec[0] = r0.x; rec[1] = r0.y; rec[2] = r0.z; rec[3] = r0.w; rec[4] = r1.x; rec[5] = r1.y; rec[6] = r1.z;
-              rec[7] = r1.w; rec[8] = r2.x; rec[9] = r2.y;
-              e = __float_as_uint(r2.z);
-            } else {
-              e = a.order ? a.order[id] : id;
-              if (e < a.n) {
-#pragma unroll
-                for (int i = 0; i < NJ; ++i) rec[i] = a.q_start[(size_t)e * NJ + i];
-#pragma unroll
-                for (int i = 0; i < 3; ++i) rec[7 + i] = a.target[(size_t)e * 3 + i];
-              }
-            }
-            if (e < a.n) {  // an out-of-range entry of a caller-made order is skipped: nothing is read or written for it
-              env[k] = e;
-#pragma unroll
-              for (int i = 0; i < NJ; ++i) {
-                Slots<V>::set(qs[i], k, rec[i]);
-                qa[(k * NJ + i) * kBlock] = rec[i];
-              }
-#pragma unroll
-              for (int i = 0; i < 3; ++i) Slots<V>::set(goal[i], k, rec[7 + i]);
-              len[k] = 0; solves[k] = 0; st[k] = 0; point_count[k] = 0; cf[k] = 0; outer[k] = 0; astep[k] = 0.0f; it[k] = 0;
-              state[k] = INIT;
-            }
+    for (int k = 0; k < S; ++k) want[k] = state[k] == IDLE && !exhausted;
+    pool.refill(want, exhausted, a.n, a.ticket, a.chunk, [&](int k, unsigned id) {
+          float rec[12];
+          unsigned e;
+          if (a.records) {  // warp-uniform
+            const float4 r0 = a.records[(size_t)id * 3u], r1 = a.records[(size_t)id * 3u + 1], r2 = a.records[(size_t)id * 3u + 2];
+            rec[0] = r0.x; rec[1] = r0.y; rec[2] = r0.z; rec[3] = r0.w; rec[4] = r1.x; rec[5] = r1.y; rec[6] = r1.z;
+            rec[7] = r1.w; rec[8] = r2.x; rec[9] = r2.y;
+            e = __float_as_uint(r2.z);
           } else {
-            ran_out = true;
+            e = a.order ? a.order[id] : id;
+            if (e < a.n) {
+#pragma unroll
+              for (int i = 0; i < NJ; ++i) rec[i] = a.q_start[(size_t)e * NJ + i];
+#pragma unroll
+              for (int i = 0; i < 3; ++i) rec[7 + i] = a.target[(size_t)e * 3 + i];
+            }
           }
-        }
-        before += (unsigned)__popc(need[k]);
-      }
-      exhausted = exhausted || ran_out;
-      if (count > avail) { pool_next = fresh + (count - avail); pool_end = fresh + a.chunk; }
-      else pool_next += count;
-    }
+          if (e < a.n) {  // an out-of-range entry of a caller-made order is skipped: nothing is read or written for it
+            env[k] = e;
+#pragma unroll
+            for (int i = 0; i < NJ; ++i) {
+              Slots<V>::set(qs[i], k, rec[i]);
+              qa[(k * NJ + i) * kBlock] = rec[i];
+            }
+#pragma unroll
+            for (int i = 0; i < 3; ++i) Slots<V>::set(goal[i], k, rec[7 + i]);
+            len[k] = 0; solves[k] = 0; st[k] = 0; point_count[k] = 0; cf[k] = 0; outer[k] = 0; astep[k] = 0.0f; it[k] = 0;
+            state[k] = INIT;
+          }
+        });
     bool any_live = false;
 #pragma unroll
     for (int k = 0; k < S; ++k) any_live = any_live || state[k] != IDLE;
@@ -2855,15 +2735,7 @@ __global__ void __launch_bounds__(kBlock, (Slots<V>::kN == 2 || kBlock == PLAN_B
       }
     }
   }
-  if (a.counters) {
-    c_n = warp_sum(c_n); c_conv = warp_sum(c_conv); c_iter = warp_sum(c_iter);
-    if (lane == 0) {
-      atomicAdd(a.counters + PNP_IK_CNT_N, c_n);
-      atomicAdd(a.counters + PNP_IK_CNT_CONVERGED, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_SUCCESS, c_conv);
-      atomicAdd(a.counters + PNP_IK_CNT_ITERATIONS, c_iter);
-    }
-  }
+  ik_counters_add(a.counters, c_n, c_conv, c_iter);
 }
 
 // =============================================================================================

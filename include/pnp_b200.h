@@ -16,6 +16,7 @@
  *   pnp_ik_pose_solve_*    FrankaEnv.solve_ik(target_pos, target_quat, q_init) (panda_env.py:399-409;
  *                          dangling in the reference - an extension defined here)
  *   pnp_move_ik_plan_*     the whole MoveIKSkill.reset planner (skills/move.py:76-191)
+ *   pnp_move_ik_plan_pose_*  the same planner to a goal position and orientation (an extension defined here)
  *   pnp_get_obs_*          FrankaEnv._get_obs (envs/panda_env.py:279-301) from kinematic state
  *   pnp_reward_*           FrankaEnv.compute_reward / _is_success / goal_distance
  *                          (envs/panda_env.py:205-245, 303-306, 311-315), row-wise
@@ -277,8 +278,9 @@ typedef struct PnpMoveParams {
   int32_t compute_order;    /* pnp_move_ik_plan_ordered_* only: 1 = `order` is scratch, fill it first
                                (pnp_move_plan_order_*) and then take the envs in that order; 0 = `order` is an input */
 } PnpMoveParams;
-#define PNP_MOVE_BROKE 1u      /* fallback strategies exhausted (reference `break`, move.py:178-180) */
-#define PNP_MOVE_CAPPED 2u     /* max_outer reached */
+#define PNP_MOVE_BROKE 1u      /* fallback strategies exhausted (reference `break`, move.py:178-180);
+                                  pose planner: three rejected solves in one round, or a non-finite / zero goal */
+#define PNP_MOVE_CAPPED 2u     /* max_outer reached; pose planner: max_traj_points points reached */
 #define PNP_MOVE_OVERFLOW 4u   /* more than traj_cap points: extra points dropped, traj_len still counts */
 /* Per env: q_start[n,7], target[n,3].  The whole adaptive-waypoint state machine (accept rule,
  * failure counting incl. the double increment, fallback strategies 1-3, final-point append) runs
@@ -323,6 +325,42 @@ int pnp_move_ik_plan_sorted_f32(const float* q_start, const float* target, void*
                                 const PnpMoveParams* move, const PnpIkParams* params, float* traj,
                                 int32_t* traj_len, float* q_final, int32_t* n_solves, int32_t* status,
                                 unsigned long long* counters, void* stream);
+
+/* ---- pose-mode move planner: plan to a goal position AND orientation (EXTENSION) ------------ */
+typedef struct PnpMovePoseParams {
+  double pos_thresh;       /* 0.01 m   the plan ends when |goal_pos - p| <= pos_thresh ...                        */
+  double rot_thresh;       /* 0.05 rad ... and the remaining rotation angle <= rot_thresh                        */
+  double step_size;        /* 0.01 m   largest translation per waypoint                                          */
+  double rot_step;         /* 0.05 rad largest rotation per waypoint                                             */
+  double ik_rot_thresh;    /* 0.01 rad rot_thresh of every pose solve (pnp_ik_pose_solve_*)                     */
+  double ik_rot_weight;    /* 1.0      rot_weight of every pose solve                                            */
+  int32_t max_traj_points; /* 200      solved waypoints at most                                                  */
+  int32_t traj_cap;        /* >= 1     points of storage per env; max_traj_points + 1 never overflows           */
+} PnpMovePoseParams;
+/* Per env: q_start[n,7], goal_pos[n,3], goal_quat[n,4] wxyz (normalised on load).  (p, r) = FK(q_start) (site position
+ * and quaternion) is point 0.  Each round: d = goal_pos - p, w = rotation vector of goal_quat (x) conj(r) (the pose
+ * solver's error, short path).  The plan ends with status 0 when |d| <= pos_thresh and |w| <= rot_thresh, and with
+ * PNP_MOVE_CAPPED after max_traj_points points.  Otherwise f = min(1, step_size / |d|, rot_step / |w|) and up to three
+ * pose solves (pnp_ik_pose_solve_* from the current q with `params`, ik_rot_thresh, ik_rot_weight) aim at the fractions
+ * f, f/2, f/20 of the remaining motion: (p + g d, quat(g w) (x) r), or exactly the goal when g == 1.  The first success
+ * appends its (final_pos, final_quat, q) and moves there; three rejections end the plan with PNP_MOVE_BROKE, as does a
+ * non-finite goal or a zero goal quaternion (then traj_len = 1).  The unreached goal is never appended: every point is a
+ * solved pose, and pos_traj, quat_traj and q_traj line up.  traj_len <= max_traj_points + 1, n_solves <=
+ * 3 max_traj_points; points past traj_cap are dropped and set PNP_MOVE_OVERFLOW (traj_len still counts them).
+ * Outputs: pos_traj[n,traj_cap,3], quat_traj[n,traj_cap,4], q_traj[n,traj_cap,7] (nullable), traj_len[n], q_final[n,7]
+ * (the joints of the last point), n_solves[n], status[n] (PNP_MOVE_* bits), counters[4] (nullable: every pose solve, as
+ * pnp_ik_pose_solve_*).  Rejected with PNP_EINVAL before anything is enqueued: pos_thresh < params->pos_thresh or
+ * rot_thresh < ik_rot_thresh (a solve converged short of the plan's tolerance would re-aim at the goal forever),
+ * step_size or rot_step <= 0, NULL outputs other than q_traj and counters, n >= 2^31.  The call never synchronises the
+ * host and can be captured in a CUDA graph.  The oracle is oracle/move_pose_oracle.py. */
+int pnp_move_ik_plan_pose_f32(const float* q_start, const float* goal_pos, const float* goal_quat, int64_t n,
+                              const PnpMovePoseParams* move, const PnpIkParams* params, float* pos_traj,
+                              float* quat_traj, float* q_traj, int32_t* traj_len, float* q_final, int32_t* n_solves,
+                              int32_t* status, unsigned long long* counters, void* stream);
+int pnp_move_ik_plan_pose_f64(const double* q_start, const double* goal_pos, const double* goal_quat, int64_t n,
+                              const PnpMovePoseParams* move, const PnpIkParams* params, double* pos_traj,
+                              double* quat_traj, double* q_traj, int32_t* traj_len, double* q_final, int32_t* n_solves,
+                              int32_t* status, unsigned long long* counters, void* stream);
 
 /* ---- compute_reward / _is_success, row-wise --------------------------------------------- */
 /* Per row: achieved_goal[n,3], desired_goal[n,3], ee_pos[n,3], ee_quat[n,4] wxyz,

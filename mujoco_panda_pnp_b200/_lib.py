@@ -55,6 +55,19 @@ class PnpMoveParams(ctypes.Structure):
     ]
 
 
+class PnpMovePoseParams(ctypes.Structure):
+    _fields_ = [
+        ("pos_thresh", c_double),
+        ("rot_thresh", c_double),
+        ("step_size", c_double),
+        ("rot_step", c_double),
+        ("ik_rot_thresh", c_double),
+        ("ik_rot_weight", c_double),
+        ("max_traj_points", c_int32),
+        ("traj_cap", c_int32),
+    ]
+
+
 class PnpNormalizeParams(ctypes.Structure):
     _fields_ = [
         ("mean", c_double * 25),
@@ -109,6 +122,10 @@ SIGNATURES = {
     "pnp_move_ik_plan_ordered_f32": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMoveParams), POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_ik_plan_sorted_f32": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMoveParams), POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_ik_plan_ordered_f64": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMoveParams), POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_move_ik_plan_pose_f32": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMovePoseParams), POINTER(PnpIkParams), _P, _P, _P, _P,
+                                          _P, _P, _P, _P, _P]),
+    "pnp_move_ik_plan_pose_f64": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMovePoseParams), POINTER(PnpIkParams), _P, _P, _P, _P,
+                                          _P, _P, _P, _P, _P]),
     "pnp_reward_f32": (c_int, [_P, _P, _P, _P, _P, _P, c_int64, POINTER(PnpRewardParams), _P, _P, _P, _P]),
     "pnp_reward_f64": (c_int, [_P, _P, _P, _P, _P, _P, c_int64, POINTER(PnpRewardParams), _P, _P, _P, _P]),
     "pnp_get_obs_f32": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int32, c_int64, c_double, _P, c_int32, _P]),

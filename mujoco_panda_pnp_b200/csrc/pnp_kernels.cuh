@@ -2187,6 +2187,193 @@ __global__ void __launch_bounds__(IK_BLOCK) move_ik_plan_kernel(const MoveArgs<T
 }
 
 // =============================================================================================
+// Pose-mode move planner (pnp_move_ik_plan_pose_*, an EXTENSION stated in oracle/move_pose_oracle.py): plan a move to
+// a goal position AND orientation, every waypoint a solved pose with its joints.
+//   round: d = goal_pos - p, w = quat2vel(goal_quat (x) conj(r)); done when |d| <= pos_thresh and |w| <= rot_thresh,
+//          CAPPED at max_traj_points points; f = min(1, step_size / |d|, rot_step / |w|)
+//   up to three pose solves from q at the fractions f, f/2, f/20 of (d, w) (the goal itself when the fraction is 1);
+//   the first success appends (final_pos, final_quat, q) and moves there; three rejections: BROKE.
+// Same lane machinery as move_ik_plan_kernel: one env per lane, persistent warps refilled from WarpPool, one shared
+// pose_pass per warp trip.  Every waypoint solve is pose_pass / pose_success unchanged, i.e. the plain pose solve of
+// that aim from that q (ik_pose_solve_kernel's arithmetic).  A fresh env enters as INIT with its pass number set to
+// max_iters: the pass then ends at once and hands the lane FK(q_start) - no divergent FK.
+// =============================================================================================
+template <typename T>
+struct MovePoseArgs {
+  PoseIkArgs<T> ik;  // every waypoint's pose solve: k, rot_thresh (= ik_rot_thresh), rot_weight; target_pos /
+                     // target_quat = the goals (pose_load_target); n, counters, ticket, chunk, solo_warp
+  const T* q_start;
+  T pos_thresh, rot_thresh, step_size, rot_step;
+  int max_traj_points, traj_cap;
+  T* pos_traj;       // [n][traj_cap][3]
+  T* quat_traj;      // [n][traj_cap][4]
+  T* q_traj;         // [n][traj_cap][7], nullable
+  int32_t* traj_len;
+  T* q_final;        // [n][7]
+  int32_t* n_solves;
+  int32_t* status;
+};
+
+// a / b: FP64 literally, FP32 on one MUFU.RCP (the planner's bookkeeping, as muldiv / divmul above)
+__device__ __forceinline__ double div_fast(double a, double b) { return a / b; }
+__device__ __forceinline__ float div_fast(float a, float b) { return a * rcp_approx(b); }
+
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(IK_BLOCK) move_pose_plan_kernel(const MovePoseArgs<T> a) {
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  if (a.ik.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
+  const Trig<T> trig{s_tab};
+  enum { SOLVE = 0, DONE = 1, INIT = 2, IDLE = 3 };
+  unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
+  WarpPool pool;
+  bool exhausted = false, bad_goal = false;
+  unsigned e = 0;
+  size_t row = 0;  // e * traj_cap
+  // q: joints of the last point; qs: the running solve; (p, r): pose of the last point; (tp, tq): the running aim
+  T q[NJ], qs[NJ], p[3] = {T(0), T(0), T(0)}, r[4] = {T(1), T(0), T(0), T(0)};
+  T gp[3] = {T(0), T(0), T(0)}, gq[4] = {T(1), T(0), T(0), T(0)}, tp[3] = {T(0), T(0), T(0)}, tq[4] = {T(1), T(0), T(0), T(0)};
+#pragma unroll
+  for (int i = 0; i < NJ; ++i) q[i] = qs[i] = T(0);
+  int len = 0, solves = 0, st = 0, state = IDLE, it = 0, points = 0, attempt = 0;
+  auto append = [&]() {
+    if (len < a.traj_cap) {
+      const size_t k = row + (size_t)len;
+#pragma unroll
+      for (int i = 0; i < 3; ++i) a.pos_traj[k * 3 + i] = p[i];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) a.quat_traj[k * 4 + i] = r[i];
+      if (a.q_traj) {
+#pragma unroll
+        for (int i = 0; i < NJ; ++i) a.q_traj[k * NJ + i] = q[i];
+      }
+    } else {
+      st |= (int)PNP_MOVE_OVERFLOW;
+    }
+    ++len;
+  };
+
+  while (true) {
+    // ---- write back finished envs, refill idle lanes -------------------------------------------
+    if (state == DONE) {
+#pragma unroll
+      for (int i = 0; i < NJ; ++i) a.q_final[(size_t)e * NJ + i] = q[i];
+      a.traj_len[e] = len;
+      a.n_solves[e] = solves;
+      a.status[e] = st;
+      state = IDLE;
+    }
+    const bool want[1] = {state == IDLE && !exhausted};
+    pool.refill(want, exhausted, a.ik.n, a.ik.ticket, a.ik.chunk, [&](int, unsigned idx) {
+          e = idx;
+#pragma unroll
+          for (int i = 0; i < NJ; ++i) q[i] = qs[i] = a.q_start[(size_t)e * NJ + i];
+          pose_load_target(a.ik, e, gp, gq);
+          bad_goal = false;
+#pragma unroll
+          for (int i = 0; i < 3; ++i) bad_goal = bad_goal || !isfinite(gp[i]);
+#pragma unroll
+          for (int i = 0; i < 4; ++i) bad_goal = bad_goal || !isfinite(gq[i]);  // a zero quaternion normalises to NaN
+#pragma unroll
+          for (int i = 0; i < 3; ++i) tp[i] = gp[i];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) tq[i] = gq[i];
+          row = (size_t)e * (size_t)a.traj_cap;
+          len = 0; solves = 0; st = 0; points = 0; attempt = 0;
+          it = a.ik.k.max_iters;
+          state = INIT;
+        });
+    if (!__any_sync(FULL, state != IDLE)) break;
+
+    // ---- one 6-row DLS pass for all lanes; a lane whose solve ends post-processes it --------------
+    bool choose = false;  // this lane starts a new solve: pick its aim below
+    pose_pass<T, Kin>(a.ik, trig, qs, tp, tq, it, state != IDLE,
+                      [&](const T* pp, const T* qcur, T pe, T re, int iterations, bool conv) {
+                        bool accept = true;  // INIT: point 0 = FK(q_start)
+                        if (state == SOLVE) {
+                          ++solves;
+                          c_n += 1; c_conv += conv ? 1 : 0; c_iter += (unsigned long long)iterations;
+                          accept = pose_success(a.ik, pe, re, conv);
+                          if (accept) {
+#pragma unroll
+                            for (int i = 0; i < NJ; ++i) q[i] = qs[i];
+                            ++points;
+                          }
+                        }
+                        if (accept) {
+#pragma unroll
+                          for (int i = 0; i < 3; ++i) p[i] = pp[i];
+#pragma unroll
+                          for (int i = 0; i < 4; ++i) r[i] = qcur[i];
+                          append();
+                          attempt = 0;
+                        } else if (++attempt == 3) {
+                          st |= (int)PNP_MOVE_BROKE;
+                        }
+                        state = attempt == 3 ? DONE : SOLVE;
+                        choose = state == SOLVE;
+                      });
+
+    // ---- stop tests at the start of a round, then the aim of the next solve ------------------------
+    if (choose) {
+      const T d[3] = {gp[0] - p[0], gp[1] - p[1], gp[2] - p[2]};
+      const T dist = finish_sqrt((d[0] * d[0] + d[1] * d[1]) + d[2] * d[2]);
+      // goal (x) conj(r) and its angle, written as pose_pass writes the solver's error: a solve aimed at the goal that
+      // converges ends the plan by construction (pos_thresh >= the IK's, rot_thresh >= ik_rot_thresh)
+      const T eq[4] = {gq[0] * r[0] + gq[1] * r[1] + gq[2] * r[2] + gq[3] * r[3],
+                       -gq[0] * r[1] + gq[1] * r[0] - gq[2] * r[3] + gq[3] * r[2],
+                       -gq[0] * r[2] + gq[1] * r[3] + gq[2] * r[0] - gq[3] * r[1],
+                       -gq[0] * r[3] - gq[1] * r[2] + gq[2] * r[1] + gq[3] * r[0]};
+      T w[3];
+      quat2vel_fast(eq, w);
+      const T th = finish_sqrt((w[0] * w[0] + w[1] * w[1]) + w[2] * w[2]);
+      if (attempt == 0) {
+        if (bad_goal) {
+          st |= (int)PNP_MOVE_BROKE;
+          state = DONE;
+        } else if (dist <= a.pos_thresh && th <= a.rot_thresh) {
+          state = DONE;
+        } else if (points >= a.max_traj_points) {
+          st |= (int)PNP_MOVE_CAPPED;
+          state = DONE;
+        }
+      }
+      if (state == SOLVE) {
+        T f = T(1);
+        if (dist > T(0)) f = fmin(f, div_fast(a.step_size, dist));
+        if (th > T(0)) f = fmin(f, div_fast(a.rot_step, th));
+        const T g = attempt == 0 ? f : f * (attempt == 1 ? T(0.5) : T(0.05));
+        if (g == T(1)) {
+#pragma unroll
+          for (int i = 0; i < 3; ++i) tp[i] = gp[i];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) tq[i] = gq[i];
+        } else {
+#pragma unroll
+          for (int i = 0; i < 3; ++i) tp[i] = p[i] + g * d[i];
+          // aim rotation quat(g w) (x) r, one sincos of the half angle
+          T s, c;
+          trig(T(0.5) * g * th, &s, &c);
+          const T k = th > T(0) ? div_fast(s, th) : T(0);
+          const T h[4] = {c, k * w[0], k * w[1], k * w[2]};
+          tq[0] = h[0] * r[0] - h[1] * r[1] - h[2] * r[2] - h[3] * r[3];
+          tq[1] = h[0] * r[1] + h[1] * r[0] + h[2] * r[3] - h[3] * r[2];
+          tq[2] = h[0] * r[2] - h[1] * r[3] + h[2] * r[0] + h[3] * r[1];
+          tq[3] = h[0] * r[3] + h[1] * r[2] - h[2] * r[1] + h[3] * r[0];
+        }
+#pragma unroll
+        for (int i = 0; i < NJ; ++i) qs[i] = q[i];  // every solve starts from the joints of the last point
+        it = 0;
+      }
+    } else {
+      ++it;
+    }
+  }
+  ik_counters_add(a.ik.counters, c_n, c_conv, c_iter);
+}
+
+// =============================================================================================
 // compute_reward / _is_success streaming kernel (panda_env.py:205-245, 303-306).
 //
 // HBM-bound: 60 B in + 4 B out per row (FP32 storage).  Each lane owns kRows consecutive rows

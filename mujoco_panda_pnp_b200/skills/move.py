@@ -5,7 +5,9 @@ fills ``pos_traj`` / ``quat_traj`` (the whole planning loop of move.py:76-191 ru
 ``move_ik_plan_kernel``), ``step()`` replays the waypoints through the env exactly like the
 reference (set_mocap_pose + 5 physics sub-steps; physics itself is the env's, out of scope here).
 
-Additive API: ``plan_moves(model, q_start[N,7], targets[N,3])`` plans N moves in one launch.
+Additive API: ``plan_moves(model, q_start[N,7], targets[N,3])`` plans N moves in one launch;
+``plan_pose_moves(model, q_start, target_pos, target_quat)`` plans N moves to a position AND an orientation
+(``move_pose_plan_kernel``, every waypoint a solved pose), and ``MoveIKSkill(..., target_quat=q)`` uses it.
 
 Difference to the reference, on purpose: the planning loop is bounded (``max_outer`` rounds,
 default 4*max_traj_points+64).  The reference loop never terminates for unreachable targets.
@@ -40,13 +42,43 @@ def plan_moves(model: Any, q_start, targets, pos_thresh: float = 0.01, max_traj_
                                    max_outer=max_outer, traj_cap=traj_cap or max_traj_points + 56)
 
 
+def plan_pose_moves(model: Any, q_start, target_pos, target_quat, pos_thresh: float = 0.01, rot_thresh: float = 0.05,
+                    step_size: float = 0.01, rot_step: float = 0.05, ik_rot_thresh: float = 1e-2, rot_weight: float = 1.0,
+                    max_traj_points: int = 200, traj_cap: Optional[int] = None, precision: str = "fp32",
+                    site_name: str = "ee_center_site", device=None, tree=None):
+    """Plan N moves to target_pos[N,3] and target_quat[N,4] (wxyz) at once (engine.move_ik_plan_pose).  Returns the
+    engine dict (device tensors): pos_traj, quat_traj, q_traj, traj_len, q_final, n_solves, status."""
+    if not torch.cuda.is_available():
+        raise engine._lib.PnpLibraryError("no CUDA device: plan_pose_moves has no CPU path")
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    dt = torch.float32 if precision == "fp32" else torch.float64
+    tree = tree or KinematicTree.from_mjmodel(model, site_name)
+    to = lambda x: (x if isinstance(x, torch.Tensor) else torch.as_tensor(np.asarray(x))).to(device=dev, dtype=dt)  # noqa: E731
+    with torch.cuda.device(dev):
+        engine.set_tree(tree)
+        return engine.move_ik_plan_pose(to(q_start).reshape(-1, 7), to(target_pos).reshape(-1, 3),
+                                        to(target_quat).reshape(-1, 4), engine.ik_params(), pos_thresh=pos_thresh,
+                                        rot_thresh=rot_thresh, step_size=step_size, rot_step=rot_step,
+                                        ik_rot_thresh=ik_rot_thresh, rot_weight=rot_weight,
+                                        max_traj_points=max_traj_points, traj_cap=traj_cap)
+
+
 class MoveIKSkill:
-    """Adaptive IK trajectory planning (reference: skills/move.py:61-208)."""
+    """Adaptive IK trajectory planning (reference: skills/move.py:61-208).
+
+    With ``target_quat`` (wxyz) the move also turns the gripper to that orientation: ``reset()`` plans with the pose
+    planner (plan_pose_moves), every waypoint a solved pose, and keeps its joints in ``q_traj``.  Without it the move
+    is the reference's position-only plan."""
 
     def __init__(self, env, target_pos: np.ndarray, pos_thresh: float = 0.01,
-                 max_traj_points: int = 200, step_size: float = 0.01, *, precision: str = "fp32"):
+                 max_traj_points: int = 200, step_size: float = 0.01, *, precision: str = "fp32",
+                 target_quat: Optional[np.ndarray] = None, rot_thresh: float = 0.05, rot_step: float = 0.05):
         self.env = env
         self.target_pos = np.asarray(target_pos, float)
+        self.target_quat = None if target_quat is None else np.asarray(target_quat, float)
+        self.rot_thresh = rot_thresh
+        self.rot_step = rot_step
+        self.q_traj: list = []
         self.pos_thresh = pos_thresh
         self.max_traj_points = max_traj_points
         self.step_size = step_size
@@ -64,6 +96,16 @@ class MoveIKSkill:
         data = self.env.unwrapped.data
         start_quat = np.asarray(self.env.get_ee_orientation(), dtype=np.float64).copy()  # :92
         q_current = np.asarray(data.qpos[:7], dtype=np.float64).copy()  # :93
+        if self.target_quat is not None:
+            out = plan_pose_moves(model, q_current[None], self.target_pos[None], self.target_quat[None], self.pos_thresh,
+                                  self.rot_thresh, self.step_size, self.rot_step, max_traj_points=self.max_traj_points,
+                                  precision=self.precision)
+            n = min(int(out["traj_len"][0]), out["pos_traj"].shape[1])
+            self.status = int(out["status"][0])
+            self.pos_traj = list(out["pos_traj"][0, :n].double().cpu().numpy())
+            self.quat_traj = list(out["quat_traj"][0, :n].double().cpu().numpy())
+            self.q_traj = list(out["q_traj"][0, :n].double().cpu().numpy())
+            return
         out = plan_moves(model, q_current[None], self.target_pos[None], self.pos_thresh, self.max_traj_points,
                          self.step_size, precision=self.precision)
         n = int(out["traj_len"][0])

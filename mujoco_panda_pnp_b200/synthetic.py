@@ -149,6 +149,14 @@ def reachable_move_envs(n: int, lower, upper, seed: int = 0, device="cpu", dtype
     return dict(q_start=q0.to(dtype).contiguous(), q_goal=torch.minimum(torch.maximum(qs, lo), hi).to(dtype).contiguous())
 
 
+def reachable_pose_move_envs(n: int, lower, upper, seed: int = 0, device="cpu", dtype=torch.float32, spread: float = 0.6):
+    """Pose-planner workload, reachable by construction: start = neutral +- 0.05 rad, goal pose = (FK(q*), quat(q*))
+    with q* = neutral +- ``spread`` rad clipped to the limits.  The caller evaluates FK of q_goal for the goal position
+    and orientation.  Same draws as reachable_move_envs, so the position planner can run the same starts and goal
+    positions."""
+    return reachable_move_envs(n, lower, upper, seed=seed, device=device, dtype=dtype, spread=spread)
+
+
 def her_future_indices(n: int, episode_len: int = 300, seed: int = 0, device="cpu", keep_fraction: float = 0.2,
                        strategy: str = "future") -> torch.Tensor:
     """int32[n] `future_idx` of a HER relabel over a replay buffer that stores its episodes as runs of ``episode_len``

@@ -298,9 +298,12 @@ def ik_restart_seeds(k: int, lower=None, upper=None, seed: int = 0, dtype=torch.
     """A seed table for ik_solve_multistart: k joint configurations ~ U(lower, upper), shape (k, 7).
 
     Drawn from a CPU ``torch.Generator`` and then moved to ``device``, so a seed gives the same table on every device.
-    ``lower`` / ``upper`` default to the joint limits of the packaged kinematic tree."""
+    ``lower`` / ``upper`` default to the joint limits of the tree set_tree last uploaded to the current device (a
+    JacobianIKController uploads its model's tree when it is made), so that the default seeds lie inside the limits the
+    solver clamps to; before any upload, and without a CUDA device, they are the packaged tree's."""
     if lower is None or upper is None:
-        t = KinematicTree.from_mjcf()
+        hit = _uploaded_obj.get(torch.cuda.current_device()) if _uploaded_obj and torch.cuda.is_available() else None
+        t = hit[0] if hit is not None else KinematicTree.from_mjcf()
         lower = t.lower if lower is None else lower
         upper = t.upper if upper is None else upper
     from .synthetic import random_joint_configs

@@ -188,7 +188,7 @@ def _check_fp64(chain, got, ref, pos, quat, tol=1e-8):
     return int(tie.sum())
 
 
-def _check_fp32(chain, got, ref, pos, quat, budget, q_budget=2, **p):
+def _check_fp32(chain, got, ref, pos, quat, budget, q_budget=2, dq_cap=1e-3, **p):
     """FP32 kernel vs the statement on the FP32-rounded inputs (pos, quat).
 
     - Iteration flips (one side crosses a threshold a pass earlier) are counted and bounded by ``budget``, converged /
@@ -196,8 +196,9 @@ def _check_fp32(chain, got, ref, pos, quat, budget, q_budget=2, **p):
       W-cold, at most 2 of 2048 in the representation test and at most 2 of 512 (0.4 %, pos_thresh = 1e-4) in the
       parameter tests; converged flips at most 1 per batch.  Budgets are max(2, 2x observed).
     - Solves that converge in the same number of passes on both sides agree in q within 2e-5 rad, except for at most
-      ``q_budget`` of them, and all of them within 1e-3 rad.  The exceptions are long cold-start walks and weak damping,
-      where FP32 rounding early in the walk is amplified: measured |dq|max quantiles (50/99/99.9/100 %) W-near
+      ``q_budget`` of them, and all of them within ``dq_cap`` (1e-3 rad).  The exceptions are long cold-start walks
+      and weak damping, where FP32 rounding early in the walk is amplified: measured |dq|max quantiles (50/99/99.9/100 %)
+      W-near
       3.7e-7/2.5e-6/4.2e-6/5.7e-6; W-cold 6.6e-7/1.0e-5/4.9e-5/4.1e-4 (7 and 9 of ~1400 above 2e-5); damping 1e-4
       5.3e-7/1.9e-5/1.6e-4/5.1e-4 (4 and 11 of ~500).  Their FP64-FK poses still agree within 1e-4 m and 1e-4 rad
       (measured at most 6.6e-5 m, 5.8e-5 rad), which is asserted for every one of them.
@@ -213,7 +214,7 @@ def _check_fp32(chain, got, ref, pos, quat, budget, q_budget=2, **p):
     q = got["q"].astype(np.float64)
     same = conv & ref["converged"] & (iters == ref["iterations"])
     dq = np.abs(q[same] - ref["q"][same]).max(axis=1)
-    assert (dq > 2e-5).sum() <= q_budget and dq.max(initial=0.0) < 1e-3, (int((dq > 2e-5).sum()), dq.max(initial=0.0))
+    assert (dq > 2e-5).sum() <= q_budget and dq.max(initial=0.0) < dq_cap, (int((dq > 2e-5).sum()), dq.max(initial=0.0))
     ee, mat, _ = c_oracle.fk_jac(chain, q, nthreads=8)
     ref_mat = c_oracle.fk_jac(chain, ref["q"], nthreads=8)[1]
     assert np.linalg.norm(ee[same] - ref["final_pos"][same], axis=1).max(initial=0.0) < 1e-4

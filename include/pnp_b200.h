@@ -15,6 +15,8 @@
  *                          (skills/move.py:106-137), fixed number of waypoints per env
  *   pnp_ik_pose_solve_*    FrankaEnv.solve_ik(target_pos, target_quat, q_init) (panda_env.py:399-409;
  *                          dangling in the reference - an extension defined here)
+ *   pnp_ik_axis_solve_*    a tool position and approach direction, the roll about the tool axis free (an extension
+ *                          defined here)
  *   pnp_move_ik_plan_*     the whole MoveIKSkill.reset planner (skills/move.py:76-191)
  *   pnp_move_ik_plan_pose_*  the same planner to a goal position and orientation (an extension defined here)
  *   pnp_get_obs_*          FrankaEnv._get_obs (envs/panda_env.py:279-301) from kinematic state
@@ -265,6 +267,51 @@ int pnp_ik_pose_solve_multistart_f64(const double* target_pos, const double* tar
                                      const PnpIkParams* params, double rot_thresh, double rot_weight, double* q_out,
                                      double* final_pos, double* final_quat, double* pos_err, double* rot_err,
                                      int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                     unsigned long long* restart_stats, void* scratch, void* stream);
+
+/* ---- axis-constrained IK: tool position and approach direction, roll free (EXTENSION) ----- */
+/* target_pos[n,3] and target_axis[n,3] (normalised on load) in the world frame; tool_axis[3] (host memory, one per
+ * call, e.g. {0, 0, 1}: the packaged Panda's site +z, the approach direction) in the site frame.  The host normalises
+ * t = tool_axis and completes it to the site-frame basis (u1, u2, t): u1 = normalize(t x e_k), e_k the basis vector of
+ * t's smallest-magnitude component (lowest index on a tie), u2 = t x u1.  Each pass, with R the site frame:
+ *   a = R t, b1 = R u1, b2 = R u2;  c = a x d, s = |c|, theta = atan2(s, a.d)   (d = the normalised target axis)
+ *   n = c / s if s > 0;  b1 if s == 0 and a.d < 0;  0 otherwise
+ *   e = [tp - p ; w theta n.b1 ; w theta n.b2],  J = [jacp ; w b1^T jacr ; w b2^T jacr]  (w = rot_weight)
+ *   dq = J^T (J J^T + damping I5)^-1 e, same clips and loop semantics as pnp_ik_pose_solve_*;
+ *   converged when |tp - p| < pos_thresh and theta < rot_thresh; success adds |tp - p| < 2 pos_thresh and
+ *   theta < 2 rot_thresh.
+ * The roll about t is whatever the solve reaches.  Outputs: q_out[n,7], final_pos[n,3], final_axis[n,3] (a),
+ * final_quat[n,4] (site frame, wxyz), pos_err[n], axis_err[n] (theta, rad), iters, flags (all but q_out nullable),
+ * counters[4] (nullable).  Rejected with PNP_EINVAL before anything is enqueued: a NULL, non-finite or zero tool_axis,
+ * rot_thresh or rot_weight not > 0, NULL inputs or q_out, n >= 2^31.  The call never synchronises the host (it can be
+ * captured in a CUDA graph).  The statement is oracle/axis_ik_oracle.py. */
+int pnp_ik_axis_solve_f32(const float* target_pos, const float* target_axis, const float* q_init, int32_t q_init_stride,
+                          int64_t n, const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                          double rot_weight, float* q_out, float* final_pos, float* final_axis, float* final_quat,
+                          float* pos_err, float* axis_err, int32_t* iters, uint8_t* flags, unsigned long long* counters,
+                          void* stream);
+int pnp_ik_axis_solve_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                          int32_t q_init_stride, int64_t n, const PnpIkParams* params, const double* tool_axis,
+                          double rot_thresh, double rot_weight, double* q_out, double* final_pos, double* final_axis,
+                          double* final_quat, double* pos_err, double* axis_err, int32_t* iters, uint8_t* flags,
+                          unsigned long long* counters, void* stream);
+/* Multi-start axis solve: pnp_ik_axis_solve_* from q_init (attempt 0, unchanged), then the restarts of
+ * pnp_ik_pose_solve_multistart_* (same seeds, attempt, counters, restart_stats and scratch contract, flags required):
+ * a query returns its FIRST successful attempt in the order 0, 1, ..., n_seeds, or attempt 0's when none succeeds, and
+ * every output is bit-identical to the plain entry point's for that target from that start. */
+int pnp_ik_axis_solve_multistart_f32(const float* target_pos, const float* target_axis, const float* q_init,
+                                     int32_t q_init_stride, int64_t n, const float* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                     double rot_weight, float* q_out, float* final_pos, float* final_axis,
+                                     float* final_quat, float* pos_err, float* axis_err, int32_t* iters, uint8_t* flags,
+                                     uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats,
+                                     void* scratch, void* stream);
+int pnp_ik_axis_solve_multistart_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                                     int32_t q_init_stride, int64_t n, const double* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                     double rot_weight, double* q_out, double* final_pos, double* final_axis,
+                                     double* final_quat, double* pos_err, double* axis_err, int32_t* iters,
+                                     uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
                                      unsigned long long* restart_stats, void* scratch, void* stream);
 
 /* ---- full MoveIKSkill.reset trajectory planner (skills/move.py:76-191) -------------------- */

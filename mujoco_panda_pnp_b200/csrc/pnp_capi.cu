@@ -1073,6 +1073,111 @@ int pose_multistart_impl(const T* tpos, const T* tquat, const T* q_init, int32_t
       });
 }
 
+// Axis solver: as for the pose solver, a failing attempt runs all max_iters passes and the narrowest group spends no
+// attempt on a query an earlier seed already rescues.  Measured (DESIGN.md 4.8: A-cold, 8 seeds, FP32): 2^20 in
+// 2.60 / 2.48 / 2.84 ms and 2^22 in 8.49 / 8.70 / 10.46 ms at G = 1 / 2 / 4; G = 1 is fastest at 2^22 and over both
+// sizes.  PNP_MS_AXIS_GROUP overrides it (1, 2, 4 or 8), for measurements.
+constexpr int kMsAxisGroup = 1;
+
+// The site-frame basis (t, u1, u2) of a tool axis: t = tool_axis / |tool_axis|; u1 = normalize(t x e_k), e_k the basis
+// vector of t's smallest-magnitude component (the lowest index on a tie); u2 = t x u1.  The statement's rule
+// (oracle/axis_ik_oracle.py tool_basis).  False for a NULL, non-finite or zero tool_axis.
+bool tool_basis(const double* tool_axis, double (&out)[9]) {
+  if (!tool_axis) return false;
+  double m = 0.0;
+  for (int i = 0; i < 3; ++i) {
+    if (!std::isfinite(tool_axis[i])) return false;
+    m = std::max(m, std::fabs(tool_axis[i]));
+  }
+  if (!(m > 0.0)) return false;
+  double t[3] = {tool_axis[0] / m, tool_axis[1] / m, tool_axis[2] / m};  // scaled first: no overflow or underflow
+  const double nt = std::sqrt(t[0] * t[0] + t[1] * t[1] + t[2] * t[2]);
+  for (double& v : t) v /= nt;
+  int k = 0;
+  for (int i = 1; i < 3; ++i)
+    if (std::fabs(t[i]) < std::fabs(t[k])) k = i;
+  const double e[3] = {k == 0 ? 1.0 : 0.0, k == 1 ? 1.0 : 0.0, k == 2 ? 1.0 : 0.0};
+  double u1[3] = {t[1] * e[2] - t[2] * e[1], t[2] * e[0] - t[0] * e[2], t[0] * e[1] - t[1] * e[0]};
+  const double n1 = std::sqrt(u1[0] * u1[0] + u1[1] * u1[1] + u1[2] * u1[2]);
+  for (double& v : u1) v /= n1;
+  const double u2[3] = {t[1] * u1[2] - t[2] * u1[1], t[2] * u1[0] - t[0] * u1[2], t[0] * u1[1] - t[1] * u1[0]};
+  for (int i = 0; i < 3; ++i) { out[i] = t[i]; out[3 + i] = u1[i]; out[6 + i] = u2[i]; }
+  return true;
+}
+
+template <typename T>
+int axis_solve_impl(const T* tpos, const T* taxis, const T* q_init, int32_t q_init_stride, int64_t n,
+                    const PnpIkParams* params, const double* tool_axis, double rot_thresh, double rot_weight, T* q_out,
+                    T* final_pos, T* final_axis, T* final_quat, T* pos_err, T* axis_err, int32_t* iters, uint8_t* flags,
+                    unsigned long long* counters, void* stream, pnp::AxisIkArgs<T>* args_out = nullptr) {
+  int rc = check_ik_params(params);
+  if (rc) return rc;
+  double basis[9];
+  if (!tool_basis(tool_axis, basis)) return fail(PNP_EINVAL, "ik_axis_solve: tool_axis must be non-null, finite and nonzero");
+  if (!(rot_thresh > 0.0) || !(rot_weight > 0.0)) return fail(PNP_EINVAL, "rot_thresh and rot_weight must be > 0");
+  if (n < 0 || (n > 0 && (!tpos || !taxis || !q_init || !q_out)))
+    return fail(PNP_EINVAL, "ik_axis_solve: null pointer or negative n");
+  if (q_init_stride != 0 && q_init_stride != PNP_NJOINT) return fail(PNP_EINVAL, "q_init_stride must be 0 or 7");
+  DeviceState* s;
+  if ((rc = current_state(&s))) return rc;
+  bool spec;
+  if ((rc = pick_kin(s, params->kinematics, &spec))) return rc;
+  if (n == 0) return PNP_OK;
+  if (n >= (int64_t(1) << 31)) return fail(PNP_EINVAL, "ik_axis_solve: n must be < 2^31 per call");
+  cudaStream_t st = (cudaStream_t)stream;
+  pnp::AxisIkArgs<T> a;
+  if ((rc = stream_ticket(s, st, &a.ticket))) return rc;
+  a.target_pos = tpos; a.target_axis = taxis; a.q_init = q_init; a.q_init_stride = q_init_stride; a.n = (unsigned)n;
+  a.k = make_ik_const<T>(params);
+  a.rot_thresh = (T)rot_thresh; a.rot_weight = (T)rot_weight;
+  for (int i = 0; i < 9; ++i) a.basis[i] = (T)basis[i];
+  a.q_out = q_out; a.final_pos = final_pos; a.final_axis = final_axis; a.final_quat = final_quat;
+  a.pos_err = pos_err; a.axis_err = axis_err; a.iters = iters; a.flags = flags; a.counters = counters;
+  const bool small = n <= (long long)s->sm_count * pnp::IK_BLOCK;
+  const int block = pnp::IK_BLOCK;
+  int occ;
+  rc = spec ? occupancy<pnp::ik_axis_solve_kernel<T, pnp::SpecKin>>(s, block, 0, &occ)
+            : occupancy<pnp::ik_axis_solve_kernel<T, pnp::GenericKin>>(s, block, 0, &occ);
+  if (rc) return rc;
+  const PersistentGrid g = persistent_grid(s, n, 1, block, occ, small, 16, 256);
+  a.chunk = g.chunk;
+  a.solo_warp = small ? 1u : 0u;
+  if (args_out) *args_out = a;  // the multistart's restarts use this block
+  if (spec)
+    pnp::ik_axis_solve_kernel<T, pnp::SpecKin><<<g.grid, block, 0, st>>>(a);
+  else
+    pnp::ik_axis_solve_kernel<T, pnp::GenericKin><<<g.grid, block, 0, st>>>(a);
+  ++g_launches;
+  CUDA_TRY(cudaGetLastError());
+  return PNP_OK;
+}
+
+// Multi-start axis solve: axis_solve_impl, then the restart waves of ms_axis_wave_kernel (see multistart_impl).
+template <typename T>
+int axis_multistart_impl(const T* tpos, const T* taxis, const T* q_init, int32_t q_init_stride, int64_t n, const T* seeds,
+                         int32_t n_seeds, const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                         double rot_weight, T* q_out, T* final_pos, T* final_axis, T* final_quat, T* pos_err,
+                         T* axis_err, int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                         unsigned long long* restart_stats, void* scratch, void* stream) {
+  const size_t m = (size_t)n;
+  return multistart_impl<pnp::AxisIkArgs<T>, pnp::IK_OUT_SEPARATE>(
+      "ik_axis_multistart", n, seeds, n_seeds, params, flags, iters, attempt, counters, restart_stats, scratch,
+      {byte_range(q_out, m * PNP_NJOINT * sizeof(T)), byte_range(final_pos, m * 3 * sizeof(T)),
+       byte_range(final_axis, m * 3 * sizeof(T)), byte_range(final_quat, m * 4 * sizeof(T)),
+       byte_range(pos_err, m * sizeof(T)), byte_range(axis_err, m * sizeof(T)), byte_range(iters, m * sizeof(int32_t)),
+       byte_range(flags, m)},
+      kMsAxisGroup, "PNP_MS_AXIS_GROUP", stream,
+      [&](int32_t* iters0, pnp::AxisIkArgs<T>& a) {
+        return axis_solve_impl<T>(tpos, taxis, q_init, q_init_stride, n, params, tool_axis, rot_thresh, rot_weight, q_out,
+                                  final_pos, final_axis, final_quat, pos_err, axis_err, iters0, flags, counters, stream,
+                                  &a);
+      },
+      [&](DeviceState* s, bool spec, const auto& m, cudaStream_t st) {
+        return spec ? launch_ms_wave<pnp::ms_axis_wave_kernel<T, pnp::SpecKin>>(s, m, st)
+                    : launch_ms_wave<pnp::ms_axis_wave_kernel<T, pnp::GenericKin>>(s, m, st);
+      });
+}
+
 template <typename T>
 int plan_order_impl(const T* q_start, const T* target, int64_t n, uint32_t* order, int32_t kinematics, void* stream,
                     float4* records = nullptr) {
@@ -1296,6 +1401,48 @@ int pnp_ik_pose_solve_multistart_f64(const double* target_pos, const double* tar
   return pose_multistart_impl<double>(target_pos, target_quat, q_init, q_init_stride, n, seeds, n_seeds, params,
                                       rot_thresh, rot_weight, q_out, final_pos, final_quat, pos_err, rot_err, iters, flags,
                                       attempt, counters, restart_stats, scratch, stream);
+}
+
+int pnp_ik_axis_solve_f32(const float* target_pos, const float* target_axis, const float* q_init, int32_t q_init_stride,
+                          int64_t n, const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                          double rot_weight, float* q_out, float* final_pos, float* final_axis, float* final_quat,
+                          float* pos_err, float* axis_err, int32_t* iters, uint8_t* flags, unsigned long long* counters,
+                          void* stream) {
+  return axis_solve_impl<float>(target_pos, target_axis, q_init, q_init_stride, n, params, tool_axis, rot_thresh,
+                                rot_weight, q_out, final_pos, final_axis, final_quat, pos_err, axis_err, iters, flags,
+                                counters, stream);
+}
+int pnp_ik_axis_solve_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                          int32_t q_init_stride, int64_t n, const PnpIkParams* params, const double* tool_axis,
+                          double rot_thresh, double rot_weight, double* q_out, double* final_pos, double* final_axis,
+                          double* final_quat, double* pos_err, double* axis_err, int32_t* iters, uint8_t* flags,
+                          unsigned long long* counters, void* stream) {
+  return axis_solve_impl<double>(target_pos, target_axis, q_init, q_init_stride, n, params, tool_axis, rot_thresh,
+                                 rot_weight, q_out, final_pos, final_axis, final_quat, pos_err, axis_err, iters, flags,
+                                 counters, stream);
+}
+
+int pnp_ik_axis_solve_multistart_f32(const float* target_pos, const float* target_axis, const float* q_init,
+                                     int32_t q_init_stride, int64_t n, const float* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                     double rot_weight, float* q_out, float* final_pos, float* final_axis,
+                                     float* final_quat, float* pos_err, float* axis_err, int32_t* iters, uint8_t* flags,
+                                     uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats,
+                                     void* scratch, void* stream) {
+  return axis_multistart_impl<float>(target_pos, target_axis, q_init, q_init_stride, n, seeds, n_seeds, params, tool_axis,
+                                     rot_thresh, rot_weight, q_out, final_pos, final_axis, final_quat, pos_err, axis_err,
+                                     iters, flags, attempt, counters, restart_stats, scratch, stream);
+}
+int pnp_ik_axis_solve_multistart_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                                     int32_t q_init_stride, int64_t n, const double* seeds, int32_t n_seeds,
+                                     const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                     double rot_weight, double* q_out, double* final_pos, double* final_axis,
+                                     double* final_quat, double* pos_err, double* axis_err, int32_t* iters,
+                                     uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                     unsigned long long* restart_stats, void* scratch, void* stream) {
+  return axis_multistart_impl<double>(target_pos, target_axis, q_init, q_init_stride, n, seeds, n_seeds, params,
+                                      tool_axis, rot_thresh, rot_weight, q_out, final_pos, final_axis, final_quat, pos_err,
+                                      axis_err, iters, flags, attempt, counters, restart_stats, scratch, stream);
 }
 
 int pnp_move_plan_order_f32(const float* q_start, const float* target, int64_t n, uint32_t* order, int32_t kinematics,

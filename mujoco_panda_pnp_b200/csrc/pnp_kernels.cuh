@@ -1868,6 +1868,267 @@ __global__ void __launch_bounds__(MS_BLOCK) ms_pose_wave_kernel(const MsArgs<Pos
 }
 
 // =============================================================================================
+// Axis-constrained IK (pnp_ik_axis_solve_*, an EXTENSION stated in oracle/axis_ik_oracle.py): the tool position and
+// the direction of one site-frame tool axis t, the roll about that axis left free.  Same loop as the pose solver with a
+// 5-row task in the basis (u1, u2, t) the host completes t to:
+//   a = R t, b1 = R u1, b2 = R u2;  c = a x d, s = |c|, theta = atan2(s, a.d)    (d = the normalised target axis)
+//   n = c / s if s > 0;  b1 if s == 0 and a.d < 0;  0 otherwise
+//   e = [tp - p ; w theta n.b1 ; w theta n.b2],  J = [jacp ; w b1^T jacr ; w b2^T jacr]  (5x7)
+//   converged  <=>  |tp - p| < pos_thresh  and  theta < rot_thresh                (tested before update)
+// This is the damped 6-row task with the rotation rows projected off a, written in a basis whose a row is zero; it
+// needs no quaternion per pass (final_quat is formed once, by the lane that finishes, when asked for).
+// =============================================================================================
+template <typename T>
+struct AxisIkArgs {
+  const T* target_pos;
+  const T* target_axis;
+  const T* q_init;
+  int q_init_stride;
+  unsigned n;       // < 2^31 (checked on the host)
+  IkConst<T> k;
+  T rot_thresh, rot_weight;
+  T basis[9];       // site frame: t, u1, u2 (the host's tool_basis rule)
+  T* q_out;
+  T* final_pos;
+  T* final_axis;
+  T* final_quat;
+  T* pos_err;
+  T* axis_err;
+  int32_t* iters;
+  uint8_t* flags;
+  unsigned long long* counters;
+  unsigned* ticket; // zeroed before launch
+  unsigned chunk;   // queries a warp reserves per ticket atomic
+  unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works
+};
+
+// The pieces of an axis solve that ik_axis_solve_kernel and the multistart restarts (ms_axis_wave_kernel) share, so
+// that a restart attempt runs the plain kernel's arithmetic bit for bit.
+// Target of query e: its position and its axis normalised on load.
+template <typename T>
+__device__ __forceinline__ void axis_load_target(const AxisIkArgs<T>& a, unsigned e, T (&tp)[3], T (&d)[3]) {
+#pragma unroll
+  for (int i = 0; i < 3; ++i) tp[i] = a.target_pos[(size_t)e * 3 + i];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) d[i] = a.target_axis[(size_t)e * 3 + i];
+  const T nd = sqrt_t(d[0] * d[0] + d[1] * d[1] + d[2] * d[2]);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) d[i] = d[i] / nd;
+}
+
+// One 5-row DLS pass at q (pass number `it`): evaluate the error and test convergence; a lane that is `active` and
+// finishes in this pass calls done(pp, R, ax, pe, th, iterations, conv) with the site position and frame, the world
+// tool axis and the errors at the q it finished at (q is still that q during the call).  Then q takes the DLS step -
+// unconditionally: the caller discards the q of a lane that has finished.
+template <typename T, typename Kin, typename Done>
+__device__ __forceinline__ void axis_pass_inline(const AxisIkArgs<T>& a, const Trig<T>& trig, T (&q)[NJ],
+                                                 const T (&tp)[3], const T (&d)[3], int it, bool active, Done done) {
+  T s[NJ], c[NJ];
+#pragma unroll
+  for (int i = 0; i < NJ; ++i) trig(q[i] - Kin::template qref<T>(i), &s[i], &c[i]);
+  T pp[3], J[42], R[9];
+  Kin::template fk_full<T>(s, c, pp, J, R);
+  T ax[3], b1[3], b2[3];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    ax[i] = R[3 * i] * a.basis[0] + R[3 * i + 1] * a.basis[1] + R[3 * i + 2] * a.basis[2];
+    b1[i] = R[3 * i] * a.basis[3] + R[3 * i + 1] * a.basis[4] + R[3 * i + 2] * a.basis[5];
+    b2[i] = R[3 * i] * a.basis[6] + R[3 * i + 1] * a.basis[7] + R[3 * i + 2] * a.basis[8];
+  }
+  const T cr[3] = {ax[1] * d[2] - ax[2] * d[1], ax[2] * d[0] - ax[0] * d[2], ax[0] * d[1] - ax[1] * d[0]};
+  const T sn = sqrt_t((cr[0] * cr[0] + cr[1] * cr[1]) + cr[2] * cr[2]);
+  const T ad = (ax[0] * d[0] + ax[1] * d[1]) + ax[2] * d[2];
+  const T th = atan2_t(sn, ad);
+  // n.b1, n.b2: (c.b1) / s, (c.b2) / s; at s == 0 antiparallel n = b1 (b1.b1 = 1, b1.b2 = 0), aligned n = 0
+  const bool tilted = sn > T(0);
+  const T inv = tilted ? rcp_t(sn) : T(0);
+  const T nb1 = tilted ? ((cr[0] * b1[0] + cr[1] * b1[1]) + cr[2] * b1[2]) * inv : (ad < T(0) ? T(1) : T(0));
+  const T nb2 = tilted ? ((cr[0] * b2[0] + cr[1] * b2[1]) + cr[2] * b2[2]) * inv : T(0);
+  const T wth = a.rot_weight * th;
+  T err[5] = {tp[0] - pp[0], tp[1] - pp[1], tp[2] - pp[2], wth * nb1, wth * nb2};
+  const T pe = finish_sqrt((err[0] * err[0] + err[1] * err[1]) + err[2] * err[2]);
+  const bool last = it >= a.k.max_iters;
+  const bool conv = !last && (pe < a.k.pos_thresh) && (th < a.rot_thresh);
+  if (active && (conv || last)) done(pp, R, ax, pe, th, conv ? it + 1 : it, conv);
+  // rows 3 and 4: w b1^T jacr, w b2^T jacr
+  T Jt[35];
+#pragma unroll
+  for (int j = 0; j < 21; ++j) Jt[j] = J[j];
+  const T wb1[3] = {a.rot_weight * b1[0], a.rot_weight * b1[1], a.rot_weight * b1[2]};
+  const T wb2[3] = {a.rot_weight * b2[0], a.rot_weight * b2[1], a.rot_weight * b2[2]};
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) {
+    Jt[21 + j] = (wb1[0] * J[21 + j] + wb1[1] * J[28 + j]) + wb1[2] * J[35 + j];
+    Jt[28 + j] = (wb2[0] * J[21 + j] + wb2[1] * J[28 + j]) + wb2[2] * J[35 + j];
+  }
+  T A[5][5];
+#pragma unroll
+  for (int r = 0; r < 5; ++r)
+#pragma unroll
+    for (int c2 = 0; c2 <= r; ++c2) {
+      T acc = T(0);
+#pragma unroll
+      for (int j = 0; j < NJ; ++j) acc = acc + Jt[r * 7 + j] * Jt[c2 * 7 + j];
+      A[r][c2] = acc + (r == c2 ? a.k.damping : T(0));
+    }
+  ldlt_solve<T, 5>(A, err);
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) {
+    T dq = T(0);
+#pragma unroll
+    for (int r = 0; r < 5; ++r) dq = dq + Jt[r * 7 + j] * err[r];
+    dq = clamp_t(dq, -a.k.step_limit, a.k.step_limit);
+    q[j] = clamp_t(q[j] + dq, Kin::template lower<T>(j), Kin::template upper<T>(j));
+  }
+}
+
+// FP64: one out-of-line copy of the pass for the plain kernel and the restarts, returning what the pass hands to done.
+// NVVM fuses a multiply into an FMA or not depending on the code around it: with the pass inlined in both kernels, an
+// FP64 restart row differed from the plain solve from the same seed (one term of the generated FK was an FMA in one
+// kernel and a multiply and subtract in the other, DESIGN.md 4.8).  One function makes a restart bit-identical to the
+// plain solve by construction, for 528-640 B of stack per thread and 7 % more time per FP64 pass.  (FP32, the product
+// path, stays inlined; its plain and restart kernels are compared bit for bit by tests/test_gpu_axis_ik.py.)
+template <typename T, typename Kin>
+__device__ __noinline__ void axis_pass_call(const AxisIkArgs<T>& a, const Trig<T>& trig, T (&q)[NJ], const T (&tp)[3],
+                                            const T (&d)[3], int it, bool active, bool& fin, T (&pp)[3], T (&R)[9],
+                                            T (&ax)[3], T& pe, T& th, int& its, bool& conv) {
+  fin = false;
+  axis_pass_inline<T, Kin>(a, trig, q, tp, d, it, active,
+                           [&](const T* p_, const T* r_, const T* x_, T pe_, T th_, int its_, bool conv_) {
+                             for (int i = 0; i < 3; ++i) { pp[i] = p_[i]; ax[i] = x_[i]; }
+                             for (int i = 0; i < 9; ++i) R[i] = r_[i];
+                             pe = pe_; th = th_; its = its_; conv = conv_; fin = true;
+                           });
+}
+
+// axis_pass_inline's contract, for either precision
+template <typename T, typename Kin, typename Done>
+__device__ __forceinline__ void axis_pass(const AxisIkArgs<T>& a, const Trig<T>& trig, T (&q)[NJ], const T (&tp)[3],
+                                          const T (&d)[3], int it, bool active, Done done) {
+  if constexpr (std::is_same<T, double>::value) {
+    T qn[NJ], pp[3], R[9], ax[3], pe, th;
+    int its;
+    bool fin, conv;
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) qn[j] = q[j];
+    axis_pass_call<T, Kin>(a, trig, qn, tp, d, it, active, fin, pp, R, ax, pe, th, its, conv);
+    if (fin) done(pp, R, ax, pe, th, its, conv);  // q is still the q the lane finished at
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) q[j] = qn[j];
+  } else {
+    axis_pass_inline<T, Kin>(a, trig, q, tp, d, it, active, done);
+  }
+}
+
+// the success rule of a finished axis solve
+template <typename T>
+__device__ __forceinline__ bool axis_success(const AxisIkArgs<T>& a, T pe, T th, bool conv) {
+  return conv && (pe < a.k.pos_thresh * T(2)) && (th < a.rot_thresh * T(2));
+}
+
+// Store the record of query e (every output but q_out nullable); qcur is read only when final_quat is asked for
+template <typename T>
+__device__ __forceinline__ void axis_store(const AxisIkArgs<T>& a, unsigned e, const T (&q)[NJ], const T* pp,
+                                           const T* ax, const T* qcur, T pe, T th, int iterations, bool conv) {
+  const bool success = axis_success(a, pe, th, conv);
+#pragma unroll
+  for (int i = 0; i < NJ; ++i) a.q_out[(size_t)e * NJ + i] = q[i];
+  if (a.final_pos) { a.final_pos[(size_t)e * 3] = pp[0]; a.final_pos[(size_t)e * 3 + 1] = pp[1]; a.final_pos[(size_t)e * 3 + 2] = pp[2]; }
+  if (a.final_axis) { a.final_axis[(size_t)e * 3] = ax[0]; a.final_axis[(size_t)e * 3 + 1] = ax[1]; a.final_axis[(size_t)e * 3 + 2] = ax[2]; }
+  if (a.final_quat) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) a.final_quat[(size_t)e * 4 + i] = qcur[i];
+  }
+  if (a.pos_err) a.pos_err[e] = pe;
+  if (a.axis_err) a.axis_err[e] = th;
+  if (a.iters) a.iters[e] = iterations;
+  if (a.flags) a.flags[e] = (uint8_t)((conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u));
+}
+
+// Persistent warps with lane refill, as ik_pose_solve_kernel.  The FP32 instantiation uses the table trig.
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(IK_BLOCK) ik_axis_solve_kernel(const AxisIkArgs<T> a) {
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
+  const Trig<T> trig{s_tab};
+  unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
+  WarpPool pool;
+  bool exhausted = false, active = false;
+  unsigned e = 0;
+  int it = 0;
+  T q[NJ], tp[3] = {T(0), T(0), T(0)}, d[3] = {T(0), T(0), T(1)};
+#pragma unroll
+  for (int i = 0; i < NJ; ++i) q[i] = T(0);
+
+  while (true) {
+    const bool want[1] = {!active && !exhausted};
+    pool.refill(want, exhausted, a.n, a.ticket, a.chunk, [&](int, unsigned idx) {
+          e = idx;
+          const T* qi = a.q_init + (size_t)a.q_init_stride * e;
+#pragma unroll
+          for (int i = 0; i < NJ; ++i) q[i] = qi[i];
+          axis_load_target(a, e, tp, d);
+          it = 0;
+          active = true;
+        });
+    if (!__any_sync(FULL, active)) break;
+
+    axis_pass<T, Kin>(a, trig, q, tp, d, it, active,
+                      [&](const T* pp, const T* R, const T* ax, T pe, T th, int iterations, bool conv) {
+                        T qcur[4];
+                        if (a.final_quat) mat2quat_fast(R, qcur);
+                        axis_store(a, e, q, pp, ax, qcur, pe, th, iterations, conv);
+                        c_n += 1; c_conv += conv ? 1 : 0; c_iter += (unsigned long long)iterations;
+                        active = false;
+                      });
+    ++it;
+  }
+  ik_counters_add(a.counters, c_n, c_conv, c_iter);
+}
+
+// ---- multi-start axis IK (pnp_ik_axis_solve_multistart_*): ms_pose_wave_kernel with axis_pass / axis_store ---------
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(MS_BLOCK) ms_axis_wave_kernel(const MsArgs<AxisIkArgs<T>> m) {
+  const unsigned cnt = *m.cnt_in;
+  if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;  // no work for any warp of this block
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  const Trig<T> trig{s_tab};
+  // the finished attempt of this lane: q, position, axis, quaternion (when asked for) and errors at its last pass
+  T qk[NJ], pk[3], ak[3], qck[4], pek = T(0), thk = T(0);
+  bool conv = false;
+  int it_kept = 0;
+  auto solve = [&](bool valid, unsigned id, int seed, bool& succ, int& iterations) {
+    T q[NJ], tp[3], d[3];
+    axis_load_target(m.a, id, tp, d);
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) q[i] = m.seeds[seed * NJ + i];
+    bool active = valid;
+    conv = false;
+    it_kept = 0;
+    for (int it = 0; __any_sync(FULL, active); ++it)
+      axis_pass<T, Kin>(m.a, trig, q, tp, d, it, active,
+                        [&](const T* pp, const T* R, const T* ax, T pe, T th, int its, bool cv) {
+#pragma unroll
+                          for (int i = 0; i < NJ; ++i) qk[i] = q[i];
+#pragma unroll
+                          for (int i = 0; i < 3; ++i) { pk[i] = pp[i]; ak[i] = ax[i]; }
+                          if (m.a.final_quat) mat2quat_fast(R, qck);
+                          pek = pe; thk = th; it_kept = its; conv = cv;
+                          active = false;
+                        });
+    iterations = it_kept;
+    succ = axis_success(m.a, pek, thk, conv);
+  };
+  auto prev = [&](unsigned id, unsigned& fl, unsigned& it) { ms_ik_prev<IK_OUT_SEPARATE>(m, id, fl, it); };
+  auto store = [&](unsigned id) { axis_store(m.a, id, qk, pk, ak, qck, pek, thk, it_kept, conv); };
+  ms_wave(m, cnt, solve, prev, store);
+}
+
+// =============================================================================================
 // MoveIKSkill.reset trajectory planner (skills/move.py:76-191) as a per-lane state machine.
 //
 // One lane per env.  Every trip of the warp loop is ONE shared, divergence-free DLS pass

@@ -467,6 +467,81 @@ def ik_pose_solve_multistart(target_pos: torch.Tensor, target_quat: torch.Tensor
                 converged=(flags & 1) != 0, success=(flags & 2) != 0, attempt=attempt)
 
 
+def _axis_inputs(target_pos, target_axis, tool_axis):
+    dt = target_pos.dtype
+    if dt not in (torch.float32, torch.float64):
+        raise ValueError("target_pos must be float32 or float64")
+    target_pos = _check_cuda("target_pos", target_pos, dt, (3,))
+    target_axis = _check_cuda("target_axis", target_axis, dt, (3,))
+    if target_axis.shape[0] != target_pos.shape[0]:
+        raise ValueError("target_pos and target_axis disagree on N")
+    tool = np.asarray(tool_axis, dtype=np.float64).reshape(-1)
+    if tool.shape != (3,):
+        raise ValueError("tool_axis must have 3 components")
+    return target_pos, target_axis, (ctypes.c_double * 3)(*tool.tolist())
+
+
+def _axis_outputs(n, dt, dev):
+    return dict(q=torch.empty((n, 7), dtype=dt, device=dev), final_pos=torch.empty((n, 3), dtype=dt, device=dev),
+                final_axis=torch.empty((n, 3), dtype=dt, device=dev), final_quat=torch.empty((n, 4), dtype=dt, device=dev),
+                pos_error=torch.empty((n,), dtype=dt, device=dev), axis_error=torch.empty((n,), dtype=dt, device=dev),
+                iterations=torch.empty((n,), dtype=torch.int32, device=dev),
+                flags=torch.empty((n,), dtype=torch.uint8, device=dev))
+
+
+def _axis_result(o, **extra):
+    flags = o.pop("flags")
+    return dict(o, converged=(flags & 1) != 0, success=(flags & 2) != 0, **extra)
+
+
+def ik_axis_solve(target_pos: torch.Tensor, target_axis: torch.Tensor, q_init: torch.Tensor, params: PnpIkParams,
+                  tool_axis=(0.0, 0.0, 1.0), rot_thresh: float = 1e-2, rot_weight: float = 1.0,
+                  counters: Optional[torch.Tensor] = None) -> dict:
+    """Axis-constrained IK (extension, pnp_ik_axis_solve_*): put the site at target_pos[N,3] with its ``tool_axis``
+    (site frame, (3,)) along target_axis[N,3] (world frame, any norm), the roll about that axis free.  q_init[N,7] or
+    [7].  Returns q, final_pos, final_axis (the tool axis in the world frame), final_quat, pos_error, axis_error (the
+    angle between final_axis and the target axis, rad), iterations, converged, success."""
+    lib = _lib.load()
+    target_pos, target_axis, tool = _axis_inputs(target_pos, target_axis, tool_axis)
+    dt, n, dev = target_pos.dtype, target_pos.shape[0], target_pos.device
+    q_init, stride = _q_init_arg(q_init, n, dt, dev)
+    fn = lib.pnp_ik_axis_solve_f32 if dt == torch.float32 else lib.pnp_ik_axis_solve_f64
+    with torch.cuda.device(dev):
+        o = _axis_outputs(n, dt, dev)
+        _lib.check(
+            fn(_ptr(target_pos), _ptr(target_axis), _ptr(q_init), stride, n, ctypes.byref(params), tool,
+               float(rot_thresh), float(rot_weight), *(_ptr(t) for t in o.values()), _ptr(counters), _stream()),
+            "pnp_ik_axis_solve",
+        )
+    return _axis_result(o)
+
+
+def ik_axis_solve_multistart(target_pos: torch.Tensor, target_axis: torch.Tensor, q_init: torch.Tensor,
+                             seeds: torch.Tensor, params: PnpIkParams, tool_axis=(0.0, 0.0, 1.0),
+                             rot_thresh: float = 1e-2, rot_weight: float = 1.0, counters: Optional[torch.Tensor] = None,
+                             restart_stats: Optional[torch.Tensor] = None) -> dict:
+    """ik_axis_solve, then every query it did not solve is solved again from the rows of ``seeds`` (K, 7), in order,
+    until one succeeds (pnp_ik_axis_solve_multistart_*).  Each row of the result is, bit for bit, the plain
+    ik_axis_solve of that target from the start ``attempt`` names (0 = q_init, k = seeds[k - 1]).  Returns
+    ik_axis_solve's dict plus ``attempt`` (uint8[N]); ``counters`` / ``restart_stats`` as ik_pose_solve_multistart.
+    Never synchronises."""
+    lib = _lib.load()
+    target_pos, target_axis, tool = _axis_inputs(target_pos, target_axis, tool_axis)
+    dt, n, dev = target_pos.dtype, target_pos.shape[0], target_pos.device
+    q_init, stride = _q_init_arg(q_init, n, dt, dev)
+    seeds, scratch, attempt = _multistart_inputs(seeds, n, dt, dev, counters, restart_stats)
+    fn = lib.pnp_ik_axis_solve_multistart_f32 if dt == torch.float32 else lib.pnp_ik_axis_solve_multistart_f64
+    with torch.cuda.device(dev):
+        o = _axis_outputs(n, dt, dev)
+        _lib.check(
+            fn(_ptr(target_pos), _ptr(target_axis), _ptr(q_init), stride, n, _ptr(seeds), seeds.shape[0],
+               ctypes.byref(params), tool, float(rot_thresh), float(rot_weight), *(_ptr(t) for t in o.values()),
+               _ptr(attempt), _ptr(counters), _ptr(restart_stats), _ptr(scratch), _stream()),
+            "pnp_ik_axis_solve_multistart",
+        )
+    return _axis_result(o, attempt=attempt)
+
+
 PLAN_ORDER_MIN = 1 << 16  # below this a launch has fewer envs than lanes: nothing to balance (2^14 measured slower)
 
 

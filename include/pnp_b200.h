@@ -19,6 +19,8 @@
  *                          defined here)
  *   pnp_move_ik_plan_*     the whole MoveIKSkill.reset planner (skills/move.py:76-191)
  *   pnp_move_ik_plan_pose_*  the same planner to a goal position and orientation (an extension defined here)
+ *   pnp_move_ik_plan_axis_*  the same planner to a goal position and tool-axis direction, the roll free (an
+ *                          extension defined here)
  *   pnp_get_obs_*          FrankaEnv._get_obs (envs/panda_env.py:279-301) from kinematic state
  *   pnp_reward_*           FrankaEnv.compute_reward / _is_success / goal_distance
  *                          (envs/panda_env.py:205-245, 303-306, 311-315), row-wise
@@ -326,8 +328,8 @@ typedef struct PnpMoveParams {
                                (pnp_move_plan_order_*) and then take the envs in that order; 0 = `order` is an input */
 } PnpMoveParams;
 #define PNP_MOVE_BROKE 1u      /* fallback strategies exhausted (reference `break`, move.py:178-180);
-                                  pose planner: three rejected solves in one round, or a non-finite / zero goal */
-#define PNP_MOVE_CAPPED 2u     /* max_outer reached; pose planner: max_traj_points points reached */
+                                  pose / axis planner: three rejected solves in one round, or a non-finite / zero goal */
+#define PNP_MOVE_CAPPED 2u     /* max_outer reached; pose / axis planner: max_traj_points points reached */
 #define PNP_MOVE_OVERFLOW 4u   /* more than traj_cap points: extra points dropped, traj_len still counts */
 /* Per env: q_start[n,7], target[n,3].  The whole adaptive-waypoint state machine (accept rule,
  * failure counting incl. the double increment, fallback strategies 1-3, final-point append) runs
@@ -408,6 +410,39 @@ int pnp_move_ik_plan_pose_f64(const double* q_start, const double* goal_pos, con
                               const PnpMovePoseParams* move, const PnpIkParams* params, double* pos_traj,
                               double* quat_traj, double* q_traj, int32_t* traj_len, double* q_final, int32_t* n_solves,
                               int32_t* status, unsigned long long* counters, void* stream);
+
+/* ---- axis-mode move planner: plan to a goal position and tool-axis direction, roll free (EXTENSION) ---------------- */
+/* Per env: q_start[n,7], goal_pos[n,3], goal_axis[n,3] (world frame, normalised on load); tool_axis[3] (host memory,
+ * one per call, site frame) with its basis (t, u1, u2) as in pnp_ik_axis_solve_*.  PnpMovePoseParams as for the pose
+ * planner, with rot_thresh, rot_step, ik_rot_thresh and ik_rot_weight applying to the axis angle theta.  (p, R) =
+ * FK(q_start), a = R t: point 0 is (p, a, quat(R), q_start).  Each round: d = goal_pos - p, theta = atan2(|a x g|, a.g)
+ * (g the goal axis, evaluated as the axis solver evaluates its error).  The plan ends with status 0 when |d| <=
+ * pos_thresh and theta <= rot_thresh, and with PNP_MOVE_CAPPED after max_traj_points points.  Otherwise f = min(1,
+ * step_size / |d|, rot_step / theta) and up to three axis solves (pnp_ik_axis_solve_* from the current q with `params`,
+ * tool_axis, ik_rot_thresh, ik_rot_weight) aim at the fractions h = f, f/2, f/20 of the remaining motion:
+ * (p + h d, normalize(cos(h theta) a + sin(h theta) m)) with m = (g - (a.g) a) / |a x g| the unit tangent turning a
+ * toward g (m = -R u2 when a and g are exactly antiparallel, the solver's own choice of tilt direction), or exactly the
+ * goal when h == 1.  The first success appends its (final_pos, final_axis, final_quat, q) and moves there; three
+ * rejections end the plan with PNP_MOVE_BROKE, as does a non-finite goal or a zero goal axis (then traj_len = 1).  The
+ * roll about t is whatever the solves reach.  The unreached goal is never appended: every point is a solved axis task,
+ * and pos_traj, axis_traj, quat_traj and q_traj line up.  traj_len <= max_traj_points + 1, n_solves <=
+ * 3 max_traj_points; points past traj_cap are dropped and set PNP_MOVE_OVERFLOW (traj_len still counts them).
+ * Outputs: pos_traj[n,traj_cap,3], axis_traj[n,traj_cap,3] (a, world frame), quat_traj[n,traj_cap,4] (site frame,
+ * wxyz), q_traj[n,traj_cap,7] (nullable), traj_len[n], q_final[n,7] (the joints of the last point), n_solves[n],
+ * status[n] (PNP_MOVE_* bits), counters[4] (nullable: every axis solve, as pnp_ik_axis_solve_*).  Rejected with
+ * PNP_EINVAL before anything is enqueued: everything pnp_move_ik_plan_pose_* rejects, a NULL, non-finite or zero
+ * tool_axis, NULL outputs other than q_traj and counters.  The call never synchronises the host and can be captured in
+ * a CUDA graph.  The oracle is oracle/move_axis_oracle.py. */
+int pnp_move_ik_plan_axis_f32(const float* q_start, const float* goal_pos, const float* goal_axis, int64_t n,
+                              const PnpMovePoseParams* move, const PnpIkParams* params, const double* tool_axis,
+                              float* pos_traj, float* axis_traj, float* quat_traj, float* q_traj, int32_t* traj_len,
+                              float* q_final, int32_t* n_solves, int32_t* status, unsigned long long* counters,
+                              void* stream);
+int pnp_move_ik_plan_axis_f64(const double* q_start, const double* goal_pos, const double* goal_axis, int64_t n,
+                              const PnpMovePoseParams* move, const PnpIkParams* params, const double* tool_axis,
+                              double* pos_traj, double* axis_traj, double* quat_traj, double* q_traj, int32_t* traj_len,
+                              double* q_final, int32_t* n_solves, int32_t* status, unsigned long long* counters,
+                              void* stream);
 
 /* ---- compute_reward / _is_success, row-wise --------------------------------------------- */
 /* Per row: achieved_goal[n,3], desired_goal[n,3], ee_pos[n,3], ee_quat[n,4] wxyz,

@@ -136,6 +136,10 @@ SIGNATURES = {
                                           _P, _P, _P, _P, _P]),
     "pnp_move_ik_plan_pose_f64": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMovePoseParams), POINTER(PnpIkParams), _P, _P, _P, _P,
                                           _P, _P, _P, _P, _P]),
+    "pnp_move_ik_plan_axis_f32": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMovePoseParams), POINTER(PnpIkParams),
+                                          POINTER(c_double), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_move_ik_plan_axis_f64": (c_int, [_P, _P, _P, c_int64, POINTER(PnpMovePoseParams), POINTER(PnpIkParams),
+                                          POINTER(c_double), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "pnp_reward_f32": (c_int, [_P, _P, _P, _P, _P, _P, c_int64, POINTER(PnpRewardParams), _P, _P, _P, _P]),
     "pnp_reward_f64": (c_int, [_P, _P, _P, _P, _P, _P, c_int64, POINTER(PnpRewardParams), _P, _P, _P, _P]),
     "pnp_get_obs_f32": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int32, c_int64, c_double, _P, c_int32, _P]),

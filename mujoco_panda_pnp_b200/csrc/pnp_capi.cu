@@ -1363,6 +1363,69 @@ int move_pose_plan_impl(const T* q_start, const T* goal_pos, const T* goal_quat,
   CUDA_TRY(cudaGetLastError());
   return PNP_OK;
 }
+
+// Axis-mode planner: move_pose_plan_impl's checks plus the tool axis, all before anything is enqueued on the stream.
+template <typename T>
+int move_axis_plan_impl(const T* q_start, const T* goal_pos, const T* goal_axis, int64_t n, const PnpMovePoseParams* mp,
+                        const PnpIkParams* params, const double* tool_axis, T* pos_traj, T* axis_traj, T* quat_traj,
+                        T* q_traj, int32_t* traj_len, T* q_final, int32_t* n_solves, int32_t* status,
+                        unsigned long long* counters, void* stream) {
+  int rc = check_ik_params(params);
+  if (rc) return rc;
+  if (!mp) return fail(PNP_EINVAL, "move_axis params is NULL");
+  if (mp->traj_cap < 1 || mp->max_traj_points < 0)
+    return fail(PNP_EINVAL, "move_axis params: need traj_cap >= 1 and max_traj_points >= 0");
+  if (!(mp->step_size > 0.0) || !(mp->rot_step > 0.0))
+    return fail(PNP_EINVAL, "move_axis params: step_size and rot_step must be > 0");
+  if (!(mp->ik_rot_thresh > 0.0) || !(mp->ik_rot_weight > 0.0))
+    return fail(PNP_EINVAL, "move_axis params: ik_rot_thresh and ik_rot_weight must be > 0");
+  // a plan whose last solve converged short of the planner's tolerance would re-aim at the goal forever
+  if (!(mp->pos_thresh >= params->pos_thresh) || !(mp->rot_thresh >= mp->ik_rot_thresh))
+    return fail(PNP_EINVAL, "move_axis params: need pos_thresh >= params->pos_thresh and rot_thresh >= ik_rot_thresh");
+  double basis[9];
+  if (!tool_basis(tool_axis, basis))
+    return fail(PNP_EINVAL, "move_ik_plan_axis: tool_axis must be non-null, finite and nonzero");
+  if (n < 0 || (n > 0 && (!q_start || !goal_pos || !goal_axis || !pos_traj || !axis_traj || !quat_traj || !traj_len ||
+                          !q_final || !n_solves || !status)))
+    return fail(PNP_EINVAL, "move_ik_plan_axis: null pointer or negative n");
+  if (n >= (int64_t(1) << 31)) return fail(PNP_EINVAL, "move_ik_plan_axis: n must be < 2^31 per call");
+  DeviceState* s;
+  if ((rc = current_state(&s))) return rc;
+  bool spec;
+  if ((rc = pick_kin(s, params->kinematics, &spec))) return rc;
+  if (n == 0) return PNP_OK;
+  const bool small = n <= (long long)s->sm_count * pnp::IK_BLOCK;
+  const int block = pnp::IK_BLOCK;
+  int occ;
+  rc = spec ? occupancy<pnp::move_axis_plan_kernel<T, pnp::SpecKin>>(s, block, 0, &occ)
+            : occupancy<pnp::move_axis_plan_kernel<T, pnp::GenericKin>>(s, block, 0, &occ);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  pnp::MoveAxisArgs<T> a{};
+  if ((rc = stream_ticket(s, st, &a.ik.ticket))) return rc;
+  a.ik.target_pos = goal_pos; a.ik.target_axis = goal_axis; a.ik.n = (unsigned)n;
+  a.ik.k = make_ik_const<T>(params);
+  a.ik.rot_thresh = (T)mp->ik_rot_thresh; a.ik.rot_weight = (T)mp->ik_rot_weight;
+  for (int i = 0; i < 9; ++i) a.ik.basis[i] = (T)basis[i];
+  a.ik.counters = counters;
+  a.q_start = q_start;
+  a.pos_thresh = (T)mp->pos_thresh; a.rot_thresh = (T)mp->rot_thresh;
+  a.step_size = (T)mp->step_size; a.rot_step = (T)mp->rot_step;
+  a.max_traj_points = mp->max_traj_points; a.traj_cap = mp->traj_cap;
+  a.pos_traj = pos_traj; a.axis_traj = axis_traj; a.quat_traj = quat_traj; a.q_traj = q_traj;
+  a.traj_len = traj_len; a.q_final = q_final; a.n_solves = n_solves; a.status = status;
+  // the pose planner's geometry: plans differ in length, so warps reserve ~1/8 of their share within [32, 128]
+  const PersistentGrid g = persistent_grid(s, n, 1, block, occ, small, 8, 128);
+  a.ik.chunk = g.chunk;
+  a.ik.solo_warp = small ? 1u : 0u;
+  if (spec)
+    pnp::move_axis_plan_kernel<T, pnp::SpecKin><<<g.grid, block, 0, st>>>(a);
+  else
+    pnp::move_axis_plan_kernel<T, pnp::GenericKin><<<g.grid, block, 0, st>>>(a);
+  ++g_launches;
+  CUDA_TRY(cudaGetLastError());
+  return PNP_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1517,6 +1580,23 @@ int pnp_move_ik_plan_pose_f64(const double* q_start, const double* goal_pos, con
                               int32_t* status, unsigned long long* counters, void* stream) {
   return move_pose_plan_impl<double>(q_start, goal_pos, goal_quat, n, move, params, pos_traj, quat_traj, q_traj, traj_len,
                                      q_final, n_solves, status, counters, stream);
+}
+
+int pnp_move_ik_plan_axis_f32(const float* q_start, const float* goal_pos, const float* goal_axis, int64_t n,
+                              const PnpMovePoseParams* move, const PnpIkParams* params, const double* tool_axis,
+                              float* pos_traj, float* axis_traj, float* quat_traj, float* q_traj, int32_t* traj_len,
+                              float* q_final, int32_t* n_solves, int32_t* status, unsigned long long* counters,
+                              void* stream) {
+  return move_axis_plan_impl<float>(q_start, goal_pos, goal_axis, n, move, params, tool_axis, pos_traj, axis_traj,
+                                    quat_traj, q_traj, traj_len, q_final, n_solves, status, counters, stream);
+}
+int pnp_move_ik_plan_axis_f64(const double* q_start, const double* goal_pos, const double* goal_axis, int64_t n,
+                              const PnpMovePoseParams* move, const PnpIkParams* params, const double* tool_axis,
+                              double* pos_traj, double* axis_traj, double* quat_traj, double* q_traj, int32_t* traj_len,
+                              double* q_final, int32_t* n_solves, int32_t* status, unsigned long long* counters,
+                              void* stream) {
+  return move_axis_plan_impl<double>(q_start, goal_pos, goal_axis, n, move, params, tool_axis, pos_traj, axis_traj,
+                                     quat_traj, q_traj, traj_len, q_final, n_solves, status, counters, stream);
 }
 
 int pnp_reward_f32(const float* ag, const float* dg, const float* ee_pos, const float* ee_quat, const float* width,

@@ -2635,6 +2635,195 @@ __global__ void __launch_bounds__(IK_BLOCK) move_pose_plan_kernel(const MovePose
 }
 
 // =============================================================================================
+// Axis-mode move planner (pnp_move_ik_plan_axis_*, an EXTENSION stated in oracle/move_axis_oracle.py): plan a move to
+// a goal position and a goal direction of the tool axis t, the roll about t free, every waypoint a solved axis task.
+//   round: d = goal_pos - p, a = R t, theta = atan2(|a x g|, a.g) (axis_pass_inline's expression); done when
+//          |d| <= pos_thresh and theta <= rot_thresh, CAPPED at max_traj_points points;
+//          f = min(1, step_size / |d|, rot_step / theta)
+//   up to three axis solves from q at the fractions h = f, f/2, f/20: (p + h d, normalize(cos(h theta) a +
+//   sin(h theta) m)), m = (g - (a.g) a) / |a x g| (the tangent turning a toward g; -b2 = -R u2 when exactly
+//   antiparallel, the solver's own n = b1), or the goal itself when h == 1; the first success appends (final_pos,
+//   final_axis, quat of the final frame, q) and moves there; three rejections: BROKE.
+// move_pose_plan_kernel's lane machinery with axis_pass / axis_success unchanged, i.e. every waypoint solve is the
+// plain axis solve of that aim from that q (in FP64 through the shared out-of-line axis_pass_call).  The lane keeps a
+// and b2 of its last point; the quaternion is formed once per accepted point, not per pass.
+// =============================================================================================
+template <typename T>
+struct MoveAxisArgs {
+  AxisIkArgs<T> ik;  // every waypoint's axis solve: k, rot_thresh (= ik_rot_thresh), rot_weight, basis; target_pos /
+                     // target_axis = the goals (axis_load_target); n, counters, ticket, chunk, solo_warp
+  const T* q_start;
+  T pos_thresh, rot_thresh, step_size, rot_step;
+  int max_traj_points, traj_cap;
+  T* pos_traj;       // [n][traj_cap][3]
+  T* axis_traj;      // [n][traj_cap][3]
+  T* quat_traj;      // [n][traj_cap][4]
+  T* q_traj;         // [n][traj_cap][7], nullable
+  int32_t* traj_len;
+  T* q_final;        // [n][7]
+  int32_t* n_solves;
+  int32_t* status;
+};
+
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(IK_BLOCK) move_axis_plan_kernel(const MoveAxisArgs<T> a) {
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  if (a.ik.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
+  const Trig<T> trig{s_tab};
+  enum { SOLVE = 0, DONE = 1, INIT = 2, IDLE = 3 };
+  unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
+  WarpPool pool;
+  bool exhausted = false, bad_goal = false;
+  unsigned e = 0;
+  size_t row = 0;  // e * traj_cap
+  // q: joints of the last point; qs: the running solve; (p, ax, b2): position, R t and R u2 of the last point;
+  // (gp, gd): the goal; (tp, td): the running aim
+  T q[NJ], qs[NJ], p[3] = {T(0), T(0), T(0)}, ax[3] = {T(0), T(0), T(1)}, b2[3] = {T(0), T(0), T(0)};
+  T gp[3] = {T(0), T(0), T(0)}, gd[3] = {T(0), T(0), T(1)}, tp[3] = {T(0), T(0), T(0)}, td[3] = {T(0), T(0), T(1)};
+#pragma unroll
+  for (int i = 0; i < NJ; ++i) q[i] = qs[i] = T(0);
+  int len = 0, solves = 0, st = 0, state = IDLE, it = 0, points = 0, attempt = 0;
+  auto append = [&](const T (&r)[4]) {
+    if (len < a.traj_cap) {
+      const size_t k = row + (size_t)len;
+#pragma unroll
+      for (int i = 0; i < 3; ++i) a.pos_traj[k * 3 + i] = p[i];
+#pragma unroll
+      for (int i = 0; i < 3; ++i) a.axis_traj[k * 3 + i] = ax[i];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) a.quat_traj[k * 4 + i] = r[i];
+      if (a.q_traj) {
+#pragma unroll
+        for (int i = 0; i < NJ; ++i) a.q_traj[k * NJ + i] = q[i];
+      }
+    } else {
+      st |= (int)PNP_MOVE_OVERFLOW;
+    }
+    ++len;
+  };
+
+  while (true) {
+    // ---- write back finished envs, refill idle lanes -------------------------------------------
+    if (state == DONE) {
+#pragma unroll
+      for (int i = 0; i < NJ; ++i) a.q_final[(size_t)e * NJ + i] = q[i];
+      a.traj_len[e] = len;
+      a.n_solves[e] = solves;
+      a.status[e] = st;
+      state = IDLE;
+    }
+    const bool want[1] = {state == IDLE && !exhausted};
+    pool.refill(want, exhausted, a.ik.n, a.ik.ticket, a.ik.chunk, [&](int, unsigned idx) {
+          e = idx;
+#pragma unroll
+          for (int i = 0; i < NJ; ++i) q[i] = qs[i] = a.q_start[(size_t)e * NJ + i];
+          axis_load_target(a.ik, e, gp, gd);
+          bad_goal = false;
+#pragma unroll
+          for (int i = 0; i < 3; ++i) bad_goal = bad_goal || !isfinite(gp[i]) || !isfinite(gd[i]);  // zero axis: NaN
+#pragma unroll
+          for (int i = 0; i < 3; ++i) { tp[i] = gp[i]; td[i] = gd[i]; }
+          row = (size_t)e * (size_t)a.traj_cap;
+          len = 0; solves = 0; st = 0; points = 0; attempt = 0;
+          it = a.ik.k.max_iters;
+          state = INIT;
+        });
+    if (!__any_sync(FULL, state != IDLE)) break;
+
+    // ---- one 5-row DLS pass for all lanes; a lane whose solve ends post-processes it --------------
+    bool choose = false;  // this lane starts a new solve: pick its aim below
+    axis_pass<T, Kin>(a.ik, trig, qs, tp, td, it, state != IDLE,
+                      [&](const T* pp, const T* R, const T* x, T pe, T th, int iterations, bool conv) {
+                        bool accept = true;  // INIT: point 0 = FK(q_start)
+                        if (state == SOLVE) {
+                          ++solves;
+                          c_n += 1; c_conv += conv ? 1 : 0; c_iter += (unsigned long long)iterations;
+                          accept = axis_success(a.ik, pe, th, conv);
+                          if (accept) {
+#pragma unroll
+                            for (int i = 0; i < NJ; ++i) q[i] = qs[i];
+                            ++points;
+                          }
+                        }
+                        if (accept) {
+#pragma unroll
+                          for (int i = 0; i < 3; ++i) {
+                            p[i] = pp[i];
+                            ax[i] = x[i];
+                            b2[i] = R[3 * i] * a.ik.basis[6] + R[3 * i + 1] * a.ik.basis[7] + R[3 * i + 2] * a.ik.basis[8];
+                          }
+                          T r[4];
+                          mat2quat_fast(R, r);
+                          append(r);
+                          attempt = 0;
+                        } else if (++attempt == 3) {
+                          st |= (int)PNP_MOVE_BROKE;
+                        }
+                        state = attempt == 3 ? DONE : SOLVE;
+                        choose = state == SOLVE;
+                      });
+
+    // ---- stop tests at the start of a round, then the aim of the next solve ------------------------
+    if (choose) {
+      const T d[3] = {gp[0] - p[0], gp[1] - p[1], gp[2] - p[2]};
+      const T dist = finish_sqrt((d[0] * d[0] + d[1] * d[1]) + d[2] * d[2]);
+      // the tilt left, written as axis_pass_inline writes the solver's: a solve aimed at the goal that converges ends
+      // the plan by construction (pos_thresh >= the IK's, rot_thresh >= ik_rot_thresh)
+      const T cr[3] = {ax[1] * gd[2] - ax[2] * gd[1], ax[2] * gd[0] - ax[0] * gd[2], ax[0] * gd[1] - ax[1] * gd[0]};
+      const T sn = sqrt_t((cr[0] * cr[0] + cr[1] * cr[1]) + cr[2] * cr[2]);
+      const T ad = (ax[0] * gd[0] + ax[1] * gd[1]) + ax[2] * gd[2];
+      const T th = atan2_t(sn, ad);
+      if (attempt == 0) {
+        if (bad_goal) {
+          st |= (int)PNP_MOVE_BROKE;
+          state = DONE;
+        } else if (dist <= a.pos_thresh && th <= a.rot_thresh) {
+          state = DONE;
+        } else if (points >= a.max_traj_points) {
+          st |= (int)PNP_MOVE_CAPPED;
+          state = DONE;
+        }
+      }
+      if (state == SOLVE) {
+        T f = T(1);
+        if (dist > T(0)) f = fmin(f, div_fast(a.step_size, dist));
+        if (th > T(0)) f = fmin(f, div_fast(a.rot_step, th));
+        const T h = attempt == 0 ? f : f * (attempt == 1 ? T(0.5) : T(0.05));
+        if (h == T(1)) {
+#pragma unroll
+          for (int i = 0; i < 3; ++i) { tp[i] = gp[i]; td[i] = gd[i]; }
+        } else {
+          // cos(h theta) a + sin(h theta) m, one sincos; sin(h theta) m = k w with w = g - (a.g) a and k = sin / |a x g|,
+          // or w = b2 and k = -sin when exactly antiparallel (k = 0 when aligned: theta = 0, the aim axis is a)
+          T s, c;
+          trig(h * th, &s, &c);
+          const bool tilted = sn > T(0);
+          const T k = tilted ? div_fast(s, sn) : (ad < T(0) ? -s : T(0));
+          T v[3];
+#pragma unroll
+          for (int i = 0; i < 3; ++i) {
+            tp[i] = p[i] + h * d[i];
+            v[i] = c * ax[i] + k * (tilted ? gd[i] - ad * ax[i] : b2[i]);
+          }
+          // normalised as axis_load_target normalises a loaded target axis
+          const T nv = sqrt_t(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
+#pragma unroll
+          for (int i = 0; i < 3; ++i) td[i] = v[i] / nv;
+        }
+#pragma unroll
+        for (int i = 0; i < NJ; ++i) qs[i] = q[i];  // every solve starts from the joints of the last point
+        it = 0;
+      }
+    } else {
+      ++it;
+    }
+  }
+  ik_counters_add(a.ik.counters, c_n, c_conv, c_iter);
+}
+
+// =============================================================================================
 // compute_reward / _is_success streaming kernel (panda_env.py:205-245, 303-306).
 //
 // HBM-bound: 60 B in + 4 B out per row (FP32 storage).  Each lane owns kRows consecutive rows

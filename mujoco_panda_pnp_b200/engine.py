@@ -701,6 +701,54 @@ def move_ik_plan_pose(q_start: torch.Tensor, goal_pos: torch.Tensor, goal_quat: 
                 status=status)
 
 
+def move_ik_plan_axis(q_start: torch.Tensor, goal_pos: torch.Tensor, goal_axis: torch.Tensor, params: PnpIkParams,
+                      tool_axis=(0.0, 0.0, 1.0), pos_thresh: float = 0.01, rot_thresh: float = 0.05,
+                      step_size: float = 0.01, rot_step: float = 0.05, ik_rot_thresh: float = 1e-2,
+                      rot_weight: float = 1.0, max_traj_points: int = 200, traj_cap: Optional[int] = None,
+                      want_q_traj: bool = True, counters: Optional[torch.Tensor] = None) -> dict:
+    """Axis-mode move planner (pnp_move_ik_plan_axis_*, extension): plan N moves to a goal position and a goal
+    direction goal_axis[N,3] (world frame, any norm) of the site-frame ``tool_axis``, the roll about it free, every
+    waypoint a solved axis task (oracle/move_axis_oracle.py states the semantics).  rot_thresh, rot_step, ik_rot_thresh
+    and rot_weight apply to the axis angle.  Otherwise as move_ik_plan_pose: ``pos_thresh`` >= params.pos_thresh,
+    ``rot_thresh`` >= ``ik_rot_thresh``, traj_cap defaults to max_traj_points + 1.  Never synchronises.
+
+    Returns dict(pos_traj[N,cap,3], axis_traj[N,cap,3] (the world tool axis), quat_traj[N,cap,4], q_traj[N,cap,7] (None
+    unless want_q_traj), traj_len[N], q_final[N,7], n_solves[N], status[N]); rows past traj_len are zero."""
+    lib = _lib.load()
+    dt = q_start.dtype
+    if dt not in (torch.float32, torch.float64):
+        raise ValueError("q_start must be float32 or float64")
+    q_start = _check_cuda("q_start", q_start, dt, (7,))
+    goal_pos, goal_axis, tool = _axis_inputs(goal_pos, goal_axis, tool_axis)
+    n = q_start.shape[0]
+    if goal_pos.dtype != dt or goal_pos.shape[0] != n:
+        raise ValueError("q_start, goal_pos and goal_axis disagree on N or dtype")
+    if counters is not None and (counters.dtype != torch.int64 or counters.numel() < 4 or not counters.is_cuda):
+        raise ValueError("counters must be a CUDA int64 tensor with >= 4 elements")
+    cap = int(traj_cap) if traj_cap is not None else int(max_traj_points) + 1
+    mp = _lib.PnpMovePoseParams(float(pos_thresh), float(rot_thresh), float(step_size), float(rot_step),
+                                float(ik_rot_thresh), float(rot_weight), int(max_traj_points), cap)
+    dev = q_start.device
+    with torch.cuda.device(dev):
+        pos_traj = torch.zeros((n, max(cap, 0), 3), dtype=dt, device=dev)
+        axis_traj = torch.zeros((n, max(cap, 0), 3), dtype=dt, device=dev)
+        quat_traj = torch.zeros((n, max(cap, 0), 4), dtype=dt, device=dev)
+        q_traj = torch.zeros((n, max(cap, 0), 7), dtype=dt, device=dev) if want_q_traj else None
+        tlen = torch.empty((n,), dtype=torch.int32, device=dev)
+        qf = torch.empty((n, 7), dtype=dt, device=dev)
+        solves = torch.empty((n,), dtype=torch.int32, device=dev)
+        status = torch.empty((n,), dtype=torch.int32, device=dev)
+        fn = lib.pnp_move_ik_plan_axis_f32 if dt == torch.float32 else lib.pnp_move_ik_plan_axis_f64
+        _lib.check(
+            fn(_ptr(q_start), _ptr(goal_pos), _ptr(goal_axis), n, ctypes.byref(mp), ctypes.byref(params), tool,
+               _ptr(pos_traj), _ptr(axis_traj), _ptr(quat_traj), _ptr(q_traj), _ptr(tlen), _ptr(qf), _ptr(solves),
+               _ptr(status), _ptr(counters), _stream()),
+            "pnp_move_ik_plan_axis",
+        )
+    return dict(pos_traj=pos_traj, axis_traj=axis_traj, quat_traj=quat_traj, q_traj=q_traj, traj_len=tlen, q_final=qf,
+                n_solves=solves, status=status)
+
+
 # ---------------------------------------------------------------------------------------------
 # reward
 # ---------------------------------------------------------------------------------------------

@@ -17,6 +17,7 @@
  *                          dangling in the reference - an extension defined here)
  *   pnp_ik_axis_solve_*    a tool position and approach direction, the roll about the tool axis free (an extension
  *                          defined here)
+ *   pnp_ik_axis_cone_solve_*  the same with the approach direction anywhere within a cone (an extension defined here)
  *   pnp_move_ik_plan_*     the whole MoveIKSkill.reset planner (skills/move.py:76-191)
  *   pnp_move_ik_plan_pose_*  the same planner to a goal position and orientation (an extension defined here)
  *   pnp_move_ik_plan_axis_*  the same planner to a goal position and tool-axis direction, the roll free (an
@@ -315,6 +316,46 @@ int pnp_ik_axis_solve_multistart_f64(const double* target_pos, const double* tar
                                      double* final_quat, double* pos_err, double* axis_err, int32_t* iters,
                                      uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
                                      unsigned long long* restart_stats, void* scratch, void* stream);
+
+/* ---- cone-tolerant axis IK: the approach direction anywhere within a cone (EXTENSION) -------- */
+/* pnp_ik_axis_solve_* with cone_angle alpha in [0, pi] (radians, one per call): the tool axis a may end anywhere within
+ * alpha of the target axis d.  With theta, n, b1, b2 as in the axis solve, each pass:
+ *   on = theta > alpha (false for a NaN theta);  w' = rot_weight if on, else 0;  g = theta - alpha if on, else 0
+ *   e = [tp - p ; w' g n.b1 ; w' g n.b2],  J = [jacp ; w' b1^T jacr ; w' b2^T jacr],  dq as in the axis solve;
+ *   converged when |tp - p| < pos_thresh and theta - alpha < rot_thresh; success adds |tp - p| < 2 pos_thresh and
+ *   theta - alpha < 2 rot_thresh.
+ * Inside the cone the tilt rows are dropped, so the pass is the damped position pass and the axis moves freely within
+ * the cone; alpha = 0 is the axis solve and alpha = pi the position solve.  axis_err stays theta, the true angle.
+ * Outputs, counters, restarts, seeds and scratch as pnp_ik_axis_solve_* / pnp_ik_axis_solve_multistart_*.  Rejected
+ * with PNP_EINVAL before anything is enqueued: everything the axis entry points reject, and a NaN, negative or > pi
+ * cone_angle.  The call never synchronises the host (it can be captured in a CUDA graph).  The statement is
+ * oracle/cone_ik_oracle.py. */
+int pnp_ik_axis_cone_solve_f32(const float* target_pos, const float* target_axis, const float* q_init,
+                               int32_t q_init_stride, int64_t n, const PnpIkParams* params, const double* tool_axis,
+                               double rot_thresh, double cone_angle, double rot_weight, float* q_out, float* final_pos,
+                               float* final_axis, float* final_quat, float* pos_err, float* axis_err, int32_t* iters,
+                               uint8_t* flags, unsigned long long* counters, void* stream);
+int pnp_ik_axis_cone_solve_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                               int32_t q_init_stride, int64_t n, const PnpIkParams* params, const double* tool_axis,
+                               double rot_thresh, double cone_angle, double rot_weight, double* q_out,
+                               double* final_pos, double* final_axis, double* final_quat, double* pos_err,
+                               double* axis_err, int32_t* iters, uint8_t* flags, unsigned long long* counters,
+                               void* stream);
+int pnp_ik_axis_cone_solve_multistart_f32(const float* target_pos, const float* target_axis, const float* q_init,
+                                          int32_t q_init_stride, int64_t n, const float* seeds, int32_t n_seeds,
+                                          const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                          double cone_angle, double rot_weight, float* q_out, float* final_pos,
+                                          float* final_axis, float* final_quat, float* pos_err, float* axis_err,
+                                          int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                          unsigned long long* restart_stats, void* scratch, void* stream);
+int pnp_ik_axis_cone_solve_multistart_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                                          int32_t q_init_stride, int64_t n, const double* seeds, int32_t n_seeds,
+                                          const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                          double cone_angle, double rot_weight, double* q_out, double* final_pos,
+                                          double* final_axis, double* final_quat, double* pos_err, double* axis_err,
+                                          int32_t* iters, uint8_t* flags, uint8_t* attempt,
+                                          unsigned long long* counters, unsigned long long* restart_stats,
+                                          void* scratch, void* stream);
 
 /* ---- full MoveIKSkill.reset trajectory planner (skills/move.py:76-191) -------------------- */
 typedef struct PnpMoveParams {

@@ -124,6 +124,16 @@ SIGNATURES = {
     "pnp_ik_axis_solve_multistart_f64": (c_int, [_P, _P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams),
                                                  POINTER(c_double), c_double, c_double, _P, _P, _P, _P, _P, _P, _P, _P,
                                                  _P, _P, _P, _P, _P]),
+    "pnp_ik_axis_cone_solve_f32": (c_int, [_P, _P, _P, c_int32, c_int64, POINTER(PnpIkParams), POINTER(c_double),
+                                           c_double, c_double, c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_ik_axis_cone_solve_f64": (c_int, [_P, _P, _P, c_int32, c_int64, POINTER(PnpIkParams), POINTER(c_double),
+                                           c_double, c_double, c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_ik_axis_cone_solve_multistart_f32": (c_int, [_P, _P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams),
+                                                      POINTER(c_double), c_double, c_double, c_double, _P, _P, _P, _P,
+                                                      _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pnp_ik_axis_cone_solve_multistart_f64": (c_int, [_P, _P, _P, c_int32, c_int64, _P, c_int32, POINTER(PnpIkParams),
+                                                      POINTER(c_double), c_double, c_double, c_double, _P, _P, _P, _P,
+                                                      _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_ik_plan_f32": (c_int, [_P, _P, c_int64, POINTER(PnpMoveParams), POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_ik_plan_f64": (c_int, [_P, _P, c_int64, POINTER(PnpMoveParams), POINTER(PnpIkParams), _P, _P, _P, _P, _P, _P, _P]),
     "pnp_move_plan_order_f32": (c_int, [_P, _P, c_int64, _P, c_int32, _P]),

@@ -1105,16 +1105,24 @@ bool tool_basis(const double* tool_axis, double (&out)[9]) {
   return true;
 }
 
-template <typename T>
+// The argument block of the axis solve (kCone false) or of the cone solve (kCone true)
+template <typename T, bool kCone>
+using AxisArgsOf = std::conditional_t<kCone, pnp::AxisConeIkArgs<T>, pnp::AxisIkArgs<T>>;
+
+// The axis solve, or with kCone the cone solve of cone angle cone_angle (ignored without kCone)
+template <typename T, bool kCone = false>
 int axis_solve_impl(const T* tpos, const T* taxis, const T* q_init, int32_t q_init_stride, int64_t n,
-                    const PnpIkParams* params, const double* tool_axis, double rot_thresh, double rot_weight, T* q_out,
-                    T* final_pos, T* final_axis, T* final_quat, T* pos_err, T* axis_err, int32_t* iters, uint8_t* flags,
-                    unsigned long long* counters, void* stream, pnp::AxisIkArgs<T>* args_out = nullptr) {
+                    const PnpIkParams* params, const double* tool_axis, double rot_thresh, double rot_weight,
+                    double cone_angle, T* q_out, T* final_pos, T* final_axis, T* final_quat, T* pos_err, T* axis_err,
+                    int32_t* iters, uint8_t* flags, unsigned long long* counters, void* stream,
+                    AxisArgsOf<T, kCone>* args_out = nullptr) {
   int rc = check_ik_params(params);
   if (rc) return rc;
   double basis[9];
   if (!tool_basis(tool_axis, basis)) return fail(PNP_EINVAL, "ik_axis_solve: tool_axis must be non-null, finite and nonzero");
   if (!(rot_thresh > 0.0) || !(rot_weight > 0.0)) return fail(PNP_EINVAL, "rot_thresh and rot_weight must be > 0");
+  if (kCone && !(cone_angle >= 0.0 && cone_angle <= M_PI))  // NaN fails both
+    return fail(PNP_EINVAL, "ik_axis_cone_solve: cone_angle must be in [0, pi]");
   if (n < 0 || (n > 0 && (!tpos || !taxis || !q_init || !q_out)))
     return fail(PNP_EINVAL, "ik_axis_solve: null pointer or negative n");
   if (q_init_stride != 0 && q_init_stride != PNP_NJOINT) return fail(PNP_EINVAL, "q_init_stride must be 0 or 7");
@@ -1125,8 +1133,9 @@ int axis_solve_impl(const T* tpos, const T* taxis, const T* q_init, int32_t q_in
   if (n == 0) return PNP_OK;
   if (n >= (int64_t(1) << 31)) return fail(PNP_EINVAL, "ik_axis_solve: n must be < 2^31 per call");
   cudaStream_t st = (cudaStream_t)stream;
-  pnp::AxisIkArgs<T> a;
+  AxisArgsOf<T, kCone> a;
   if ((rc = stream_ticket(s, st, &a.ticket))) return rc;
+  if constexpr (kCone) a.cone_angle = (T)cone_angle;
   a.target_pos = tpos; a.target_axis = taxis; a.q_init = q_init; a.q_init_stride = q_init_stride; a.n = (unsigned)n;
   a.k = make_ik_const<T>(params);
   a.rot_thresh = (T)rot_thresh; a.rot_weight = (T)rot_weight;
@@ -1136,45 +1145,61 @@ int axis_solve_impl(const T* tpos, const T* taxis, const T* q_init, int32_t q_in
   const bool small = n <= (long long)s->sm_count * pnp::IK_BLOCK;
   const int block = pnp::IK_BLOCK;
   int occ;
-  rc = spec ? occupancy<pnp::ik_axis_solve_kernel<T, pnp::SpecKin>>(s, block, 0, &occ)
-            : occupancy<pnp::ik_axis_solve_kernel<T, pnp::GenericKin>>(s, block, 0, &occ);
+  if constexpr (kCone)
+    rc = spec ? occupancy<pnp::ik_axis_cone_solve_kernel<T, pnp::SpecKin>>(s, block, 0, &occ)
+              : occupancy<pnp::ik_axis_cone_solve_kernel<T, pnp::GenericKin>>(s, block, 0, &occ);
+  else
+    rc = spec ? occupancy<pnp::ik_axis_solve_kernel<T, pnp::SpecKin>>(s, block, 0, &occ)
+              : occupancy<pnp::ik_axis_solve_kernel<T, pnp::GenericKin>>(s, block, 0, &occ);
   if (rc) return rc;
   const PersistentGrid g = persistent_grid(s, n, 1, block, occ, small, 16, 256);
   a.chunk = g.chunk;
   a.solo_warp = small ? 1u : 0u;
   if (args_out) *args_out = a;  // the multistart's restarts use this block
-  if (spec)
-    pnp::ik_axis_solve_kernel<T, pnp::SpecKin><<<g.grid, block, 0, st>>>(a);
-  else
-    pnp::ik_axis_solve_kernel<T, pnp::GenericKin><<<g.grid, block, 0, st>>>(a);
+  if constexpr (kCone) {
+    if (spec)
+      pnp::ik_axis_cone_solve_kernel<T, pnp::SpecKin><<<g.grid, block, 0, st>>>(a);
+    else
+      pnp::ik_axis_cone_solve_kernel<T, pnp::GenericKin><<<g.grid, block, 0, st>>>(a);
+  } else {
+    if (spec)
+      pnp::ik_axis_solve_kernel<T, pnp::SpecKin><<<g.grid, block, 0, st>>>(a);
+    else
+      pnp::ik_axis_solve_kernel<T, pnp::GenericKin><<<g.grid, block, 0, st>>>(a);
+  }
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return PNP_OK;
 }
 
-// Multi-start axis solve: axis_solve_impl, then the restart waves of ms_axis_wave_kernel (see multistart_impl).
-template <typename T>
+// Multi-start axis solve: axis_solve_impl, then the restart waves of ms_axis_wave_kernel (see multistart_impl); with
+// kCone the cone solve and ms_axis_cone_wave_kernel, same group width and override.
+template <typename T, bool kCone = false>
 int axis_multistart_impl(const T* tpos, const T* taxis, const T* q_init, int32_t q_init_stride, int64_t n, const T* seeds,
                          int32_t n_seeds, const PnpIkParams* params, const double* tool_axis, double rot_thresh,
-                         double rot_weight, T* q_out, T* final_pos, T* final_axis, T* final_quat, T* pos_err,
-                         T* axis_err, int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
-                         unsigned long long* restart_stats, void* scratch, void* stream) {
+                         double rot_weight, double cone_angle, T* q_out, T* final_pos, T* final_axis, T* final_quat,
+                         T* pos_err, T* axis_err, int32_t* iters, uint8_t* flags, uint8_t* attempt,
+                         unsigned long long* counters, unsigned long long* restart_stats, void* scratch, void* stream) {
   const size_t m = (size_t)n;
-  return multistart_impl<pnp::AxisIkArgs<T>, pnp::IK_OUT_SEPARATE>(
-      "ik_axis_multistart", n, seeds, n_seeds, params, flags, iters, attempt, counters, restart_stats, scratch,
+  return multistart_impl<AxisArgsOf<T, kCone>, pnp::IK_OUT_SEPARATE>(
+      kCone ? "ik_axis_cone_multistart" : "ik_axis_multistart", n, seeds, n_seeds, params, flags, iters, attempt, counters, restart_stats, scratch,
       {byte_range(q_out, m * PNP_NJOINT * sizeof(T)), byte_range(final_pos, m * 3 * sizeof(T)),
        byte_range(final_axis, m * 3 * sizeof(T)), byte_range(final_quat, m * 4 * sizeof(T)),
        byte_range(pos_err, m * sizeof(T)), byte_range(axis_err, m * sizeof(T)), byte_range(iters, m * sizeof(int32_t)),
        byte_range(flags, m)},
       kMsAxisGroup, "PNP_MS_AXIS_GROUP", stream,
-      [&](int32_t* iters0, pnp::AxisIkArgs<T>& a) {
-        return axis_solve_impl<T>(tpos, taxis, q_init, q_init_stride, n, params, tool_axis, rot_thresh, rot_weight, q_out,
-                                  final_pos, final_axis, final_quat, pos_err, axis_err, iters0, flags, counters, stream,
-                                  &a);
+      [&](int32_t* iters0, AxisArgsOf<T, kCone>& a) {
+        return axis_solve_impl<T, kCone>(tpos, taxis, q_init, q_init_stride, n, params, tool_axis, rot_thresh,
+                                         rot_weight, cone_angle, q_out, final_pos, final_axis, final_quat, pos_err,
+                                         axis_err, iters0, flags, counters, stream, &a);
       },
       [&](DeviceState* s, bool spec, const auto& m, cudaStream_t st) {
-        return spec ? launch_ms_wave<pnp::ms_axis_wave_kernel<T, pnp::SpecKin>>(s, m, st)
-                    : launch_ms_wave<pnp::ms_axis_wave_kernel<T, pnp::GenericKin>>(s, m, st);
+        if constexpr (kCone)
+          return spec ? launch_ms_wave<pnp::ms_axis_cone_wave_kernel<T, pnp::SpecKin>>(s, m, st)
+                      : launch_ms_wave<pnp::ms_axis_cone_wave_kernel<T, pnp::GenericKin>>(s, m, st);
+        else
+          return spec ? launch_ms_wave<pnp::ms_axis_wave_kernel<T, pnp::SpecKin>>(s, m, st)
+                      : launch_ms_wave<pnp::ms_axis_wave_kernel<T, pnp::GenericKin>>(s, m, st);
       });
 }
 
@@ -1472,8 +1497,8 @@ int pnp_ik_axis_solve_f32(const float* target_pos, const float* target_axis, con
                           float* pos_err, float* axis_err, int32_t* iters, uint8_t* flags, unsigned long long* counters,
                           void* stream) {
   return axis_solve_impl<float>(target_pos, target_axis, q_init, q_init_stride, n, params, tool_axis, rot_thresh,
-                                rot_weight, q_out, final_pos, final_axis, final_quat, pos_err, axis_err, iters, flags,
-                                counters, stream);
+                                rot_weight, 0.0, q_out, final_pos, final_axis, final_quat, pos_err, axis_err, iters,
+                                flags, counters, stream);
 }
 int pnp_ik_axis_solve_f64(const double* target_pos, const double* target_axis, const double* q_init,
                           int32_t q_init_stride, int64_t n, const PnpIkParams* params, const double* tool_axis,
@@ -1481,8 +1506,8 @@ int pnp_ik_axis_solve_f64(const double* target_pos, const double* target_axis, c
                           double* final_quat, double* pos_err, double* axis_err, int32_t* iters, uint8_t* flags,
                           unsigned long long* counters, void* stream) {
   return axis_solve_impl<double>(target_pos, target_axis, q_init, q_init_stride, n, params, tool_axis, rot_thresh,
-                                 rot_weight, q_out, final_pos, final_axis, final_quat, pos_err, axis_err, iters, flags,
-                                 counters, stream);
+                                 rot_weight, 0.0, q_out, final_pos, final_axis, final_quat, pos_err, axis_err, iters,
+                                 flags, counters, stream);
 }
 
 int pnp_ik_axis_solve_multistart_f32(const float* target_pos, const float* target_axis, const float* q_init,
@@ -1493,8 +1518,8 @@ int pnp_ik_axis_solve_multistart_f32(const float* target_pos, const float* targe
                                      uint8_t* attempt, unsigned long long* counters, unsigned long long* restart_stats,
                                      void* scratch, void* stream) {
   return axis_multistart_impl<float>(target_pos, target_axis, q_init, q_init_stride, n, seeds, n_seeds, params, tool_axis,
-                                     rot_thresh, rot_weight, q_out, final_pos, final_axis, final_quat, pos_err, axis_err,
-                                     iters, flags, attempt, counters, restart_stats, scratch, stream);
+                                     rot_thresh, rot_weight, 0.0, q_out, final_pos, final_axis, final_quat, pos_err,
+                                     axis_err, iters, flags, attempt, counters, restart_stats, scratch, stream);
 }
 int pnp_ik_axis_solve_multistart_f64(const double* target_pos, const double* target_axis, const double* q_init,
                                      int32_t q_init_stride, int64_t n, const double* seeds, int32_t n_seeds,
@@ -1504,8 +1529,54 @@ int pnp_ik_axis_solve_multistart_f64(const double* target_pos, const double* tar
                                      uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
                                      unsigned long long* restart_stats, void* scratch, void* stream) {
   return axis_multistart_impl<double>(target_pos, target_axis, q_init, q_init_stride, n, seeds, n_seeds, params,
-                                      tool_axis, rot_thresh, rot_weight, q_out, final_pos, final_axis, final_quat, pos_err,
-                                      axis_err, iters, flags, attempt, counters, restart_stats, scratch, stream);
+                                      tool_axis, rot_thresh, rot_weight, 0.0, q_out, final_pos, final_axis, final_quat,
+                                      pos_err, axis_err, iters, flags, attempt, counters, restart_stats, scratch, stream);
+}
+
+int pnp_ik_axis_cone_solve_f32(const float* target_pos, const float* target_axis, const float* q_init,
+                               int32_t q_init_stride, int64_t n, const PnpIkParams* params, const double* tool_axis,
+                               double rot_thresh, double cone_angle, double rot_weight, float* q_out, float* final_pos,
+                               float* final_axis, float* final_quat, float* pos_err, float* axis_err, int32_t* iters,
+                               uint8_t* flags, unsigned long long* counters, void* stream) {
+  return axis_solve_impl<float, true>(target_pos, target_axis, q_init, q_init_stride, n, params, tool_axis, rot_thresh,
+                                      rot_weight, cone_angle, q_out, final_pos, final_axis, final_quat, pos_err, axis_err,
+                                      iters, flags, counters, stream);
+}
+int pnp_ik_axis_cone_solve_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                               int32_t q_init_stride, int64_t n, const PnpIkParams* params, const double* tool_axis,
+                               double rot_thresh, double cone_angle, double rot_weight, double* q_out,
+                               double* final_pos, double* final_axis, double* final_quat, double* pos_err,
+                               double* axis_err, int32_t* iters, uint8_t* flags, unsigned long long* counters,
+                               void* stream) {
+  return axis_solve_impl<double, true>(target_pos, target_axis, q_init, q_init_stride, n, params, tool_axis, rot_thresh,
+                                       rot_weight, cone_angle, q_out, final_pos, final_axis, final_quat, pos_err,
+                                       axis_err, iters, flags, counters, stream);
+}
+
+int pnp_ik_axis_cone_solve_multistart_f32(const float* target_pos, const float* target_axis, const float* q_init,
+                                          int32_t q_init_stride, int64_t n, const float* seeds, int32_t n_seeds,
+                                          const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                          double cone_angle, double rot_weight, float* q_out, float* final_pos,
+                                          float* final_axis, float* final_quat, float* pos_err, float* axis_err,
+                                          int32_t* iters, uint8_t* flags, uint8_t* attempt, unsigned long long* counters,
+                                          unsigned long long* restart_stats, void* scratch, void* stream) {
+  return axis_multistart_impl<float, true>(target_pos, target_axis, q_init, q_init_stride, n, seeds, n_seeds, params,
+                                           tool_axis, rot_thresh, rot_weight, cone_angle, q_out, final_pos, final_axis,
+                                           final_quat, pos_err, axis_err, iters, flags, attempt, counters,
+                                           restart_stats, scratch, stream);
+}
+int pnp_ik_axis_cone_solve_multistart_f64(const double* target_pos, const double* target_axis, const double* q_init,
+                                          int32_t q_init_stride, int64_t n, const double* seeds, int32_t n_seeds,
+                                          const PnpIkParams* params, const double* tool_axis, double rot_thresh,
+                                          double cone_angle, double rot_weight, double* q_out, double* final_pos,
+                                          double* final_axis, double* final_quat, double* pos_err, double* axis_err,
+                                          int32_t* iters, uint8_t* flags, uint8_t* attempt,
+                                          unsigned long long* counters, unsigned long long* restart_stats,
+                                          void* scratch, void* stream) {
+  return axis_multistart_impl<double, true>(target_pos, target_axis, q_init, q_init_stride, n, seeds, n_seeds, params,
+                                            tool_axis, rot_thresh, rot_weight, cone_angle, q_out, final_pos, final_axis,
+                                            final_quat, pos_err, axis_err, iters, flags, attempt, counters,
+                                            restart_stats, scratch, stream);
 }
 
 int pnp_move_plan_order_f32(const float* q_start, const float* target, int64_t n, uint32_t* order, int32_t kinematics,

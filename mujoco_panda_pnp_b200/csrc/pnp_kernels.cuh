@@ -1902,6 +1902,25 @@ struct AxisIkArgs {
   unsigned solo_warp;  // small batches: 4 warps load the trig table, only warp 0 works
 };
 
+// x * y and x - y rounded on their own: never fused into an FMA
+__device__ __forceinline__ float mul_rn(float x, float y) { return __fmul_rn(x, y); }
+__device__ __forceinline__ double mul_rn(double x, double y) { return __dmul_rn(x, y); }
+__device__ __forceinline__ float sub_rn(float x, float y) { return __fsub_rn(x, y); }
+__device__ __forceinline__ double sub_rn(double x, double y) { return __dsub_rn(x, y); }
+
+// Cone-tolerant axis IK (pnp_ik_axis_cone_solve_*, stated in oracle/cone_ik_oracle.py): the axis solve with the target
+// axis accepted anywhere within cone_angle alpha of d.  The tilt rows are live only outside the cone:
+//   on = theta > alpha (false for a NaN theta);  w' = on ? w : 0;  g = on ? theta - alpha : 0
+//   e = [tp - p ; w' g n.b1 ; w' g n.b2],  J = [jacp ; w' b1^T jacr ; w' b2^T jacr]
+//   converged  <=>  |tp - p| < pos_thresh  and  theta - alpha < rot_thresh
+// Inside the cone the rows are zero and the 5x5 system is the position solver's 3x3 plus damping I2, so the step is the
+// damped position step.  The switch is a select on the weight, one compare per pass; the kernels are the axis kernels'
+// pieces with kCone set, and alpha rides after the axis block so that block keeps its layout.
+template <typename T>
+struct AxisConeIkArgs : AxisIkArgs<T> {
+  T cone_angle;     // alpha in [0, pi] (checked on the host)
+};
+
 // The pieces of an axis solve that ik_axis_solve_kernel and the multistart restarts (ms_axis_wave_kernel) share, so
 // that a restart attempt runs the plain kernel's arithmetic bit for bit.
 // Target of query e: its position and its axis normalised on load.
@@ -1919,10 +1938,12 @@ __device__ __forceinline__ void axis_load_target(const AxisIkArgs<T>& a, unsigne
 // One 5-row DLS pass at q (pass number `it`): evaluate the error and test convergence; a lane that is `active` and
 // finishes in this pass calls done(pp, R, ax, pe, th, iterations, conv) with the site position and frame, the world
 // tool axis and the errors at the q it finished at (q is still that q during the call).  Then q takes the DLS step -
-// unconditionally: the caller discards the q of a lane that has finished.
-template <typename T, typename Kin, typename Done>
+// unconditionally: the caller discards the q of a lane that has finished.  kCone: the cone pass of cone angle alpha
+// (th stays theta, the true angle).
+template <typename T, typename Kin, bool kCone = false, typename Done>
 __device__ __forceinline__ void axis_pass_inline(const AxisIkArgs<T>& a, const Trig<T>& trig, T (&q)[NJ],
-                                                 const T (&tp)[3], const T (&d)[3], int it, bool active, Done done) {
+                                                 const T (&tp)[3], const T (&d)[3], int it, bool active, Done done,
+                                                 T alpha = T(0)) {
   T s[NJ], c[NJ];
 #pragma unroll
   for (int i = 0; i < NJ; ++i) trig(q[i] - Kin::template qref<T>(i), &s[i], &c[i]);
@@ -1944,18 +1965,27 @@ __device__ __forceinline__ void axis_pass_inline(const AxisIkArgs<T>& a, const T
   const T inv = tilted ? rcp_t(sn) : T(0);
   const T nb1 = tilted ? ((cr[0] * b1[0] + cr[1] * b1[1]) + cr[2] * b1[2]) * inv : (ad < T(0) ? T(1) : T(0));
   const T nb2 = tilted ? ((cr[0] * b2[0] + cr[1] * b2[1]) + cr[2] * b2[2]) * inv : T(0);
-  const T wth = a.rot_weight * th;
-  T err[5] = {tp[0] - pp[0], tp[1] - pp[1], tp[2] - pp[2], wth * nb1, wth * nb2};
+  // cone: the tilt rows are live only outside the cone, a select on the weight (false for a NaN theta: the rows drop
+  // and the pass is a position pass).  The cone's products are rounded on their own (mul_rn): the FP32 pass is inlined
+  // in the plain and the restart kernel, and a product ptxas may fuse into its neighbours in one kernel and not in the
+  // other would break their bit-identity.
+  const bool on = kCone ? th > alpha : true;
+  const T wth = kCone ? (on ? mul_rn(a.rot_weight, sub_rn(th, alpha)) : T(0)) : a.rot_weight * th;
+  T err[5] = {tp[0] - pp[0], tp[1] - pp[1], tp[2] - pp[2], kCone ? mul_rn(wth, nb1) : wth * nb1,
+              kCone ? mul_rn(wth, nb2) : wth * nb2};
   const T pe = finish_sqrt((err[0] * err[0] + err[1] * err[1]) + err[2] * err[2]);
   const bool last = it >= a.k.max_iters;
-  const bool conv = !last && (pe < a.k.pos_thresh) && (th < a.rot_thresh);
+  const bool conv = !last && (pe < a.k.pos_thresh) && ((kCone ? th - alpha : th) < a.rot_thresh);
   if (active && (conv || last)) done(pp, R, ax, pe, th, conv ? it + 1 : it, conv);
   // rows 3 and 4: w b1^T jacr, w b2^T jacr
   T Jt[35];
 #pragma unroll
   for (int j = 0; j < 21; ++j) Jt[j] = J[j];
-  const T wb1[3] = {a.rot_weight * b1[0], a.rot_weight * b1[1], a.rot_weight * b1[2]};
-  const T wb2[3] = {a.rot_weight * b2[0], a.rot_weight * b2[1], a.rot_weight * b2[2]};
+  const T w = on ? a.rot_weight : T(0);
+  const T wb1[3] = {kCone ? mul_rn(w, b1[0]) : w * b1[0], kCone ? mul_rn(w, b1[1]) : w * b1[1],
+                    kCone ? mul_rn(w, b1[2]) : w * b1[2]};
+  const T wb2[3] = {kCone ? mul_rn(w, b2[0]) : w * b2[0], kCone ? mul_rn(w, b2[1]) : w * b2[1],
+                    kCone ? mul_rn(w, b2[2]) : w * b2[2]};
 #pragma unroll
   for (int j = 0; j < NJ; ++j) {
     Jt[21 + j] = (wb1[0] * J[21 + j] + wb1[1] * J[28 + j]) + wb1[2] * J[35 + j];
@@ -2001,36 +2031,57 @@ __device__ __noinline__ void axis_pass_call(const AxisIkArgs<T>& a, const Trig<T
                            });
 }
 
+// The cone pass's one out-of-line FP64 copy, for the same reason: the cone kernel and its restarts both call it.
+template <typename T, typename Kin>
+__device__ __noinline__ void axis_cone_pass_call(const AxisIkArgs<T>& a, const Trig<T>& trig, T (&q)[NJ],
+                                                 const T (&tp)[3], const T (&d)[3], int it, bool active, T alpha,
+                                                 bool& fin, T (&pp)[3], T (&R)[9], T (&ax)[3], T& pe, T& th, int& its,
+                                                 bool& conv) {
+  fin = false;
+  axis_pass_inline<T, Kin, true>(a, trig, q, tp, d, it, active,
+                                 [&](const T* p_, const T* r_, const T* x_, T pe_, T th_, int its_, bool conv_) {
+                                   for (int i = 0; i < 3; ++i) { pp[i] = p_[i]; ax[i] = x_[i]; }
+                                   for (int i = 0; i < 9; ++i) R[i] = r_[i];
+                                   pe = pe_; th = th_; its = its_; conv = conv_; fin = true;
+                                 },
+                                 alpha);
+}
+
 // axis_pass_inline's contract, for either precision
-template <typename T, typename Kin, typename Done>
+template <typename T, typename Kin, bool kCone = false, typename Done>
 __device__ __forceinline__ void axis_pass(const AxisIkArgs<T>& a, const Trig<T>& trig, T (&q)[NJ], const T (&tp)[3],
-                                          const T (&d)[3], int it, bool active, Done done) {
+                                          const T (&d)[3], int it, bool active, Done done, T alpha = T(0)) {
   if constexpr (std::is_same<T, double>::value) {
     T qn[NJ], pp[3], R[9], ax[3], pe, th;
     int its;
     bool fin, conv;
 #pragma unroll
     for (int j = 0; j < NJ; ++j) qn[j] = q[j];
-    axis_pass_call<T, Kin>(a, trig, qn, tp, d, it, active, fin, pp, R, ax, pe, th, its, conv);
+    if constexpr (kCone)
+      axis_cone_pass_call<T, Kin>(a, trig, qn, tp, d, it, active, alpha, fin, pp, R, ax, pe, th, its, conv);
+    else
+      axis_pass_call<T, Kin>(a, trig, qn, tp, d, it, active, fin, pp, R, ax, pe, th, its, conv);
     if (fin) done(pp, R, ax, pe, th, its, conv);  // q is still the q the lane finished at
 #pragma unroll
     for (int j = 0; j < NJ; ++j) q[j] = qn[j];
   } else {
-    axis_pass_inline<T, Kin>(a, trig, q, tp, d, it, active, done);
+    axis_pass_inline<T, Kin, kCone>(a, trig, q, tp, d, it, active, done, alpha);
   }
 }
 
-// the success rule of a finished axis solve
-template <typename T>
-__device__ __forceinline__ bool axis_success(const AxisIkArgs<T>& a, T pe, T th, bool conv) {
+// the success rule of a finished axis solve (kCone: of the cone solve, theta - alpha in place of theta)
+template <typename T, bool kCone = false>
+__device__ __forceinline__ bool axis_success(const AxisIkArgs<T>& a, T pe, T th, bool conv, T alpha = T(0)) {
+  if constexpr (kCone) th = th - alpha;
   return conv && (pe < a.k.pos_thresh * T(2)) && (th < a.rot_thresh * T(2));
 }
 
 // Store the record of query e (every output but q_out nullable); qcur is read only when final_quat is asked for
-template <typename T>
+template <typename T, bool kCone = false>
 __device__ __forceinline__ void axis_store(const AxisIkArgs<T>& a, unsigned e, const T (&q)[NJ], const T* pp,
-                                           const T* ax, const T* qcur, T pe, T th, int iterations, bool conv) {
-  const bool success = axis_success(a, pe, th, conv);
+                                           const T* ax, const T* qcur, T pe, T th, int iterations, bool conv,
+                                           T alpha = T(0)) {
+  const bool success = axis_success<T, kCone>(a, pe, th, conv, alpha);
 #pragma unroll
   for (int i = 0; i < NJ; ++i) a.q_out[(size_t)e * NJ + i] = q[i];
   if (a.final_pos) { a.final_pos[(size_t)e * 3] = pp[0]; a.final_pos[(size_t)e * 3 + 1] = pp[1]; a.final_pos[(size_t)e * 3 + 2] = pp[2]; }
@@ -2045,14 +2096,10 @@ __device__ __forceinline__ void axis_store(const AxisIkArgs<T>& a, unsigned e, c
   if (a.flags) a.flags[e] = (uint8_t)((conv ? PNP_IK_CONVERGED : 0u) | (success ? PNP_IK_SUCCESS : 0u));
 }
 
-// Persistent warps with lane refill, as ik_pose_solve_kernel.  The FP32 instantiation uses the table trig.
-template <typename T, typename Kin>
-__global__ void __launch_bounds__(IK_BLOCK) ik_axis_solve_kernel(const AxisIkArgs<T> a) {
-  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
-  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
-  __syncthreads();
-  if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
-  const Trig<T> trig{s_tab};
+// Persistent warps with lane refill, as ik_pose_solve_kernel: the loop of one warp after the trig table is loaded.
+// The plain and the cone kernel run it with kCone false and true.
+template <typename T, typename Kin, bool kCone>
+__device__ __forceinline__ void axis_solve_warp(const AxisIkArgs<T>& a, const Trig<T>& trig, T alpha) {
   unsigned long long c_n = 0, c_conv = 0, c_iter = 0;
   WarpPool pool;
   bool exhausted = false, active = false;
@@ -2075,28 +2122,43 @@ __global__ void __launch_bounds__(IK_BLOCK) ik_axis_solve_kernel(const AxisIkArg
         });
     if (!__any_sync(FULL, active)) break;
 
-    axis_pass<T, Kin>(a, trig, q, tp, d, it, active,
-                      [&](const T* pp, const T* R, const T* ax, T pe, T th, int iterations, bool conv) {
-                        T qcur[4];
-                        if (a.final_quat) mat2quat_fast(R, qcur);
-                        axis_store(a, e, q, pp, ax, qcur, pe, th, iterations, conv);
-                        c_n += 1; c_conv += conv ? 1 : 0; c_iter += (unsigned long long)iterations;
-                        active = false;
-                      });
+    axis_pass<T, Kin, kCone>(a, trig, q, tp, d, it, active,
+                             [&](const T* pp, const T* R, const T* ax, T pe, T th, int iterations, bool conv) {
+                               T qcur[4];
+                               if (a.final_quat) mat2quat_fast(R, qcur);
+                               axis_store<T, kCone>(a, e, q, pp, ax, qcur, pe, th, iterations, conv, alpha);
+                               c_n += 1; c_conv += conv ? 1 : 0; c_iter += (unsigned long long)iterations;
+                               active = false;
+                             },
+                             alpha);
     ++it;
   }
   ik_counters_add(a.counters, c_n, c_conv, c_iter);
 }
 
-// ---- multi-start axis IK (pnp_ik_axis_solve_multistart_*): ms_pose_wave_kernel with axis_pass / axis_store ---------
+// The FP32 instantiations use the table trig.
 template <typename T, typename Kin>
-__global__ void __launch_bounds__(MS_BLOCK) ms_axis_wave_kernel(const MsArgs<AxisIkArgs<T>> m) {
-  const unsigned cnt = *m.cnt_in;
-  if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;  // no work for any warp of this block
+__global__ void __launch_bounds__(IK_BLOCK) ik_axis_solve_kernel(const AxisIkArgs<T> a) {
   __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
   if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
   __syncthreads();
-  const Trig<T> trig{s_tab};
+  if (a.solo_warp && threadIdx.x >= 32) return;  // helper warps of a small-batch block: table loaded, done
+  axis_solve_warp<T, Kin, false>(a, Trig<T>{s_tab}, T(0));
+}
+
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(IK_BLOCK) ik_axis_cone_solve_kernel(const AxisConeIkArgs<T> a) {
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  if (a.solo_warp && threadIdx.x >= 32) return;
+  axis_solve_warp<T, Kin, true>(a, Trig<T>{s_tab}, a.cone_angle);
+}
+
+// ---- multi-start axis IK (pnp_ik_axis_solve_multistart_*, pnp_ik_axis_cone_solve_multistart_*): ms_pose_wave_kernel
+// with axis_pass / axis_store, after the trig table is loaded --------------------------------------------------------
+template <typename T, typename Kin, bool kCone, typename A>
+__device__ __forceinline__ void ms_axis_wave(const MsArgs<A>& m, unsigned cnt, const Trig<T>& trig, T alpha) {
   // the finished attempt of this lane: q, position, axis, quaternion (when asked for) and errors at its last pass
   T qk[NJ], pk[3], ak[3], qck[4], pek = T(0), thk = T(0);
   bool conv = false;
@@ -2110,22 +2172,43 @@ __global__ void __launch_bounds__(MS_BLOCK) ms_axis_wave_kernel(const MsArgs<Axi
     conv = false;
     it_kept = 0;
     for (int it = 0; __any_sync(FULL, active); ++it)
-      axis_pass<T, Kin>(m.a, trig, q, tp, d, it, active,
-                        [&](const T* pp, const T* R, const T* ax, T pe, T th, int its, bool cv) {
+      axis_pass<T, Kin, kCone>(m.a, trig, q, tp, d, it, active,
+                               [&](const T* pp, const T* R, const T* ax, T pe, T th, int its, bool cv) {
 #pragma unroll
-                          for (int i = 0; i < NJ; ++i) qk[i] = q[i];
+                                 for (int i = 0; i < NJ; ++i) qk[i] = q[i];
 #pragma unroll
-                          for (int i = 0; i < 3; ++i) { pk[i] = pp[i]; ak[i] = ax[i]; }
-                          if (m.a.final_quat) mat2quat_fast(R, qck);
-                          pek = pe; thk = th; it_kept = its; conv = cv;
-                          active = false;
-                        });
+                                 for (int i = 0; i < 3; ++i) { pk[i] = pp[i]; ak[i] = ax[i]; }
+                                 if (m.a.final_quat) mat2quat_fast(R, qck);
+                                 pek = pe; thk = th; it_kept = its; conv = cv;
+                                 active = false;
+                               },
+                               alpha);
     iterations = it_kept;
-    succ = axis_success(m.a, pek, thk, conv);
+    succ = axis_success<T, kCone>(m.a, pek, thk, conv, alpha);
   };
   auto prev = [&](unsigned id, unsigned& fl, unsigned& it) { ms_ik_prev<IK_OUT_SEPARATE>(m, id, fl, it); };
-  auto store = [&](unsigned id) { axis_store(m.a, id, qk, pk, ak, qck, pek, thk, it_kept, conv); };
+  auto store = [&](unsigned id) { axis_store<T, kCone>(m.a, id, qk, pk, ak, qck, pek, thk, it_kept, conv, alpha); };
   ms_wave(m, cnt, solve, prev, store);
+}
+
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(MS_BLOCK) ms_axis_wave_kernel(const MsArgs<AxisIkArgs<T>> m) {
+  const unsigned cnt = *m.cnt_in;
+  if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;  // no work for any warp of this block
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  ms_axis_wave<T, Kin, false>(m, cnt, Trig<T>{s_tab}, T(0));
+}
+
+template <typename T, typename Kin>
+__global__ void __launch_bounds__(MS_BLOCK) ms_axis_cone_wave_kernel(const MsArgs<AxisConeIkArgs<T>> m) {
+  const unsigned cnt = *m.cnt_in;
+  if ((unsigned long long)blockIdx.x * 32u >= (unsigned long long)cnt * m.group) return;
+  __shared__ __align__(16) float s_tab[Trig<T>::kUsesTable ? kTrigVWords : 4];
+  if (Trig<T>::kUsesTable) load_trigv_table(s_tab);
+  __syncthreads();
+  ms_axis_wave<T, Kin, true>(m, cnt, Trig<T>{s_tab}, m.a.cone_angle);
 }
 
 // =============================================================================================

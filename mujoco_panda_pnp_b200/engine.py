@@ -494,24 +494,37 @@ def _axis_result(o, **extra):
     return dict(o, converged=(flags & 1) != 0, success=(flags & 2) != 0, **extra)
 
 
+def _axis_entry(lib, dt, multistart, rot_thresh, cone_angle, rot_weight):
+    """(entry point, its name, its arguments after tool_axis up to q_out): the axis solve's, or the cone solve's when
+    cone_angle is not None."""
+    name = "pnp_ik_axis_solve" if cone_angle is None else "pnp_ik_axis_cone_solve"
+    name += ("_multistart" if multistart else "") + ("_f32" if dt == torch.float32 else "_f64")
+    angles = (float(rot_thresh),) if cone_angle is None else (float(rot_thresh), float(cone_angle))
+    return getattr(lib, name), name, (*angles, float(rot_weight))
+
+
 def ik_axis_solve(target_pos: torch.Tensor, target_axis: torch.Tensor, q_init: torch.Tensor, params: PnpIkParams,
                   tool_axis=(0.0, 0.0, 1.0), rot_thresh: float = 1e-2, rot_weight: float = 1.0,
-                  counters: Optional[torch.Tensor] = None) -> dict:
+                  counters: Optional[torch.Tensor] = None, cone_angle: Optional[float] = None) -> dict:
     """Axis-constrained IK (extension, pnp_ik_axis_solve_*): put the site at target_pos[N,3] with its ``tool_axis``
     (site frame, (3,)) along target_axis[N,3] (world frame, any norm), the roll about that axis free.  q_init[N,7] or
     [7].  Returns q, final_pos, final_axis (the tool axis in the world frame), final_quat, pos_error, axis_error (the
-    angle between final_axis and the target axis, rad), iterations, converged, success."""
+    angle between final_axis and the target axis, rad), iterations, converged, success.
+
+    ``cone_angle`` (rad, in [0, pi]): accept the tool axis anywhere within that angle of the target axis
+    (pnp_ik_axis_cone_solve_*); axis_error stays the true angle.  None runs the exact axis solve."""
     lib = _lib.load()
     target_pos, target_axis, tool = _axis_inputs(target_pos, target_axis, tool_axis)
     dt, n, dev = target_pos.dtype, target_pos.shape[0], target_pos.device
     q_init, stride = _q_init_arg(q_init, n, dt, dev)
-    fn = lib.pnp_ik_axis_solve_f32 if dt == torch.float32 else lib.pnp_ik_axis_solve_f64
+    fn, name, thr = _axis_entry(lib, dt, False, rot_thresh, cone_angle, rot_weight)
     with torch.cuda.device(dev):
         o = _axis_outputs(n, dt, dev)
         _lib.check(
             fn(_ptr(target_pos), _ptr(target_axis), _ptr(q_init), stride, n, ctypes.byref(params), tool,
-               float(rot_thresh), float(rot_weight), *(_ptr(t) for t in o.values()), _ptr(counters), _stream()),
-            "pnp_ik_axis_solve",
+               *thr, *(_ptr(t) for t in o.values()), _ptr(counters),
+               _stream()),
+            name[:-4],
         )
     return _axis_result(o)
 
@@ -519,25 +532,26 @@ def ik_axis_solve(target_pos: torch.Tensor, target_axis: torch.Tensor, q_init: t
 def ik_axis_solve_multistart(target_pos: torch.Tensor, target_axis: torch.Tensor, q_init: torch.Tensor,
                              seeds: torch.Tensor, params: PnpIkParams, tool_axis=(0.0, 0.0, 1.0),
                              rot_thresh: float = 1e-2, rot_weight: float = 1.0, counters: Optional[torch.Tensor] = None,
-                             restart_stats: Optional[torch.Tensor] = None) -> dict:
+                             restart_stats: Optional[torch.Tensor] = None, cone_angle: Optional[float] = None) -> dict:
     """ik_axis_solve, then every query it did not solve is solved again from the rows of ``seeds`` (K, 7), in order,
     until one succeeds (pnp_ik_axis_solve_multistart_*).  Each row of the result is, bit for bit, the plain
     ik_axis_solve of that target from the start ``attempt`` names (0 = q_init, k = seeds[k - 1]).  Returns
-    ik_axis_solve's dict plus ``attempt`` (uint8[N]); ``counters`` / ``restart_stats`` as ik_pose_solve_multistart.
-    Never synchronises."""
+    ik_axis_solve's dict plus ``attempt`` (uint8[N]); ``counters`` / ``restart_stats`` as ik_pose_solve_multistart;
+    ``cone_angle`` as ik_axis_solve (pnp_ik_axis_cone_solve_multistart_*).  Never synchronises."""
     lib = _lib.load()
     target_pos, target_axis, tool = _axis_inputs(target_pos, target_axis, tool_axis)
     dt, n, dev = target_pos.dtype, target_pos.shape[0], target_pos.device
     q_init, stride = _q_init_arg(q_init, n, dt, dev)
     seeds, scratch, attempt = _multistart_inputs(seeds, n, dt, dev, counters, restart_stats)
-    fn = lib.pnp_ik_axis_solve_multistart_f32 if dt == torch.float32 else lib.pnp_ik_axis_solve_multistart_f64
+    fn, name, thr = _axis_entry(lib, dt, True, rot_thresh, cone_angle, rot_weight)
     with torch.cuda.device(dev):
         o = _axis_outputs(n, dt, dev)
         _lib.check(
             fn(_ptr(target_pos), _ptr(target_axis), _ptr(q_init), stride, n, _ptr(seeds), seeds.shape[0],
-               ctypes.byref(params), tool, float(rot_thresh), float(rot_weight), *(_ptr(t) for t in o.values()),
-               _ptr(attempt), _ptr(counters), _ptr(restart_stats), _ptr(scratch), _stream()),
-            "pnp_ik_axis_solve_multistart",
+               ctypes.byref(params), tool, *thr,
+               *(_ptr(t) for t in o.values()), _ptr(attempt), _ptr(counters), _ptr(restart_stats), _ptr(scratch),
+               _stream()),
+            name[:-4],
         )
     return _axis_result(o, attempt=attempt)
 

@@ -177,7 +177,7 @@ class JacobianIKController:
 
     def solve_axis(self, target_pos, target_axis, q_init, max_iters: int = 100, pos_thresh: float = 1e-3,
                    damping: float = 1e-2, step_limit: float = 0.1, tool_axis=(0.0, 0.0, 1.0), rot_thresh: float = 1e-2,
-                   rot_weight: float = 1.0, seeds=None) -> dict:
+                   rot_weight: float = 1.0, seeds=None, cone_angle=None) -> dict:
         """Axis-constrained IK (EXTENSION: see pnp_ik_axis_solve_* in include/pnp_b200.h): the site at target_pos
         with its ``tool_axis`` (site frame; the default +z is the packaged Panda's approach direction) along
         target_axis (world frame), the roll about that axis free - e.g. a top-down grasp is target_axis (0, 0, -1).
@@ -185,7 +185,9 @@ class JacobianIKController:
         with q, final_pos, final_axis, final_quat, pos_error, axis_error (rad), iterations, converged, success.
 
         ``seeds`` (K, 7), K <= 255: as solve_pose (engine.ik_axis_solve_multistart); the dict then also holds
-        ``attempt``."""
+        ``attempt``.  ``cone_angle`` (rad, in [0, pi]): accept the tool axis anywhere within that angle of target_axis
+        (pnp_ik_axis_cone_solve_*), e.g. a top-down grasp that tolerates 15 degrees of tilt; None asks for the exact
+        axis."""
         dt = self._dtype()
         with torch.cuda.device(self.device):
             engine.set_tree(self.tree)
@@ -193,7 +195,7 @@ class JacobianIKController:
             ta = _to_tensor(target_axis).to(device=self.device, dtype=dt).reshape(-1, 3)
             qi = _to_tensor(q_init).to(device=self.device, dtype=dt)
             params = self._params(max_iters, pos_thresh, damping, step_limit)
-            kw = dict(tool_axis=tool_axis, rot_thresh=rot_thresh, rot_weight=rot_weight)
+            kw = dict(tool_axis=tool_axis, rot_thresh=rot_thresh, rot_weight=rot_weight, cone_angle=cone_angle)
             if seeds is not None:
                 sd = _to_tensor(seeds).to(device=self.device, dtype=dt)
                 return engine.ik_axis_solve_multistart(tp, ta, qi, sd, params, **kw)
